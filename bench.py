@@ -2,6 +2,7 @@
 """bench.py -- Gpixel/s of the fused DCT -> quantise -> IDCT hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu]
+                    [--dump-outputs DIR]
 
 One "step" = one fused pass (b200dct_roundtrip, HpApprDCT: Haweel T, JPEG Q, all
 coefficients kept) over one 8192 x 8192 fp32 image per GPU -- BASELINE.json configs[1].
@@ -10,8 +11,8 @@ of an (N*8192) x 8192 image: block-row striping, no halo, no data-path collectiv
 scaling.  Rank 0 prints ONE JSON line.
 
 Legs of the default arm, all on the same workload:
-  value        device-resident: inputs already in HBM, K launches timed with CUDA events on
-               the launching stream, barrier + synchronize on both sides, max over ranks;
+  value        device-resident: inputs already in HBM, exactly K launches timed with CUDA
+               events on the launching stream, barrier + synchronize on both sides, max over ranks;
                the step rotates over 4 input/output buffer pairs (2 GiB) so nothing is L2
                resident (one image pair alone is 512 MiB against a 126 MB L2).
   roofline     algorithmic bytes per launch (8 B/px: 4 read + 4 written) / average launch
@@ -215,7 +216,7 @@ def run_reference_gpu(args):
     for _ in range(args.warmup):
         step()
     kms.clear()
-    steps = min(args.steps, 20)
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         step()
@@ -236,28 +237,35 @@ def run_reference_gpu(args):
 
 
 # ------------------------------------------------------------------ our arm
-WINDOWS = 5   # consecutive K-step windows timed back to back; the median window is reported
+WINDOWS = 5   # the K timed steps are split into up to 5 consecutive windows; the median window is reported
+DUMP_ROWS = 1024   # --dump-outputs: rows of output written in all, shared by the ranks (32 MiB of f32)
 
 
-def timed_windows(step, k, windows, stream, warm=0):
-    """Enqueue `warm` untimed steps and then `windows` windows of `k` steps each on `stream`, with
+def split_steps(k, windows=WINDOWS):
+    """Window sizes that add up to exactly k steps (at most `windows` windows, sizes differ by <= 1)."""
+    n = max(1, min(windows, k))
+    return [k // n + (1 if w < k % n else 0) for w in range(n)]
+
+
+def timed_windows(step, sizes, stream, warm=0):
+    """Enqueue `warm` untimed steps and then one window of sizes[w] steps per entry on `stream`, with
     NO host synchronisation anywhere in between: event i sits between window i-1 and window i, so
     every window starts on a busy GPU (the first launch of a window overlaps the previous kernel's
     tail exactly like every other launch).  Returns the window times in ms."""
     import torch
 
-    evs = [torch.cuda.Event(enable_timing=True) for _ in range(windows + 1)]
+    evs = [torch.cuda.Event(enable_timing=True) for _ in range(len(sizes) + 1)]
     for i in range(warm):
         step(i)
     evs[0].record(stream)
     n = warm
-    for w in range(windows):
+    for w, k in enumerate(sizes):
         for _ in range(k):
             step(n)
             n += 1
         evs[w + 1].record(stream)
     torch.cuda.synchronize()
-    return [evs[w].elapsed_time(evs[w + 1]) for w in range(windows)]
+    return [evs[w].elapsed_time(evs[w + 1]) for w in range(len(sizes))]
 
 
 def rotating(m, plan, ins, outs, stream, coef=None):
@@ -303,17 +311,21 @@ def run_ours(args):
     torch.cuda.synchronize()
     kernel_path = m.api.last_path()
 
-    # Timed region.  barrier + synchronize, then W warm-up steps and WINDOWS windows of exactly K
-    # steps are enqueued back to back with no synchronisation in between; barrier + synchronize
-    # after.  Reported: the MEDIAN window (per rank), max over ranks.
+    # Timed region.  barrier + synchronize, then W warm-up steps and exactly K timed steps, split
+    # into up to WINDOWS consecutive windows, are enqueued back to back with no synchronisation in
+    # between; barrier + synchronize after.  Reported: the MEDIAN window's time per step (per
+    # rank), max over ranks.
+    sizes = split_steps(K)
     sampler = ClockSampler(local_rank).start()
     m.dist.barrier()
     torch.cuda.synchronize()
     launches = 0
-    windows = timed_windows(step, K, WINDOWS, stream, warm=W)
+    windows = timed_windows(step, sizes, stream, warm=W)
     m.dist.barrier()
-    timed_launches = launches - W                     # kernels launched inside the WINDOWS timed windows
-    ms_local = statistics.median(windows)
+    timed_launches = launches - W                     # kernels launched inside the timed windows
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs[(W + K - 1) % NBUF], rank, world)   # what the last timed step returned
+    ms_local = statistics.median(ms / k for ms, k in zip(windows, sizes))   # per step
     # keep the identical load running briefly if the timed region was too short to sample clocks
     extra = 0
     t_end = time.perf_counter() + (0.0 if sum(windows) > 400 else 0.6)
@@ -324,16 +336,15 @@ def run_ours(args):
         extra += 64
     clocks = sampler.stop()
     clocks["sampled_over"] = "timed region" if extra == 0 else f"timed region + {extra} identical launches (region < 0.4 s)"
-    ms_total = m.dist.max_over_ranks(ms_local, dev)
-    per_rank = m.dist.all_ranks(ms_local / K, dev)
-    first_window = m.dist.max_over_ranks(windows[0], dev)
-    value = px * world * K / (ms_total * 1e-3) / 1e9
-    ms_per_step = ms_total / K
+    ms_per_step = m.dist.max_over_ranks(ms_local, dev)
+    per_rank = m.dist.all_ranks(ms_local, dev)
+    first_window = m.dist.max_over_ranks(windows[0] / sizes[0], dev)
+    value = px * world / (ms_per_step * 1e-3) / 1e9
 
-    # per-launch duration of the dominant kernel: a window is nothing but K back-to-back launches
-    # of it on this stream, so window time / K is its average duration
+    # per-launch duration of the dominant kernel: a window is nothing but back-to-back launches
+    # of it on this stream, so window time / its steps is its average duration
     peak, peak_src = measured_peak()
-    k_ms = ms_local / K
+    k_ms = ms_local
     achieved = BYTES_PER_PX * px / (k_ms * 1e-3) / 1e9
     traffic = ncu_traffic()
     roofline = {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
@@ -369,13 +380,14 @@ def run_ours(args):
                                "fused DCT+quant+dequant+IDCT (BASELINE configs[1])",
                    "striping": f"{world} block-row stripe(s) of a {N_SIDE * world}x{N_SIDE} image, no halo, no collective",
                    "l2": "inputs larger than L2: 4 rotating in/out pairs, 2 GiB working set vs 126 MB L2",
-                   "timing": f"barrier+synchronize, then {W} warm-up steps and {WINDOWS} consecutive windows of exactly {K} steps "
-                             "enqueued back to back on one stream (CUDA events between windows, no host synchronisation inside), "
-                             "barrier+synchronize; ms_per_step = median window / steps, max over ranks",
+                   "timing": f"barrier+synchronize, then {W} warm-up steps and exactly {K} timed steps in {len(sizes)} consecutive "
+                             f"windows of {'/'.join(map(str, sizes))} steps enqueued back to back on one stream (CUDA events between "
+                             "windows, no host synchronisation inside), barrier+synchronize; ms_per_step = median over windows of "
+                             "window time / its steps, max over ranks",
                    "launch": "consecutive launches overlap tail and set-up through programmatic dependent launch "
                              "(each kernel waits for its predecessor before touching memory)",
                    "kernel_path": kernel_path},
-        "windows_ms": windows, "first_window_ms_per_step": first_window / K,
+        "windows_ms": windows, "window_steps": sizes, "first_window_ms_per_step": first_window,
         "per_rank_ms_per_step": {"min": min(per_rank), "median": statistics.median(per_rank), "max": max(per_rank),
                                  "all": per_rank},
         "roofline": roofline, "e2e": e2e, "gpu_launches": timed_launches, "clocks": clocks,
@@ -406,6 +418,19 @@ def run_ours(args):
     m.dist.barrier()
     m.dist.shutdown()
     return 0
+
+
+def dump_outputs(out_dir, out, rank, world):
+    """Write DUMP_ROWS // world rows of this rank's output image `out` (a fixed, seeded choice of
+    rows, the same in every run) to out_dir/out_rank<rank>.npy as float32: DUMP_ROWS rows, 32 MiB,
+    over all ranks."""
+    import numpy as np
+    import torch
+
+    rows = np.sort(np.random.default_rng(0).choice(out.shape[0], max(1, DUMP_ROWS // world), replace=False))
+    sample = out.index_select(0, torch.from_numpy(rows).to(out.device)).float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"out_rank{rank}.npy"), sample)
 
 
 def e2e_leg(m, plan, dev, world, args):
@@ -478,7 +503,7 @@ def pcie_ceiling(world):
 def time_config(m, step, k=20, windows=3, warm=5):
     import torch
 
-    w = timed_windows(step, k, windows, torch.cuda.current_stream(), warm=warm)
+    w = timed_windows(step, [k] * windows, torch.cuda.current_stream(), warm=warm)
     return statistics.median(w) / k
 
 
@@ -626,7 +651,7 @@ def extras_multi_gpu(m, dev, rank, world):
     step(0)
     m.dist.barrier()
     torch.cuda.synchronize()
-    ms = statistics.median(timed_windows(step, 10, 3, stream, warm=3)) / 10
+    ms = statistics.median(timed_windows(step, [10] * 3, stream, warm=3)) / 10
     m.dist.barrier()
     ms = m.dist.max_over_ranks(ms, dev)
 
@@ -653,7 +678,7 @@ def extras_multi_gpu(m, dev, rank, world):
     bstep(0)
     m.dist.barrier()
     torch.cuda.synchronize()
-    bms = statistics.median(timed_windows(bstep, 5, 3, stream, warm=2)) / 5
+    bms = statistics.median(timed_windows(bstep, [5] * 3, stream, warm=2)) / 5
     m.dist.barrier()
     bms = m.dist.max_over_ranks(bms, dev)
     bok = all(int(np.abs(batch.outs[j][a:a + 16].cpu().numpy().astype(np.int16)
@@ -676,7 +701,7 @@ def extras_multi_gpu(m, dev, rank, world):
         fstep(0)
         torch.cuda.synchronize()
         m.dist.barrier()
-        fms = statistics.median(timed_windows(fstep, 5, 3, stream, warm=1)) / 5
+        fms = statistics.median(timed_windows(fstep, [5] * 3, stream, warm=1)) / 5
         m.dist.barrier()
         fms = m.dist.max_over_ranks(fms, dev)
         fok = True
@@ -745,14 +770,24 @@ def reference_gpu_kernels(d_img, d_out):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
-    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 200; 10 for --impl reference, 20 for --impl reference-gpu)")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed steps first (default: 10; 3 for --impl reference)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "reference-gpu"])
     ap.add_argument("--no-baselines", action="store_true", help="skip the CPU / reference-GPU baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help=f"after the timed steps, write {DUMP_ROWS} fixed rows in all (seeded choice, {DUMP_ROWS}/N per rank) "
+                         "of the image the last timed step returned to DIR/out_rank<rank>.npy (float32, 32 MiB in all); "
+                         "the inputs are the same in every run")
     args = ap.parse_args()
+    steps, warmup = {"ours": (200, 10), "reference": (10, 3), "reference-gpu": (20, 10)}[args.impl]
+    args.steps = steps if args.steps is None else args.steps
+    args.warmup = warmup if args.warmup is None else args.warmup
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the default arm (--impl ours)")
     if args.impl == "reference":
-        if args.steps == 200:
-            args.steps, args.warmup = 10, 3
         return run_reference_cpu(args)
     if args.impl == "reference-gpu":
         return run_reference_gpu(args)

@@ -1,8 +1,12 @@
-"""Test helper: run the UNMODIFIED reference (oracle/_ref/libref_*.so, built from
-/root/reference by oracle/Makefile) on torch CUDA tensors.  Test infrastructure only."""
+"""Test helper: run the UNMODIFIED reference (oracle/_ref/libref_*.so, built by oracle/Makefile
+where the reference's sources are present) on torch CUDA tensors, and the stored digests of the
+CPU oracle's outputs (tests/golden/refgpu_digests.json) that stand in for it where it is not
+built.  Test infrastructure only."""
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import os
 import re
 import sys
@@ -10,6 +14,7 @@ import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_DIR = os.path.join(ROOT, "oracle", "_ref")
+DIGESTS = os.path.join(ROOT, "tests", "golden", "refgpu_digests.json")
 VARIANTS = {"newappr": "libref_newappr.so", "fastappr": "libref_fastappr.so",
             "cublas": "libref_cublas.so", "cublas2": "libref_cublas2.so"}
 _libs = {}
@@ -17,6 +22,25 @@ _libs = {}
 
 def available(variant: str = "newappr") -> bool:
     return os.path.exists(os.path.join(REF_DIR, VARIANTS[variant]))
+
+
+def digest(a) -> str:
+    """sha256 over dtype, shape and the raw bytes (C order) of a numpy array or torch tensor:
+    equal digests mean equal bits, sign of zero included."""
+    import numpy as np
+
+    if hasattr(a, "detach"):
+        a = a.detach().cpu().numpy()
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def stored(case: str) -> dict:
+    """Digests (and metrics) of the oracle's outputs for one case of make_ref_digests.py."""
+    with open(DIGESTS) as f:
+        return json.load(f)["cases"][case]
 
 
 def load(variant: str) -> C.CDLL:

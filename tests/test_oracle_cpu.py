@@ -92,6 +92,22 @@ def test_reference_gpu_fixtures(oracle):
         assert np.array_equal(rec.view(np.uint32), g["rec"].view(np.uint32)), f
 
 
+def test_stored_oracle_digests_are_still_reproduced(oracle):
+    """tests/golden/refgpu_digests.json (the oracle's digests, which the GPU suite compares with
+    where the reference is not built) is still what the oracle produces, on its smaller cases.
+    A guard against changes of the oracle or edits of the file; what pins the oracle to the
+    reference is test_reference_gpu_fixtures."""
+    import refgpu
+
+    for case, img, Q in (("rand256", oracle.rand_image(256, 256, 42), None), ("adversarial32", inputs.adversarial(32), None),
+                         ("floatnoise64x256", inputs.float_noise(64, 256), None),
+                         ("rand256_seed5_halfq", oracle.rand_image(256, 256, 5), oracle.jpeg_Q() * 0.5)):
+        want = refgpu.stored(case)
+        coef, shifted = oracle.dct(img, Q=Q, want_shifted=True)
+        assert refgpu.digest(coef) == want["coef"] and refgpu.digest(shifted) == want["shifted"], case
+        assert refgpu.digest(oracle.idct(coef, Q=Q)) == want["rec"], case
+
+
 def test_split_equals_fused_and_u8(oracle):
     img = inputs.adversarial(8)
     coef = oracle.dct(img)
