@@ -27,6 +27,8 @@ from .api import (  # noqa: F401
     ImageBatch,
     roundtrip_host,
     roundtrip_rgb,
+    forward_rgb,
+    inverse_rgb,
     coded_bits,
     compression_factor,
     roundtrip_with_metrics,
@@ -39,5 +41,5 @@ from .stripes import batch_images, stripe_rows  # noqa: F401
 __all__ = [
     "ALL_COEFFS", "B200DCTError", "HostPipeline", "Plan", "build", "dct_all_blocks", "dct_all_blocks_cuda", "forward",
     "idct_all_blocks", "idct_all_blocks_cuda", "inverse", "lib", "lib_path", "metrics", "roundtrip",
-    "roundtrip_any", "roundtrip_batch", "ImageBatch", "roundtrip_host", "roundtrip_rgb", "coded_bits", "compression_factor", "roundtrip_with_metrics", "stripe_rows", "batch_images", "zigzag_mask",
+    "roundtrip_any", "roundtrip_batch", "ImageBatch", "roundtrip_host", "roundtrip_rgb", "forward_rgb", "inverse_rgb", "coded_bits", "compression_factor", "roundtrip_with_metrics", "stripe_rows", "batch_images", "zigzag_mask",
 ]

@@ -73,6 +73,8 @@ def lib() -> C.CDLL:
         L.b200dct_plan_set_chroma_quant.argtypes = [vp, C.POINTER(C.c_float)]
         L.b200dct_plan_get_chroma_quant.argtypes = [vp, C.POINTER(C.c_float)]
         L.b200dct_roundtrip_rgb.argtypes = [vp, vp, sz, vp, sz, vp, sz, i, i, vp]
+        L.b200dct_forward_rgb.argtypes = [vp, vp, sz, vp, sz, i, i, vp]
+        L.b200dct_inverse_rgb.argtypes = [vp, vp, sz, vp, sz, i, i, vp]
         L.b200dct_zigzag_coded_bits.argtypes = [vp, sz, i, i, i, vp, vp]
         L.b200dct_host_pipeline_create.argtypes = [C.POINTER(vp), sz, i]
         L.b200dct_host_pipeline_destroy.argtypes = [vp]
@@ -444,6 +446,26 @@ def roundtrip_batch(imgs, outs=None, plan: Plan | None = None, stream=None):
     return batch.run(plan, stream)
 
 
+def _rgb_image(t, H, W, what):
+    """An interleaved (H, W, 3) uint8 CUDA tensor with rows of its own pitch (H, W None: any size)."""
+    import torch
+
+    if not (t.is_cuda and t.dtype == torch.uint8 and t.dim() == 3 and t.shape[2] == 3 and t.stride(2) == 1 and t.stride(1) == 3
+            and (H is None or tuple(t.shape) == (H, W, 3))):
+        raise B200DCTError("expected an interleaved (H, W, 3) uint8 CUDA tensor" if H is None else
+                           f"{what} must be an interleaved (H, W, 3) uint8 CUDA tensor like rgb")
+
+
+def _rgb_streams(t, H, W):
+    """(pointer, plane stride in bytes) of the (3, H/8, W/8, 64) int16 zig-zag streams of Y, Cb, Cr."""
+    import torch
+
+    if not (t.is_cuda and t.dtype == torch.int16 and t.dim() == 4 and (H is None or tuple(t.shape) == (3, H // 8, W // 8, 64))
+            and t.shape[0] == 3 and t.shape[3] == 64 and t[0].is_contiguous()):
+        raise B200DCTError("streams must be a (3, H/8, W/8, 64) int16 CUDA tensor")
+    return t.data_ptr(), t.stride(0) * 2
+
+
 def roundtrip_rgb(rgb, out=None, streams=None, plan: Plan | None = None, stream=None):
     """Colour round trip in one pass (b200dct_roundtrip_rgb): `rgb` is an (H, W, 3) uint8 CUDA
     tensor (interleaved, as the reference's loader returns colour files); RGB -> YCbCr (libjpeg)
@@ -452,23 +474,47 @@ def roundtrip_rgb(rgb, out=None, streams=None, plan: Plan | None = None, stream=
     streams of Y, Cb, Cr."""
     import torch
 
-    if not (rgb.is_cuda and rgb.dtype == torch.uint8 and rgb.dim() == 3 and rgb.shape[2] == 3
-            and rgb.stride(2) == 1 and rgb.stride(1) == 3):
-        raise B200DCTError("expected an interleaved (H, W, 3) uint8 CUDA tensor")
+    _rgb_image(rgb, None, None, "rgb")
     H, W = int(rgb.shape[0]), int(rgb.shape[1])
     with _on(rgb, stream):
         if out is None:
             out = torch.empty_like(rgb)
-        if not (out.is_cuda and out.dtype == torch.uint8 and tuple(out.shape) == (H, W, 3) and out.stride(2) == 1 and out.stride(1) == 3):
-            raise B200DCTError("out must be an interleaved (H, W, 3) uint8 CUDA tensor like rgb")
-        zp, zplane = None, 0
-        if streams is not None:
-            if not (streams.is_cuda and streams.dtype == torch.int16 and tuple(streams.shape) == (3, H // 8, W // 8, 64)
-                    and streams[0].is_contiguous()):
-                raise B200DCTError("streams must be a (3, H/8, W/8, 64) int16 CUDA tensor")
-            zp, zplane = streams.data_ptr(), streams.stride(0) * 2
+        _rgb_image(out, H, W, "out")
+        zp, zplane = _rgb_streams(streams, H, W) if streams is not None else (None, 0)
         _check(lib().b200dct_roundtrip_rgb(_plan(plan)._h, rgb.data_ptr(), rgb.stride(0), out.data_ptr(), out.stride(0),
                                            zp, zplane, H, W, _stream(stream)))
+    return out
+
+
+def forward_rgb(rgb, streams=None, plan: Plan | None = None, stream=None):
+    """First half of `roundtrip_rgb` (b200dct_forward_rgb): an (H, W, 3) uint8 CUDA tensor -> YCbCr ->
+    per-plane DCT / quantise -> the (3, H/8, W/8, 64) int16 zig-zag coefficient streams of Y, Cb, Cr
+    (written into `streams` when given).  They are what `roundtrip_rgb(rgb, streams=...)` writes."""
+    import torch
+
+    _rgb_image(rgb, None, None, "rgb")
+    H, W = int(rgb.shape[0]), int(rgb.shape[1])
+    with _on(rgb, stream):
+        if streams is None:
+            streams = torch.empty((3, H // 8, W // 8, 64), dtype=torch.int16, device=rgb.device)
+        zp, zplane = _rgb_streams(streams, H, W)
+        _check(lib().b200dct_forward_rgb(_plan(plan)._h, rgb.data_ptr(), rgb.stride(0), zp, zplane, H, W, _stream(stream)))
+    return streams
+
+
+def inverse_rgb(streams, out=None, plan: Plan | None = None, stream=None):
+    """Second half of `roundtrip_rgb` (b200dct_inverse_rgb): the (3, H/8, W/8, 64) int16 zig-zag streams
+    of Y, Cb, Cr -> per-plane dequantise / IDCT -> RGB, an (H, W, 3) uint8 CUDA tensor (written into
+    `out` when given).  inverse_rgb(forward_rgb(x)) == roundtrip_rgb(x) bit for bit with the same plan."""
+    import torch
+
+    zp, zplane = _rgb_streams(streams, None, None)
+    H, W = int(streams.shape[1]) * 8, int(streams.shape[2]) * 8
+    with _on(streams, stream):
+        if out is None:
+            out = torch.empty((H, W, 3), dtype=torch.uint8, device=streams.device)
+        _rgb_image(out, H, W, "out")
+        _check(lib().b200dct_inverse_rgb(_plan(plan)._h, zp, zplane, out.data_ptr(), out.stride(0), H, W, _stream(stream)))
     return out
 
 

@@ -1,5 +1,5 @@
-// color.cu -- host side of the colour entry point (b200dct_roundtrip_rgb) and of the coded-size /
-// compression-factor kernel (b200dct_zigzag_coded_bits).  See rgb_kernels.cuh for the arithmetic.
+// color.cu -- host side of the colour entry points (b200dct_roundtrip_rgb, b200dct_forward_rgb,
+// b200dct_inverse_rgb) and of the coded-size / compression-factor kernel (b200dct_zigzag_coded_bits).  See rgb_kernels.cuh for the arithmetic.
 #include <cuda_runtime.h>
 #include <string.h>
 
@@ -7,40 +7,110 @@
 
 using namespace b200dct;
 
-// ctas_per_sm != NULL: no launch, only the occupancy of the kernel the arguments select
-template <int QK, bool FINV, bool ZZ>
-static cudaError_t launch_rgb3(const RgbParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm)
+// ctas_per_sm != NULL: no launch, only the occupancy of kernel k (`occupancy`: the caller's cache of it)
+static cudaError_t launch_rgb_kernel(void (*k)(RgbParams), int &occupancy, const RgbParams &P, dim3 grid, cudaStream_t s,
+                                     bool pdl, int *ctas_per_sm)
 {
     if (ctas_per_sm) {
-        static int cached = -1;
-        if (cached < 0) {
+        if (occupancy < 0) {
             int n = 0;
-            cached = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_rgb<QK, FINV, ZZ>, 128, 0) == cudaSuccess ? n : 0;
+            occupancy = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k, 128, 0) == cudaSuccess ? n : 0;
         }
-        *ctas_per_sm = cached;
+        *ctas_per_sm = occupancy;
         return cudaSuccess;
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
-    cfg.blockDim = block;
+    cfg.blockDim = dim3(32, 4);
     cfg.stream = s;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, k_rgb<QK, FINV, ZZ>, P);
+    return cudaLaunchKernelEx(&cfg, k, P);
 }
-template <int QK, bool FINV>
-static cudaError_t launch_rgb(const RgbParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm = nullptr)
+using RgbLauncher = cudaError_t (*)(const RgbParams &, dim3, cudaStream_t, bool, int *);
+template <int QK, bool FINV, bool ZZ>
+static cudaError_t launch_rgb3(const RgbParams &P, dim3 grid, cudaStream_t s, bool pdl, int *ctas_per_sm)
 {
-    return P.zz ? launch_rgb3<QK, FINV, true>(P, grid, block, s, pdl, ctas_per_sm) : launch_rgb3<QK, FINV, false>(P, grid, block, s, pdl, ctas_per_sm);
+    static int occupancy = -1;
+    return launch_rgb_kernel(k_rgb<QK, FINV, ZZ>, occupancy, P, grid, s, pdl, ctas_per_sm);
 }
-static cudaError_t launch_rgb_any(int qk, bool finv, const RgbParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm = nullptr)
+template <int QK>
+static cudaError_t launch_rgb_forward(const RgbParams &P, dim3 grid, cudaStream_t s, bool pdl, int *ctas_per_sm)
 {
-    if (qk == 0) return finv ? launch_rgb<0, true>(P, grid, block, s, pdl, ctas_per_sm) : launch_rgb<0, false>(P, grid, block, s, pdl, ctas_per_sm);
-    if (qk == 1) return finv ? launch_rgb<1, true>(P, grid, block, s, pdl, ctas_per_sm) : launch_rgb<1, false>(P, grid, block, s, pdl, ctas_per_sm);
-    return finv ? launch_rgb<2, true>(P, grid, block, s, pdl, ctas_per_sm) : launch_rgb<2, false>(P, grid, block, s, pdl, ctas_per_sm);
+    static int occupancy = -1;
+    return launch_rgb_kernel(k_rgb_forward<QK>, occupancy, P, grid, s, pdl, ctas_per_sm);
+}
+template <bool FINV>
+static cudaError_t launch_rgb_inverse(const RgbParams &P, dim3 grid, cudaStream_t s, bool pdl, int *ctas_per_sm)
+{
+    static int occupancy = -1;
+    return launch_rgb_kernel(k_rgb_inverse<FINV>, occupancy, P, grid, s, pdl, ctas_per_sm);
+}
+
+// The argument rules of the colour entry points and the parameters their kernels share.  rgb_in / rgb_out: the pixel
+// planes the call has (NULL where it has none), interleaved RGB with 8-byte aligned rows; zz: the three streams
+// (NULL: none), 16-byte aligned, planes >= (H/8)*(W/8)*128 bytes apart.
+static int rgb_params(const b200dct_plan *plan, const void *rgb_in, size_t in_pitch, void *rgb_out, size_t out_pitch,
+                      void *zz, size_t zz_plane_bytes, int H, int W, RgbParams &P, dim3 &grid)
+{
+    if (H <= 0 || W <= 0 || (H % 8) || (W % 8)) return B200DCT_ERR_SHAPE;
+    if ((rgb_in && in_pitch < (size_t)W * 3) || (rgb_out && out_pitch < (size_t)W * 3)) return B200DCT_ERR_SHAPE;
+    if (((uintptr_t)rgb_in & 7) || ((uintptr_t)rgb_out & 7) || (in_pitch & 7) || (out_pitch & 7)) return B200DCT_ERR_ALIGN;
+    if (!plan->sparse) return B200DCT_ERR_ARG; // the colour path is built for Haweel's T (the reference's HpApprDCT)
+    const size_t zz_bytes = (size_t)(H / 8) * (size_t)(W / 8) * 128;
+    if (zz && (((uintptr_t)zz & 15) || (zz_plane_bytes & 15) || zz_plane_bytes < zz_bytes)) return B200DCT_ERR_ALIGN;
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess) return B200DCT_ERR_NODEVICE;
+
+    memset(&P, 0, sizeof(P));
+    P.in = rgb_in; P.in_pitch = in_pitch;
+    P.out = rgb_out; P.out_pitch = out_pitch;
+    P.zz = zz; P.zz_plane = zz_plane_bytes; P.zz_pitch = (size_t)(W / 8) * 128;
+    P.bx = W / 8; P.by = H / 8;
+    for (int k = 0; k < 64; k++) {
+        P.t[0].rd[k] = make_float2(plan->cp.q.rcp[k], plan->cp.q.d[k]);
+        P.t[0].keep[k] = plan->cp.q.keep[k];
+        P.t[1].rd[k] = make_float2(plan->qc.rcp[k], plan->qc.d[k]);
+        P.t[1].keep[k] = plan->qc.keep[k];
+    }
+    grid = dim3((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32));
+    if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
+    return B200DCT_OK;
+}
+static Span rgb_span(const void *p, size_t pitch, int H, int W) { return Span{p, pitch, (size_t)W * 3, H}; }
+static Span zz_span(const void *zz, size_t plane_bytes, int H, int W) { return Span{zz, plane_bytes, (size_t)(H / 8) * (size_t)(W / 8) * 128, 3}; }
+// quantiser variant of the forward transform: 0 all coefficients kept, exact fast division; 1 mask + exact fast
+// division; 2 mask + __fdiv_rn
+static int rgb_qk(const b200dct_plan *plan)
+{
+    return (!plan->q_fastdiv || !plan->qc_fastdiv) ? 2 : (plan->mask == ~(uint64_t)0 ? 0 : 1);
+}
+// One launch of a colour kernel.  Early path across launch boundaries (b200dct.cu, "early loads"): a pass whose
+// input `rd` is not written by the library's previous machine-filling launch on this stream reads and computes
+// before it waits (rd.ptr NULL: never); w0 / w1 are what the launch writes.
+static int run_rgb(RgbLauncher launch, RgbParams &P, dim3 grid, cudaStream_t s, Span rd, Span w0, Span w1)
+{
+    const bool pdl = pdl_enabled(s);
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    const bool capturing = cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
+    int per_sm = 0;
+    if (pdl && !capturing) launch(P, grid, s, pdl, &per_sm);
+    cudaError_t e;
+    {
+        EarlyScope scope(s, pdl && !capturing, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1);
+        P.early = scope.params().early;
+        P.chain_feed = scope.params().chain_feed;
+        P.chain = scope.params().chain;
+        P.chain_target = scope.params().chain_target;
+        e = launch(P, grid, s, pdl, nullptr);
+        scope.done(e == cudaSuccess);
+    }
+    if (e != cudaSuccess) return (int)e;
+    note_launch(1, "rgb");
+    return B200DCT_OK;
 }
 
 extern "C" int b200dct_roundtrip_rgb(const b200dct_plan *plan, const void *rgb, size_t in_pitch, void *out,
@@ -49,55 +119,46 @@ extern "C" int b200dct_roundtrip_rgb(const b200dct_plan *plan, const void *rgb, 
 {
     note_launch(0, "none");
     if (!plan || !rgb || !out) return B200DCT_ERR_ARG;
-    if (H <= 0 || W <= 0 || (H % 8) || (W % 8)) return B200DCT_ERR_SHAPE;
-    if (in_pitch < (size_t)W * 3 || out_pitch < (size_t)W * 3) return B200DCT_ERR_SHAPE;
-    if (((uintptr_t)rgb & 7) || ((uintptr_t)out & 7) || (in_pitch & 7) || (out_pitch & 7)) return B200DCT_ERR_ALIGN;
-    if (!plan->sparse) return B200DCT_ERR_ARG; // the colour path is built for Haweel's T (the reference's HpApprDCT)
-    const size_t zz_bytes = (size_t)(H / 8) * (size_t)(W / 8) * 128;
-    if (zz3_or_null && (((uintptr_t)zz3_or_null & 15) || (zz_plane_bytes & 15) || zz_plane_bytes < zz_bytes)) return B200DCT_ERR_ALIGN;
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess) return B200DCT_ERR_NODEVICE;
-
     RgbParams P;
-    memset(&P, 0, sizeof(P));
-    P.in = rgb; P.in_pitch = in_pitch;
-    P.out = out; P.out_pitch = out_pitch;
-    P.zz = zz3_or_null; P.zz_plane = zz_plane_bytes; P.zz_pitch = (size_t)(W / 8) * 128;
-    P.bx = W / 8; P.by = H / 8;
-    for (int k = 0; k < 64; k++) {
-        P.t[0].rd[k] = make_float2(plan->cp.q.rcp[k], plan->cp.q.d[k]);
-        P.t[0].keep[k] = plan->cp.q.keep[k];
-        P.t[1].rd[k] = make_float2(plan->qc.rcp[k], plan->qc.d[k]);
-        P.t[1].keep[k] = plan->qc.keep[k];
-    }
-    dim3 block(32, 4), grid((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32));
-    if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
-    cudaStream_t s = (cudaStream_t)stream;
-    const bool pdl = pdl_enabled(s);
-    const bool finv = use_factored_inverse_u8(plan);
-    const int qk = (!plan->q_fastdiv || !plan->qc_fastdiv) ? 2 : (plan->mask == ~(uint64_t)0 ? 0 : 1);
-    // early path across launch boundaries (b200dct.cu, "early loads"): a pass whose input is not written by the
-    // library's previous machine-filling launch on this stream converts and transforms before it waits
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    const bool capturing = cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
-    int per_sm = 0;
-    if (pdl && !capturing) launch_rgb_any(qk, finv, P, grid, block, s, pdl, &per_sm);
-    cudaError_t e;
-    {
-        const Span rd{zz3_or_null ? nullptr : rgb, in_pitch, (size_t)W * 3, H};
-        const Span w0{out, out_pitch, (size_t)W * 3, H};
-        const Span w1{zz3_or_null, zz_plane_bytes, zz_bytes, 3};
-        EarlyScope scope(s, pdl && !capturing, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1);
-        P.early = scope.params().early;
-        P.chain_feed = scope.params().chain_feed;
-        P.chain = scope.params().chain;
-        P.chain_target = scope.params().chain_target;
-        e = launch_rgb_any(qk, finv, P, grid, block, s, pdl);
-        scope.done(e == cudaSuccess);
-    }
-    if (e != cudaSuccess) return (int)e;
-    note_launch(1, "rgb");
-    return B200DCT_OK;
+    dim3 grid;
+    const int rc = rgb_params(plan, rgb, in_pitch, out, out_pitch, zz3_or_null, zz_plane_bytes, H, W, P, grid);
+    if (rc != B200DCT_OK) return rc;
+    static const RgbLauncher launchers[3][2][2] = {
+        {{launch_rgb3<0, false, false>, launch_rgb3<0, false, true>}, {launch_rgb3<0, true, false>, launch_rgb3<0, true, true>}},
+        {{launch_rgb3<1, false, false>, launch_rgb3<1, false, true>}, {launch_rgb3<1, true, false>, launch_rgb3<1, true, true>}},
+        {{launch_rgb3<2, false, false>, launch_rgb3<2, false, true>}, {launch_rgb3<2, true, false>, launch_rgb3<2, true, true>}}};
+    // with streams every CTA writes mid-kernel, so that kernel never takes the early path
+    return run_rgb(launchers[rgb_qk(plan)][use_factored_inverse_u8(plan)][zz3_or_null != nullptr], P, grid, (cudaStream_t)stream,
+                   rgb_span(zz3_or_null ? nullptr : rgb, in_pitch, H, W), rgb_span(out, out_pitch, H, W),
+                   zz_span(zz3_or_null, zz_plane_bytes, H, W));
+}
+
+extern "C" int b200dct_forward_rgb(const b200dct_plan *plan, const void *rgb, size_t in_pitch, void *zz3,
+                                   size_t zz_plane_bytes, int H, int W, void *stream)
+{
+    note_launch(0, "none");
+    if (!plan || !rgb || !zz3) return B200DCT_ERR_ARG;
+    RgbParams P;
+    dim3 grid;
+    const int rc = rgb_params(plan, rgb, in_pitch, nullptr, 0, zz3, zz_plane_bytes, H, W, P, grid);
+    if (rc != B200DCT_OK) return rc;
+    static const RgbLauncher launchers[3] = {launch_rgb_forward<0>, launch_rgb_forward<1>, launch_rgb_forward<2>};
+    return run_rgb(launchers[rgb_qk(plan)], P, grid, (cudaStream_t)stream, rgb_span(rgb, in_pitch, H, W),
+                   zz_span(zz3, zz_plane_bytes, H, W), Span{nullptr, 0, 0, 0});
+}
+
+extern "C" int b200dct_inverse_rgb(const b200dct_plan *plan, const void *zz3, size_t zz_plane_bytes, void *out,
+                                   size_t out_pitch, int H, int W, void *stream)
+{
+    note_launch(0, "none");
+    if (!plan || !zz3 || !out) return B200DCT_ERR_ARG;
+    RgbParams P;
+    dim3 grid;
+    const int rc = rgb_params(plan, nullptr, 0, out, out_pitch, const_cast<void *>(zz3), zz_plane_bytes, H, W, P, grid);
+    if (rc != B200DCT_OK) return rc;
+    static const RgbLauncher launchers[2] = {launch_rgb_inverse<false>, launch_rgb_inverse<true>};
+    return run_rgb(launchers[use_factored_inverse_u8(plan)], P, grid, (cudaStream_t)stream, zz_span(zz3, zz_plane_bytes, H, W),
+                   rgb_span(out, out_pitch, H, W), Span{nullptr, 0, 0, 0});
 }
 
 // ------------------------------------------------------------------ coded size of a coefficient stream

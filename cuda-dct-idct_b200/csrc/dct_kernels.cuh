@@ -247,6 +247,10 @@ __device__ __forceinline__ void ld_block_zigzag(const void *base, float2 (&c)[8]
 {
     sfor<8>([&](auto g) { zigzag_unchunk<IC(g)>(__ldg(reinterpret_cast<const uint4 *>(base) + IC(g)), c); });
 }
+__device__ __forceinline__ void ld_block_zigzag_cg(const void *base, float2 (&c)[8][4]) // L2 only: never a stale L1 line
+{
+    sfor<8>([&](auto g) { zigzag_unchunk<IC(g)>(__ldcg(reinterpret_cast<const uint4 *>(base) + IC(g)), c); });
+}
 // Cooperative access for a full warp (32 adjacent blocks = one contiguous 4 KiB span): the span
 // is transposed through a 4 KiB shared-memory buffer so that every global instruction moves 512
 // contiguous bytes.  Chunk c of block b lives at b*128 + ((c ^ (b & 7)) * 16): both the per-block

@@ -25,6 +25,10 @@
  *   convertToFloat / convertToUnsignedChar utils.cu:10-24  dtype B200DCT_U8 on either side
  *   cudaMalloc/cudaMemcpy around the calls, main_newAppr.cu:88-95,103,124
  *                                                          b200dct_roundtrip_host
+ *   the same two calls on a colour image (RGB, utils.cu:62-64)
+ *     dct_all_blocks_cuda per Y/Cb/Cr plane                b200dct_forward_rgb  (RGB -> 3 zig-zag streams)
+ *     idct_all_blocks_cuda per Y/Cb/Cr plane               b200dct_inverse_rgb  (3 zig-zag streams -> RGB)
+ *     both, one fused pass                                 b200dct_roundtrip_rgb
  *
  * Conventions: images are single-channel, row-major; H and W are multiples of 8 (the
  * reference silently computes garbage otherwise, main_newAppr.cu:261-262; here it is an
@@ -48,7 +52,7 @@
 extern "C" {
 #endif
 
-#define B200DCT_VERSION 100
+#define B200DCT_VERSION 101 /* 101: b200dct_forward_rgb / b200dct_inverse_rgb */
 
 typedef enum b200dct_dtype {
     B200DCT_F32 = 0, /* float pixels / integer-valued float coefficients (the reference's type) */
@@ -249,6 +253,22 @@ int b200dct_plan_get_chroma_quant(const b200dct_plan *plan, float q[64]);
 int b200dct_roundtrip_rgb(const b200dct_plan *plan, const void *rgb, size_t in_pitch,
                           void *out, size_t out_pitch, void *zz3_or_null, size_t zz_plane_bytes,
                           int H, int W, void *stream);
+/* The two halves of b200dct_roundtrip_rgb, split at the coefficient streams, for callers that store
+ * or send the compact coefficients, size them (b200dct_zigzag_coded_bits) or change them before
+ * decoding -- what the reference's caller can do between its two calls (main_newAppr.cu:103).
+ * Arguments, stream layout and error codes as b200dct_roundtrip_rgb; zz3 is required.  One launch
+ * each (b200dct_last_path() "rgb"), legal under stream capture.  b200dct_inverse_rgb of the streams
+ * b200dct_forward_rgb wrote gives b200dct_roundtrip_rgb's pixels bit for bit, in either inverse mode,
+ * as long as no stream value saturates (never for Q entries >= 1/16).
+ * RGB -> YCbCr (libjpeg jccolor.c) -> per plane convertToFloat, dct, quantise (luminance Q for Y,
+ * chrominance Q for Cb/Cr, plan's keep mask) -> three block-major zig-zag int16 streams
+ * (B200DCT_I16_ZIGZAG layout, block-row pitch (W/8)*128, planes zz_plane_bytes apart). */
+int b200dct_forward_rgb(const b200dct_plan *plan, const void *rgb, size_t in_pitch,
+                        void *zz3, size_t zz_plane_bytes, int H, int W, void *stream);
+/* three zig-zag streams -> per plane dequantise, idct, convertToUnsignedChar (plan's inverse mode)
+ * -> YCbCr -> RGB (libjpeg jdcolor.c). */
+int b200dct_inverse_rgb(const b200dct_plan *plan, const void *zz3, size_t zz_plane_bytes,
+                        void *out, size_t out_pitch, int H, int W, void *stream);
 
 /* Size in BITS of the baseline-JPEG entropy-coded scan (ITU-T T.81 sequential Huffman with the
  * Annex K.3 tables, i.e. what libjpeg writes with optimize off; no headers, stuffing or padding)
