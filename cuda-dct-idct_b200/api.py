@@ -518,22 +518,33 @@ def inverse_rgb(streams, out=None, plan: Plan | None = None, stream=None):
     return out
 
 
+CODED_OUT_OF_RANGE = 1 << 63   # B200DCT_CODED_OUT_OF_RANGE: the stream holds a symbol baseline JPEG cannot code
+
+
 def coded_bits(zz, table: int = 0, stream=None) -> int:
     """Baseline-JPEG entropy-coded size in bits of one plane's zig-zag stream, an (H/8, W/8, 64)
-    int16 CUDA tensor (b200dct_zigzag_coded_bits); table 0 = luminance codes, 1 = chrominance."""
+    int16 CUDA tensor (b200dct_zigzag_coded_bits); table 0 = luminance codes, 1 = chrominance.
+    Baseline JPEG codes DC differences up to 2047 and AC values up to 1023 in magnitude; a stream with
+    any other value (quantiser entries below 1 produce them) has no baseline size and raises
+    B200DCTError."""
     import torch
 
     p, _, pitch, H, W = _zz_plane(zz)
     with _on(zz, stream):
         acc = torch.zeros(1, dtype=torch.int64, device=zz.device)
         _check(lib().b200dct_zigzag_coded_bits(p, pitch, H, W, int(table), acc.data_ptr(), _stream(stream)))
-        return int(acc.item())
+        bits = int(acc.item()) & ((1 << 64) - 1)
+    if bits & CODED_OUT_OF_RANGE:
+        raise B200DCTError("the stream holds a DC difference beyond +-2047 or an AC value beyond +-1023, which baseline "
+                           "JPEG cannot code (a quantiser entry below 1?): it has no baseline coded size")
+    return bits
 
 
 def compression_factor(zz, table: int = 0, stream=None) -> float:
     """8*H*W / coded_bits: the README's 'Compr. Factor' (README.md:62-69) under the baseline-JPEG
     entropy coder.  `zz`: one plane's stream, or a (3, ...) stack (Y with the luminance codes,
-    Cb and Cr with the chrominance codes; CF of the whole colour image)."""
+    Cb and Cr with the chrominance codes; CF of the whole colour image).  Raises B200DCTError for a
+    stream that baseline JPEG cannot code (see coded_bits)."""
     if zz.dim() == 4:
         bits = sum(coded_bits(zz[c], 0 if c == 0 else 1, stream) for c in range(zz.shape[0]))
         return 8.0 * zz.shape[0] * zz.shape[1] * zz.shape[2] * 64 / bits
@@ -543,7 +554,10 @@ def compression_factor(zz, table: int = 0, stream=None) -> float:
 def roundtrip_with_metrics(img, out=None, coef=None, plan: Plan | None = None, stream=None, zigzag=False):
     """Fused round trip that also returns (MSE, PEEN%, non-zero coefficient count) of the
     pass, computed inside the kernel (b200dct_roundtrip_metrics).  zigzag=True: `coef` is the
-    block-major int16 zig-zag stream."""
+    block-major int16 zig-zag stream.  u8 metrics are exact; f32 metrics add every block's f32 sums
+    as 128-bit fixed point (units of 2^-50): the same bits run to run and on either kernel family,
+    within 1e-6 relative of a float64 sum for pixels of magnitude 2^-10 .. 2^20.  An int16 or zig-zag
+    `coef` saturates to [-32768, 32767]; the pixels come from the unsaturated coefficients."""
     import torch
 
     ip, idt, ipitch, H, W = _plane(img)

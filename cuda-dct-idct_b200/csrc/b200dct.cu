@@ -87,13 +87,11 @@ static __global__ void __launch_bounds__(REDUCE_THREADS) k_reduce_partials(const
     if (threadIdx.x < 3) acc[threadIdx.x] += red[threadIdx.x][0];
 }
 
-// TMA-family metrics: the kernel leaves exact integer sums (2^-12 fixed point) in macc[0..2]
-static __global__ void k_finish_fixed_point(unsigned long long *macc, double *acc)
+// TMA-family metrics: the kernel leaves exact integer sums in macc[0..MACC_WORDS) (128-bit fixed point, dct_kernels.cuh)
+static __global__ void k_finish_fixed_point(const unsigned long long *macc, double *acc)
 {
-    if (threadIdx.x < 3) {
-        const double v = (double)(long long)macc[threadIdx.x];
-        acc[threadIdx.x] += threadIdx.x < 2 ? v / (double)METRICS_FIXED_POINT : v;
-    }
+    if (threadIdx.x < 2) acc[threadIdx.x] += u128_to_double(macc[2 * threadIdx.x], macc[2 * threadIdx.x + 1]) / METRICS_FIXED_POINT;
+    if (threadIdx.x == 2) acc[2] += (double)macc[4];
 }
 
 static cudaError_t reduce_partials_sparse(const double *partials, size_t n, double *acc, cudaStream_t s)
@@ -413,7 +411,7 @@ constexpr int SCHED_SLOTS = 4096;
 constexpr int CAPTURE_SLOTS = 4096;
 struct SchedRing {
     uint32_t *base[64] = {};
-    unsigned long long *macc[64] = {}; // one zeroed {sse, energy, nnz} integer triple per slot (metrics kernels)
+    unsigned long long *macc[64] = {}; // one zeroed MACC_WORDS accumulator per slot (metrics kernels)
     unsigned next[64] = {};
     unsigned next_capture[64] = {};
     std::mutex mu;
@@ -429,7 +427,7 @@ uint32_t *sched_slot(bool capturing)
         if (capturing) return nullptr;
         uint32_t *p = nullptr;
         const size_t nslots = (size_t)(SCHED_SLOTS + CAPTURE_SLOTS);
-        const size_t bytes = nslots * 2 * sizeof(uint32_t) + nslots * 3 * sizeof(unsigned long long);
+        const size_t bytes = nslots * 2 * sizeof(uint32_t) + nslots * MACC_WORDS * sizeof(unsigned long long);
         if (cudaMalloc(&p, bytes) != cudaSuccess) return nullptr;
         if (cudaMemset(p, 0, bytes) != cudaSuccess) { cudaFree(p); return nullptr; }
         g_sched.base[dev] = p;
@@ -447,7 +445,7 @@ unsigned long long *sched_macc(const uint32_t *slot)
 {
     int dev = -1;
     if (!slot || cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64 || !g_sched.base[dev]) return nullptr;
-    return g_sched.macc[dev] + 3 * ((slot - g_sched.base[dev]) / 2);
+    return g_sched.macc[dev] + MACC_WORDS * ((slot - g_sched.base[dev]) / 2);
 }
 } // namespace
 
@@ -818,8 +816,8 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
         P.run = (uint32_t)tma_max_run;
         const unsigned long long tail = 2ull * (unsigned long long)grid * nw;
         P.run_tickets = nt > tail ? (uint32_t)((nt - tail) / P.run) : 0u;
-        // Metrics: with the dynamic scheduler the slot owns a zeroed integer triple and the last warp out
-        // folds it into acc -- one launch.  Static split: the first 24 bytes of the caller's workspace,
+        // Metrics: with the dynamic scheduler the slot owns a zeroed integer accumulator and the last warp out
+        // folds it into acc -- one launch.  Static split: the first MACC_WORDS words of the caller's workspace,
         // zeroed before and folded after the kernel.
         std::unique_lock<std::mutex> launch_order(g_last_mu); // held until this kernel is in the stream
         const Range rd = plane_range(in.ptr, in.pitch, (size_t)W * elem_size(in.dt), H);
@@ -843,7 +841,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
                 separate_finish = true;
                 P.acc = nullptr;
                 P.macc = reinterpret_cast<unsigned long long *>(partials);
-                const cudaError_t em = cudaMemsetAsync(P.macc, 0, 3 * sizeof(unsigned long long), stream);
+                const cudaError_t em = cudaMemsetAsync(P.macc, 0, MACC_WORDS * sizeof(unsigned long long), stream);
                 if (em != cudaSuccess) return (int)em;
             }
         }
@@ -912,7 +910,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
             P.macc = macc;
             P.mdone = slot;
             P.acc = acc;
-            P.metrics_scale = pix == DT_U8 ? 1.0f : METRICS_FIXED_POINT;
+            P.metrics_scale = pix == DT_U8 ? 1.0 : METRICS_FIXED_POINT;
             e = launch_direct_metrics(pl->tk, qm, pix, finv, P, grid, block, stream, pdl);
             if (e == cudaSuccess) commit_launch_locked(ticket, false, feeds, (unsigned long long)P.chain_feed, w0, w1, w2);
             if (e != cudaSuccess) return (int)e;
@@ -1117,7 +1115,9 @@ extern "C" size_t b200dct_metrics_workspace_bytes(int H, int W)
 {
     if (H <= 0 || W <= 0) return 0;
     const size_t ctas = (size_t)((H / 8 + 3) / 4) * (size_t)((W / 8 + 31) / 32);
-    return ctas * 3 * sizeof(double);
+    // per-CTA partials of the direct family, or the TMA family's integer accumulator
+    const size_t partials = ctas * 3 * sizeof(double), fixed = MACC_WORDS * sizeof(unsigned long long);
+    return partials > fixed ? partials : fixed;
 }
 
 extern "C" int b200dct_roundtrip_metrics(const b200dct_plan *plan, const void *img, b200dct_dtype in_dt, size_t in_pitch,

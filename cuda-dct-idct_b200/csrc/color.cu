@@ -238,6 +238,7 @@ static __global__ void __launch_bounds__(256) k_coded_bits(const __grid_constant
     __syncthreads();
     const long long nblk = (long long)P.bx * P.by;
     unsigned bits = 0;
+    bool out_of_range = false;
     for (long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x; b < nblk; b += (long long)gridDim.x * blockDim.x) {
         const long long r = b / P.bx;
         const int c = (int)(b - r * P.bx);
@@ -250,6 +251,8 @@ static __global__ void __launch_bounds__(256) k_coded_bits(const __grid_constant
             prev = *reinterpret_cast<const short *>((const char *)P.zz + (size_t)pr * P.pitch + (size_t)pc * 128);
         }
         int run = 0;
+        // baseline JPEG codes DC-difference categories 0..11 and AC categories 1..10 only: a symbol outside them has no
+        // code, counts 0 bits and sets the flag (bit 63 of *P.bits); no table is indexed with it
 #pragma unroll
         for (int g = 0; g < 8; g++) {
             const uint4 w = __ldg(blk + g);
@@ -259,13 +262,15 @@ static __global__ void __launch_bounds__(256) k_coded_bits(const __grid_constant
                 const int v = (int)(short)(ws[k >> 1] >> (16 * (k & 1)));
                 if (g == 0 && k == 0) {
                     const int s = bit_size(v - prev);
-                    bits += dcl[s] + s;
+                    if (s <= 11) bits += dcl[s] + s;
+                    else out_of_range = true;
                 } else if (v == 0) {
                     run++;
                 } else {
                     while (run > 15) { bits += acl[0xf0]; run -= 16; }
                     const int s = bit_size(v);
-                    bits += acl[(run << 4) | s] + s;
+                    if (s <= 10) bits += acl[(run << 4) | s] + s;
+                    else out_of_range = true;
                     run = 0;
                 }
             }
@@ -277,6 +282,7 @@ static __global__ void __launch_bounds__(256) k_coded_bits(const __grid_constant
     if ((threadIdx.x & 31) == 0 && v) atomicAdd(&cta_bits, v);
     __syncthreads();
     if (threadIdx.x == 0 && cta_bits) atomicAdd(P.bits, cta_bits); // integer sums: order does not matter
+    if (__any_sync(0xffffffffu, out_of_range) && (threadIdx.x & 31) == 0) atomicOr(P.bits, B200DCT_CODED_OUT_OF_RANGE);
 }
 
 extern "C" int b200dct_zigzag_coded_bits(const void *zz, size_t pitch, int H, int W, int table,

@@ -98,7 +98,53 @@ __device__ __forceinline__ unsigned long long ld_counter(const unsigned long lon
     asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
     return v;
 }
-constexpr float METRICS_FIXED_POINT = 4096.0f; // f32 metrics: per-block sums are accumulated as integers in units of 2^-12
+// f32 metrics: every block's float sums are converted EXACTLY to unsigned 128-bit fixed point in units of 2^-50 and
+// accumulated as integers (order-independent => deterministic).  The floor: a block sum rounds to a multiple of
+// 2^-50; the ceiling: totals below 2^78 (2^22 blocks of 64 pixels of magnitude 2^20 sum to 2^68).
+constexpr double METRICS_FIXED_POINT = 0x1p50;
+// One metrics accumulator: {sse lo, sse hi, energy lo, energy hi, non-zero count} (64-bit words)
+constexpr int MACC_WORDS = 5;
+struct U128 {
+    unsigned long long lo, hi;
+};
+__device__ __forceinline__ U128 u128_add(U128 a, U128 b)
+{
+    U128 r;
+    r.lo = a.lo + b.lo;
+    r.hi = a.hi + b.hi + (r.lo < a.lo ? 1ull : 0ull);
+    return r;
+}
+__device__ __forceinline__ U128 u128_shfl_xor(U128 a, int o)
+{
+    return U128{__shfl_xor_sync(0xffffffffu, a.lo, o), __shfl_xor_sync(0xffffffffu, a.hi, o)};
+}
+// a non-negative finite f32 block sum s -> round(s * 2^50) as 128 bits: s * 2^50 is exact in double, its part above
+// 2^64 truncates exactly, the remainder is below 2^64 and holds at most 24 significant bits
+__device__ __forceinline__ U128 metrics_fixed(float s)
+{
+    const double d = (double)s * METRICS_FIXED_POINT;
+    const unsigned long long hi = __double2ull_rz(d * 0x1p-64);
+    return U128{__double2ull_rn(__fma_rn(-(double)hi, 0x1p64, d)), hi};
+}
+// adds v to the 128-bit slot {lo, hi} with two 64-bit atomics; the carry out of lo comes from the returned old value,
+// so the final pair is the exact sum whatever order the atomics land in
+__device__ __forceinline__ void atomic_add_u128(unsigned long long *slot, U128 v)
+{
+    const unsigned long long old = atomicAdd(&slot[0], v.lo);
+    const unsigned long long hi = v.hi + (old + v.lo < old ? 1ull : 0ull);
+    if (hi) atomicAdd(&slot[1], hi);
+}
+// CTA reductions of the metrics kernels: u8 sums stay 64-bit (exact integers far below 2^64), f32 sums are U128
+__device__ __forceinline__ unsigned long long acc_add(unsigned long long a, unsigned long long b) { return a + b; }
+__device__ __forceinline__ U128 acc_add(U128 a, U128 b) { return u128_add(a, b); }
+__device__ __forceinline__ unsigned long long acc_shfl_xor(unsigned long long a, int o) { return __shfl_xor_sync(0xffffffffu, a, o); }
+__device__ __forceinline__ U128 acc_shfl_xor(U128 a, int o) { return u128_shfl_xor(a, o); }
+__device__ __forceinline__ U128 acc_wide(unsigned long long a) { return U128{a, 0}; }
+__device__ __forceinline__ U128 acc_wide(U128 a) { return a; }
+__host__ __device__ __forceinline__ double u128_to_double(unsigned long long lo, unsigned long long hi)
+{
+    return (double)hi * 0x1p64 + (double)lo;
+}
 constexpr int DIRECT_BATCH_MAX = 64; // images per launch of the batch entry point (1 KiB of kernel parameters)
 struct DirectParams {
     const void *in;   // FWD/RT: pixels (PIX dtype); INV: coefficients (coef_dt)
@@ -110,13 +156,13 @@ struct DirectParams {
     int coef_dt;      // DT_F32 / DT_I16
     double *partials; // METRICS kernels, two-launch form: 3 doubles per CTA {sum (x-y)^2, sum x^2, non-zero coefficients}
     // METRICS kernels, one-launch form (macc != NULL): every CTA adds its integer sums {sum (x-y)^2, sum x^2} (u8: exact
-    // integers; f32: per-block float sums in units of 2^-12, the TMA family's convention) and its non-zero count to
-    // macc[0..2] with 64-bit atomics (order-independent => deterministic); the last CTA out (mdone[1] counts them) adds
-    // the totals, divided by metrics_scale, into acc[0..2] and leaves macc and the counter zeroed
+    // integers; f32: per-block float sums as 128-bit fixed point in units of 2^-50, the TMA family's convention) and its
+    // non-zero count to macc[0..MACC_WORDS) with 64-bit atomics (order-independent => deterministic); the last CTA out
+    // (mdone[1] counts them) adds the totals, divided by metrics_scale, into acc[0..2] and leaves macc and the counter zeroed
     unsigned long long *macc;
     uint32_t *mdone;
     double *acc;
-    float metrics_scale;
+    double metrics_scale;
     int zz_smem;      // 1: the launch carries ZZ_SMEM_BYTES of dynamic shared memory for the zig-zag stream transpose
     // batch of separately allocated images of one shape (b200dct_roundtrip_batch): image z of the launch
     // is blockIdx.z, its planes come from these tables instead of in / out (pixels only: no coefficient
@@ -446,36 +492,46 @@ __global__ void __launch_bounds__(128, METRICS ? B200DCT_METRICS_MIN_BLOCKS : B2
         atomicAdd(P.chain, 1ull); // one of the last CTAs of the grid is (as good as) done
     if constexpr (METRICS) {
         if (P.macc) { // one-launch form
-            long long v[3] = {0, 0, 0};
+            using Acc = std::conditional_t<PIX == DT_U8, unsigned long long, U128>;
+            Acc v[2] = {Acc{}, Acc{}};
+            unsigned long long nz = 0;
             if (valid) {
                 if constexpr (PIX == DT_U8) {
-                    v[0] = (long long)(i_xx + i_yy - 2u * i_xy);
-                    v[1] = (long long)i_xx;
+                    v[0] = i_xx + i_yy - 2u * i_xy;
+                    v[1] = i_xx;
                 } else {
-                    v[0] = __float2ll_rn(m_sse * METRICS_FIXED_POINT);
-                    v[1] = __float2ll_rn(m_en * METRICS_FIXED_POINT);
+                    v[0] = metrics_fixed(m_sse);
+                    v[1] = metrics_fixed(m_en);
                 }
-                v[2] = (long long)m_nnz;
+                nz = (unsigned long long)m_nnz;
             }
-            __shared__ long long ired[3][4];
+            __shared__ Acc ired[2][4];
+            __shared__ unsigned long long inz[4];
             const int lane = threadIdx.x, w = threadIdx.y;
-            sfor<3>([&](auto q) {
-                for (int o = 16; o > 0; o >>= 1) v[IC(q)] += __shfl_xor_sync(0xffffffffu, v[IC(q)], o);
-                if (lane == 0) ired[IC(q)][w] = v[IC(q)];
-            });
+            for (int o = 16; o > 0; o >>= 1) {
+                v[0] = acc_add(v[0], acc_shfl_xor(v[0], o));
+                v[1] = acc_add(v[1], acc_shfl_xor(v[1], o));
+                nz += __shfl_xor_sync(0xffffffffu, nz, o);
+            }
+            if (lane == 0) {
+                ired[0][w] = v[0];
+                ired[1][w] = v[1];
+                inz[w] = nz;
+            }
             __syncthreads();
             if (w == 0 && lane == 0) {
-                sfor<3>([&](auto q) {
-                    atomicAdd(&P.macc[IC(q)], (unsigned long long)((ired[IC(q)][0] + ired[IC(q)][1]) + (ired[IC(q)][2] + ired[IC(q)][3])));
+                sfor<2>([&](auto q) {
+                    atomic_add_u128(&P.macc[2 * IC(q)], acc_wide(acc_add(acc_add(ired[IC(q)][0], ired[IC(q)][1]), acc_add(ired[IC(q)][2], ired[IC(q)][3]))));
                 });
+                atomicAdd(&P.macc[4], (inz[0] + inz[1]) + (inz[2] + inz[3]));
                 __threadfence();
                 if (atomicAdd(&P.mdone[1], 1u) == gridDim.x * gridDim.y - 1u) { // every other CTA's sums are in
                     __threadfence();
-                    const long long sse = (long long)atomicExch(&P.macc[0], 0ull), en = (long long)atomicExch(&P.macc[1], 0ull),
-                                    nnz = (long long)atomicExch(&P.macc[2], 0ull);
-                    P.acc[0] += (double)sse / (double)P.metrics_scale;
-                    P.acc[1] += (double)en / (double)P.metrics_scale;
-                    P.acc[2] += (double)nnz;
+                    unsigned long long t[MACC_WORDS];
+                    sfor<MACC_WORDS>([&](auto q) { t[IC(q)] = atomicExch(&P.macc[IC(q)], 0ull); });
+                    P.acc[0] += u128_to_double(t[0], t[1]) / P.metrics_scale;
+                    P.acc[1] += u128_to_double(t[2], t[3]) / P.metrics_scale;
+                    P.acc[2] += (double)t[4];
                     P.mdone[1] = 0;
                     __threadfence();
                 }
@@ -537,8 +593,9 @@ struct TmaParams {
     uint32_t run;         // tiles per ticket for the first run_tickets tickets, then 1
     uint32_t run_tickets;
     uint32_t buf_bytes;   // size of one tile buffer: the largest tile image among the planes of this call
-    // METRICS kernels: {sum (x-y)^2, sum x^2} in units of 2^-12 and the number of non-zero
-    // coefficients, accumulated with 64-bit integer atomics (order-independent => deterministic)
+    // METRICS kernels: {sum (x-y)^2, sum x^2} as 128-bit fixed point in units of 2^-50 and the number of
+    // non-zero coefficients (MACC_WORDS words), accumulated with 64-bit integer atomics (order-independent
+    // => deterministic)
     unsigned long long *macc;
     double *acc;          // METRICS with the dynamic scheduler: the last warp out adds macc into acc[0..2] and re-zeroes macc
     // 1: the host has established that nothing this launch READS is written by the launch it may
@@ -806,7 +863,8 @@ __global__ void B200DCT_TMA_BOUNDS k_tma(const __grid_constant__ TmaParams P)
 
     uint32_t parity = 0;   // METRICS: bit b = parity of barrier b
     uint32_t cur = 0;      // METRICS: which input buffer holds the current tile
-    long long m_sse = 0, m_en = 0, m_nnz = 0;
+    U128 m_sse = {0, 0}, m_en = {0, 0};
+    unsigned long long m_nnz = 0;
     while (tile < P.ntiles) {
         const int ty = (int)(tile / P.tiles_x), tx = (int)(tile - (uint32_t)ty * P.tiles_x);
         uint32_t next_l0 = 0;
@@ -894,11 +952,11 @@ __global__ void B200DCT_TMA_BOUNDS k_tma(const __grid_constant__ TmaParams P)
                             t_en = __fmaf_rn(x[2 * IC(j)], x[2 * IC(j)], t_en); t_en = __fmaf_rn(x[2 * IC(j) + 1], x[2 * IC(j) + 1], t_en);
                         });
                     });
-                    // per-block sums (fixed order) -> 2^-12 fixed point: integer accumulation is order-independent
+                    // per-block sums (fixed order) -> 128-bit fixed point: integer accumulation is order-independent
                     if ((uint32_t)tx * 32u + (uint32_t)lane < P.bx) {
-                        m_sse += __float2ll_rn(t_sse * METRICS_FIXED_POINT);
-                        m_en += __float2ll_rn(t_en * METRICS_FIXED_POINT);
-                        m_nnz += (long long)t_nnz;
+                        m_sse = u128_add(m_sse, metrics_fixed(t_sse));
+                        m_en = u128_add(m_en, metrics_fixed(t_en));
+                        m_nnz += (unsigned long long)t_nnz;
                     }
                 }
             } else {
@@ -918,15 +976,15 @@ __global__ void B200DCT_TMA_BOUNDS k_tma(const __grid_constant__ TmaParams P)
     }
     if constexpr (METRICS) {
         for (int o = 16; o > 0; o >>= 1) {
-            m_sse += __shfl_xor_sync(0xffffffffu, m_sse, o);
-            m_en += __shfl_xor_sync(0xffffffffu, m_en, o);
+            m_sse = u128_add(m_sse, u128_shfl_xor(m_sse, o));
+            m_en = u128_add(m_en, u128_shfl_xor(m_en, o));
             m_nnz += __shfl_xor_sync(0xffffffffu, m_nnz, o);
         }
         if (lane == 0) {
             ensure_dep();
-            atomicAdd(&P.macc[0], (unsigned long long)m_sse);
-            atomicAdd(&P.macc[1], (unsigned long long)m_en);
-            atomicAdd(&P.macc[2], (unsigned long long)m_nnz);
+            atomic_add_u128(&P.macc[0], m_sse);
+            atomic_add_u128(&P.macc[2], m_en);
+            atomicAdd(&P.macc[4], m_nnz);
         }
     }
     if (lane == 0) {
@@ -939,11 +997,11 @@ __global__ void B200DCT_TMA_BOUNDS k_tma(const __grid_constant__ TmaParams P)
                 if constexpr (METRICS) {
                     if (P.acc) { // every other warp's sums are in (its atomics precede its fence + ticket)
                         __threadfence();
-                        const long long sse = (long long)atomicExch(&P.macc[0], 0ull), en = (long long)atomicExch(&P.macc[1], 0ull),
-                                        nnz = (long long)atomicExch(&P.macc[2], 0ull);
-                        P.acc[0] += (double)sse / (double)METRICS_FIXED_POINT;
-                        P.acc[1] += (double)en / (double)METRICS_FIXED_POINT;
-                        P.acc[2] += (double)nnz;
+                        unsigned long long t[MACC_WORDS];
+                        sfor<MACC_WORDS>([&](auto q) { t[IC(q)] = atomicExch(&P.macc[IC(q)], 0ull); });
+                        P.acc[0] += u128_to_double(t[0], t[1]) / METRICS_FIXED_POINT;
+                        P.acc[1] += u128_to_double(t[2], t[3]) / METRICS_FIXED_POINT;
+                        P.acc[2] += (double)t[4];
                     }
                 }
                 sched[0] = 0;

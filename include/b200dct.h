@@ -52,12 +52,16 @@
 extern "C" {
 #endif
 
-#define B200DCT_VERSION 101 /* 101: b200dct_forward_rgb / b200dct_inverse_rgb */
+#define B200DCT_VERSION 102 /* 101: b200dct_forward_rgb / b200dct_inverse_rgb; 102: b200dct_zigzag_coded_bits flags
+                               * out-of-range symbols (B200DCT_CODED_OUT_OF_RANGE), f32 metrics in 128-bit fixed point */
 
 typedef enum b200dct_dtype {
     B200DCT_F32 = 0, /* float pixels / integer-valued float coefficients (the reference's type) */
     B200DCT_U8 = 1,  /* 8-bit pixels: convertToFloat on load, clamp+truncate on store (utils.cu:10-24) */
-    B200DCT_I16 = 2, /* compact coefficients (saturating); coefficient planes only */
+    /* compact coefficients; coefficient planes only.  Written values saturate to [-32768, 32767] (round to
+     * nearest, then clamp).  A fused round trip's pixels come from the unsaturated coefficients: they do not
+     * depend on the dtype of its coefficient output. */
+    B200DCT_I16 = 2,
     /* Compact coefficient STREAM (SURVEY.md section 8f.1; the natural input of an entropy coder):
      * block-major -- block (r, c) of the H/8 x W/8 grid is 64 consecutive int16 (saturating) in
      * JPEG zig-zag scan order (ITU-T T.81 figure 5) at byte offset r*pitch + c*128.  `pitch` is
@@ -221,11 +225,20 @@ int b200dct_roundtrip_any(const b200dct_plan *plan, const void *img, b200dct_dty
  *   d_acc3[0] += sum (x - y)^2     d_acc3[1] += sum x^2     d_acc3[2] += non-zero quantised coefficients
  * so MSE = acc[0]/(H*W), PEEN% = 100*sqrt(acc[0]/acc[1]) (the definitions recovered from
  * README.md:67-68 of the reference) and the coefficient density need no second pass over the
- * images.  Per-CTA partial sums go to `workspace` (device, >= b200dct_metrics_workspace_bytes,
- * caller-owned, 8-byte aligned) and are reduced in a fixed order: results are deterministic,
- * exact for u8 images.  `out` must not alias `img`.  Large f32 images of Haweel's T run the TMA family's
- * metrics kernel (the error is taken from the input tile in shared memory, sums accumulate as 64-bit
- * fixed point: still deterministic); everything else the direct family's. */
+ * images.  `workspace`: device, >= b200dct_metrics_workspace_bytes, caller-owned, 8-byte aligned.
+ * `out` must not alias `img`.  Large f32 images of Haweel's T run the TMA family's metrics kernel (the
+ * error is taken from the input tile in shared memory); everything else the direct family's.
+ * Range and accuracy:
+ *   u8 images: exact integers, in one launch (or, under stream capture without a free scheduler slot,
+ *     per-CTA partials in `workspace` reduced in a fixed order).
+ *   f32 images: each 8x8 block's two sums are taken in f32 in a fixed order, converted exactly to 128-bit
+ *     fixed point in units of 2^-50 and added as integers, so the result does not depend on scheduling:
+ *     run to run and between the two kernel families it is the same bit for bit.  The sums are exact
+ *     to within 2^-50 per block, and the totals may reach 2^78 (2^22 blocks, a 16384^2 image, of pixels
+ *     up to 2^20 sum to 2^68).  The relative error is that of the per-block f32 sums (measured <= 1e-6 for
+ *     pixels of magnitude 2^-10 .. 2^20 with the quantiser scaled alike, tests/test_gpu_range.py).
+ *     Without a free scheduler slot under capture the f32 direct path falls back to per-CTA double
+ *     partials reduced in a fixed order: deterministic too, but its last bits can differ. */
 size_t b200dct_metrics_workspace_bytes(int H, int W);
 int b200dct_roundtrip_metrics(const b200dct_plan *plan,
                               const void *img, b200dct_dtype in_dt, size_t in_pitch,
@@ -259,7 +272,8 @@ int b200dct_roundtrip_rgb(const b200dct_plan *plan, const void *rgb, size_t in_p
  * Arguments, stream layout and error codes as b200dct_roundtrip_rgb; zz3 is required.  One launch
  * each (b200dct_last_path() "rgb"), legal under stream capture.  b200dct_inverse_rgb of the streams
  * b200dct_forward_rgb wrote gives b200dct_roundtrip_rgb's pixels bit for bit, in either inverse mode,
- * as long as no stream value saturates (never for Q entries >= 1/16).
+ * as long as no stream value saturates (never for Q entries >= 1/16).  Beyond that the streams hold the
+ * saturated values while b200dct_roundtrip_rgb's pixels still come from the unsaturated ones.
  * RGB -> YCbCr (libjpeg jccolor.c) -> per plane convertToFloat, dct, quantise (luminance Q for Y,
  * chrominance Q for Cb/Cr, plan's keep mask) -> three block-major zig-zag int16 streams
  * (B200DCT_I16_ZIGZAG layout, block-row pitch (W/8)*128, planes zz_plane_bytes apart). */
@@ -275,7 +289,12 @@ int b200dct_inverse_rgb(const b200dct_plan *plan, const void *zz3, size_t zz_pla
  * of one plane's zig-zag stream (B200DCT_I16_ZIGZAG layout; pitch = bytes per block-row), ADDED
  * to *d_bits (device, 8-byte aligned).  table: 0 luminance codes, 1 chrominance codes.  This
  * defines the "Compr. Factor" of the reference's README (README.md:62-69), for which the
- * reference has no code:  CF = 8 * H * W / bits. */
+ * reference has no code:  CF = 8 * H * W / bits.
+ * Baseline JPEG codes DC differences of magnitude <= 2047 (categories 0..11) and AC values of
+ * magnitude <= 1023 (categories 1..10) only.  A stream with any other symbol -- which quantiser
+ * entries below 1 can produce from 8-bit pixels -- has no baseline size: its symbols count 0 bits
+ * and the call ORs B200DCT_CODED_OUT_OF_RANGE (bit 63) into *d_bits. */
+#define B200DCT_CODED_OUT_OF_RANGE (1ull << 63)
 int b200dct_zigzag_coded_bits(const void *zz, size_t pitch, int H, int W, int table,
                               unsigned long long *d_bits, void *stream);
 

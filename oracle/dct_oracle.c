@@ -426,30 +426,34 @@ static int bit_size(int v) /* T.81 F.1.2.1: SSSS = number of bits of |v| */
     return n;
 }
 
-/* stream: the block-major zig-zag int16 stream of ONE plane (oracle_zigzag_i16), blocks in raster order */
+/* stream: the block-major zig-zag int16 stream of ONE plane (oracle_zigzag_i16), blocks in raster order.
+ * Baseline JPEG codes DC-difference categories 0..11 and AC categories 1..10 only: a symbol outside them
+ * has no code, counts 0 bits and sets bit 63 of the result (b200dct_zigzag_coded_bits does the same). */
 uint64_t oracle_coded_bits(const int16_t *stream, size_t nblocks, int table)
 {
     unsigned char dcl[256], acl[256];
     oracle_huffman_lengths(0, table, dcl);
     oracle_huffman_lengths(1, table, acl);
-    uint64_t bits = 0;
+    uint64_t bits = 0, out_of_range = 0;
     int prev = 0;
     for (size_t b = 0; b < nblocks; b++) {
         const int16_t *c = stream + b * 64;
         const int s = bit_size((int)c[0] - prev);
         prev = c[0];
-        bits += dcl[s] + s;
+        if (s <= 11) bits += dcl[s] + s;
+        else out_of_range = 1;
         int run = 0;
         for (int k = 1; k < 64; k++) {
             if (c[k] == 0) { run++; continue; }
             while (run > 15) { bits += acl[0xf0]; run -= 16; }
             const int sz = bit_size(c[k]);
-            bits += acl[(run << 4) | sz] + sz;
+            if (sz <= 10) bits += acl[(run << 4) | sz] + sz;
+            else out_of_range = 1;
             run = 0;
         }
         if (run) bits += acl[0x00];
     }
-    return bits;
+    return bits | (out_of_range << 63);
 }
 
 /* MSE and PEEN as recovered from the reference's README table (SURVEY.md section 6):

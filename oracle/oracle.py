@@ -138,8 +138,12 @@ def huffman_lengths(which: int, table: int) -> np.ndarray:
     return out
 
 
+CODED_OUT_OF_RANGE = 1 << 63
+
+
 def coded_bits(stream: np.ndarray, table: int = 0) -> int:
-    """Baseline-JPEG entropy-coded size in bits of one plane's zig-zag int16 stream (.., 64)."""
+    """Baseline-JPEG entropy-coded size in bits of one plane's zig-zag int16 stream (.., 64).  Symbols
+    outside the baseline categories count 0 bits and set CODED_OUT_OF_RANGE (bit 63), as on the GPU."""
     stream = np.ascontiguousarray(stream, np.int16)
     return int(lib().oracle_coded_bits(stream.reshape(-1), stream.size // 64, table))
 
@@ -147,7 +151,10 @@ def coded_bits(stream: np.ndarray, table: int = 0) -> int:
 def compression_factor(coef: np.ndarray, table: int = 0) -> float:
     """8*H*W / coded_bits of a coefficient plane (README.md:62-69 'Compr. Factor', see dct_oracle.c)."""
     H, W = coef.shape
-    return 8.0 * H * W / coded_bits(zigzag_i16(coef), table)
+    bits = coded_bits(zigzag_i16(coef), table)
+    if bits & CODED_OUT_OF_RANGE:
+        raise ValueError("coefficients outside the baseline-JPEG categories: no coded size")
+    return 8.0 * H * W / bits
 
 
 def dct2_T() -> np.ndarray:
