@@ -18,38 +18,31 @@
 #include "mma_kernels.cuh"
 
 namespace b200dct {
-// one launcher per translation unit of kernel instantiations (inst_<family>_<s|d><quantiser>.cu)
+// one launcher per family and translation unit of kernel instantiations (inst_<family>_<s|d|y><quantiser>.cu);
+// ctas_per_sm != NULL: no launch, only the resident-CTA count of the kernel the arguments select
 #define B200_DECL(tag)                                                                                                  \
-    cudaError_t launch_direct_##tag(int mode, int pix, bool finv, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm); \
-    cudaError_t launch_direct_metrics_##tag(int pix, bool finv, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm); \
+    cudaError_t launch_direct_##tag(int mode, int pix, bool finv, bool metrics, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm); \
     cudaError_t launch_tma_##tag(int mode, int pix, bool finv, const TmaParams &P, int grid, int block, size_t smem, cudaStream_t s, bool pdl);
 B200_DECL(s0) B200_DECL(s1) B200_DECL(s2) B200_DECL(d1) B200_DECL(d2) B200_DECL(y1) B200_DECL(y2)
 #undef B200_DECL
-cudaError_t launch_direct_kmask(int k, int pix, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm = nullptr); // inst_direct_k.cu
+cudaError_t launch_direct_kmask(int k, int pix, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm); // inst_direct_k.cu
 cudaError_t launch_any_f32(int tk, int qm, bool finv, const AnyParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl); // inst_any_f32.cu
 cudaError_t launch_any_u8(int tk, int qm, bool finv, const AnyParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl);  // inst_any_u8.cu
 cudaError_t launch_mma(bool fastdiv, const MmaParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl);                           // inst_mma.cu
 cudaError_t launch_tma_kmask(int k, int pix, const TmaParams &P, int grid, int block, size_t smem, cudaStream_t s, bool pdl);          // inst_tma_k.cu
 
-// ctas_per_sm != NULL: no launch, only the resident-CTA count of the kernel the arguments select
-static cudaError_t launch_direct(int tk, int mode, int q, int pix, bool finv, const DirectParams &P, dim3 g, dim3 b, cudaStream_t s, bool pdl, int *ctas_per_sm = nullptr)
+struct Unit {
+    decltype(&launch_direct_s0) direct;
+    decltype(&launch_tma_s0) tma;
+};
+// the translation unit of (T family, quantiser)
+static Unit unit_of(int tk, int q)
 {
-    int *c = ctas_per_sm;
-    if (tk == TK_DENSE_SYM) return q == 1 ? launch_direct_y1(mode, pix, finv, P, g, b, s, pdl, c) : launch_direct_y2(mode, pix, finv, P, g, b, s, pdl, c);
-    if (tk == TK_HAWEEL) return q == 0 ? launch_direct_s0(mode, pix, finv, P, g, b, s, pdl, c) : q == 1 ? launch_direct_s1(mode, pix, finv, P, g, b, s, pdl, c) : launch_direct_s2(mode, pix, finv, P, g, b, s, pdl, c);
-    return q == 1 ? launch_direct_d1(mode, pix, finv, P, g, b, s, pdl, c) : launch_direct_d2(mode, pix, finv, P, g, b, s, pdl, c);
-}
-static cudaError_t launch_direct_metrics(int tk, int q, int pix, bool finv, const DirectParams &P, dim3 g, dim3 b, cudaStream_t s, bool pdl = false, int *c = nullptr)
-{
-    if (tk == TK_DENSE_SYM) return q == 1 ? launch_direct_metrics_y1(pix, finv, P, g, b, s, pdl, c) : launch_direct_metrics_y2(pix, finv, P, g, b, s, pdl, c);
-    if (tk == TK_HAWEEL) return q == 0 ? launch_direct_metrics_s0(pix, finv, P, g, b, s, pdl, c) : q == 1 ? launch_direct_metrics_s1(pix, finv, P, g, b, s, pdl, c) : launch_direct_metrics_s2(pix, finv, P, g, b, s, pdl, c);
-    return q == 1 ? launch_direct_metrics_d1(pix, finv, P, g, b, s, pdl, c) : launch_direct_metrics_d2(pix, finv, P, g, b, s, pdl, c);
-}
-static cudaError_t launch_tma(int tk, int mode, int q, int pix, bool finv, const TmaParams &P, int g, int b, size_t smem, cudaStream_t s, bool pdl)
-{
-    if (tk == TK_DENSE_SYM) return q == 1 ? launch_tma_y1(mode, pix, finv, P, g, b, smem, s, pdl) : launch_tma_y2(mode, pix, finv, P, g, b, smem, s, pdl);
-    if (tk == TK_HAWEEL) return q == 0 ? launch_tma_s0(mode, pix, finv, P, g, b, smem, s, pdl) : q == 1 ? launch_tma_s1(mode, pix, finv, P, g, b, smem, s, pdl) : launch_tma_s2(mode, pix, finv, P, g, b, smem, s, pdl);
-    return q == 1 ? launch_tma_d1(mode, pix, finv, P, g, b, smem, s, pdl) : launch_tma_d2(mode, pix, finv, P, g, b, smem, s, pdl);
+#define B200_UNIT(tag) Unit{launch_direct_##tag, launch_tma_##tag}
+    if (tk == TK_DENSE_SYM) return q == 1 ? B200_UNIT(y1) : B200_UNIT(y2);
+    if (tk == TK_HAWEEL) return q == 0 ? B200_UNIT(s0) : q == 1 ? B200_UNIT(s1) : B200_UNIT(s2);
+    return q == 1 ? B200_UNIT(d1) : B200_UNIT(d2);
+#undef B200_UNIT
 }
 } // namespace b200dct
 
@@ -151,13 +144,6 @@ static void plan_refresh(b200dct_plan *pl)
     for (int i = 0; i < 4; i++)
         for (int n = 0; n < 4; n++) pl->cp.t.eo[i * 4 + n] = make_float2(pl->T[(2 * i) * 8 + n], pl->T[(2 * i + 1) * 8 + n]);
     pl->tk = pl->sparse ? TK_HAWEEL : ((pl->symmetric && pl->dense != B200DCT_DENSE_CHAIN) ? TK_DENSE_SYM : TK_DENSE);
-}
-
-static int qmode_of(const b200dct_plan *pl)
-{
-    if (!pl->q_fastdiv) return Q_PARAM_DIV;
-    if (pl->sparse && pl->q_default && pl->mask == ~(uint64_t)0) return Q_IMM;
-    return Q_PARAM;
 }
 
 extern "C" int b200dct_plan_create(b200dct_plan **out)
@@ -466,6 +452,8 @@ unsigned long long *sched_macc(const uint32_t *slot)
 //     successor CTA runs, and only the predecessor's writes matter;
 //   * so: predecessor on this stream = such a launch, and [input plane] disjoint from its output /
 //     coefficient planes  =>  early_loads.  Launches that do not qualify as predecessors clear the record.
+// Every launch of the library, taking part or not, happens inside a LaunchScope (plan_internal.h), which holds
+// g_last_mu across the decision, the launch and the update of the record.
 // Not under stream capture.  env B200DCT_EARLY_LOADS=0 disables (A/B).
 namespace {
 struct Range {
@@ -484,12 +472,12 @@ constexpr int LAST_SLOTS = 16;
 LastLaunch g_last[LAST_SLOTS];
 unsigned long long *g_chain[64] = {}; // per device: one completion counter per record
 std::mutex g_last_mu;
-Range plane_range(const void *p, size_t pitch, size_t row_bytes, int H)
+Range plane_range(const Span &sp)
 {
     Range r;
-    if (p) {
-        r.lo = (uintptr_t)p;
-        r.hi = r.lo + (size_t)(H - 1) * pitch + row_bytes;
+    if (sp.ptr) {
+        r.lo = (uintptr_t)sp.ptr;
+        r.hi = r.lo + (size_t)(sp.rows - 1) * sp.pitch + sp.row_bytes;
     }
     return r;
 }
@@ -527,10 +515,9 @@ struct LaunchTicket {
     unsigned long long *chain = nullptr; // the record's completion counter (NULL: none, no early path around this launch)
     unsigned long long target = 0;       // its value once the predecessor is complete
 };
-// Step 1, before the launch: may a launch of family `tma` / direct reading `rd` on `stream` load early?
-// (fills: it satisfies its family's machine-filling condition.)  Leaves the record cleared; commit_launch_locked
-// fills it in once the kernel is in the stream.  The caller holds g_last_mu across both steps and the launch:
-// the record order must be the stream order even when several host threads launch on one stream.
+// Before the launch: may a launch of family `tma` / direct reading `rd` on `stream` load early?  (fills: it
+// satisfies its family's machine-filling condition.)  Leaves the record cleared; LaunchScope::done fills it in
+// once the kernel is in the stream.  The caller holds g_last_mu from here until then.
 LaunchTicket begin_launch_locked(cudaStream_t stream, bool tma, bool fills, bool may_allocate, const Range &rd)
 {
     LaunchTicket t;
@@ -569,58 +556,41 @@ LaunchTicket begin_launch_locked(cudaStream_t stream, bool tma, bool fills, bool
     e->tma = e->direct = false; // until committed
     return t;
 }
-// Step 2, after a successful launch: this launch as the next one's predecessor.  feeds: the kernel was
-// given the counter and adds `inc` to it in total.
-void commit_launch_locked(const LaunchTicket &t, bool tma, bool feeds, unsigned long long inc, const Range &w0, const Range &w1,
-                          const Range &w2 = Range{})
-{
-    if (!t.rec) return;
-    t.rec->tma = tma && feeds;
-    t.rec->direct = !tma && feeds;
-    t.rec->w[0] = w0;
-    t.rec->w[1] = w1;
-    t.rec->w[2] = w2;
-    if (feeds) t.rec->expected += inc;
-}
 } // namespace
 namespace b200dct {
-void forget_stream(cudaStream_t s)
-{
-    std::lock_guard<std::mutex> lk(g_last_mu);
-    begin_launch_locked(s, false, false, false, Range{}); // leaves the record cleared
-}
-// the same protocol for the direct-style kernels of other translation units (colour)
-EarlyScope::EarlyScope(cudaStream_t s, bool usable, unsigned long long ctas, int ctas_per_sm, Span rd, Span w0, Span w1)
-    : rec_(nullptr), feeds_(false), finished_(false)
+LaunchScope::LaunchScope(cudaStream_t s, Family family, bool usable, unsigned long long ctas, int ctas_per_sm, Span rd, Span w0,
+                         Span w1, Span w2)
+    : family_(family), w_{w0, w1, w2}
 {
     g_last_mu.lock();
-    w_[0] = w0;
-    w_[1] = w1;
-    int sms = 0, dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) usable = false;
-    const unsigned long long machine = (unsigned long long)(ctas_per_sm > 0 ? ctas_per_sm : 0) * (unsigned long long)sms;
-    const bool fills = usable && machine > 0 && ctas > machine;
-    const Range r = (usable && rd.ptr) ? plane_range(rd.ptr, rd.pitch, rd.row_bytes, rd.rows) : Range{};
-    const LaunchTicket t = begin_launch_locked(s, false, fills, usable, r);
+    const DevInfo di = dev_info();
+    usable = usable && family != NONE && di.ok;
+    const unsigned long long machine = (unsigned long long)(ctas_per_sm > 0 ? ctas_per_sm : 0) * (unsigned long long)di.sms;
+    // direct style: more CTAs than the machine holds at once; TMA: a CTA on every SM
+    const bool fills = usable && machine > 0 && (family == TMA ? ctas >= machine : ctas > machine);
+    const LaunchTicket t = begin_launch_locked(s, family == TMA, fills, usable, usable ? plane_range(rd) : Range{});
+    const bool feeds = fills && t.chain != nullptr;
     rec_ = t.rec;
-    feeds_ = fills && t.chain != nullptr;
-    p_.early = t.early ? (int)(ctas < machine ? ctas : machine) : 0;
-    p_.chain = (feeds_ || t.early) ? t.chain : nullptr;
-    p_.chain_target = t.target;
-    p_.chain_feed = feeds_ ? (int)(ctas < 1024 ? ctas : 1024) : 0;
+    // direct style: CTAs beyond one machine-full start after the predecessor anyway, and the last CTAs of the grid
+    // feed the counter
+    early_ = t.early ? (family == TMA ? 1 : (int)(ctas < machine ? ctas : machine)) : 0;
+    chain_feed_ = feeds ? (family == TMA ? 1 : (int)(ctas < 1024 ? ctas : 1024)) : 0;
+    chain_ = (feeds || t.early) ? t.chain : nullptr;
+    chain_target_ = t.target;
 }
-void EarlyScope::done(bool launched)
+void LaunchScope::done(bool launched)
 {
     if (finished_) return;
     finished_ = true;
-    LaunchTicket t;
-    t.rec = static_cast<LastLaunch *>(rec_);
-    if (launched)
-        commit_launch_locked(t, false, feeds_, (unsigned long long)p_.chain_feed, plane_range(w_[0].ptr, w_[0].pitch, w_[0].row_bytes, w_[0].rows),
-                             plane_range(w_[1].ptr, w_[1].pitch, w_[1].row_bytes, w_[1].rows));
+    LastLaunch *r = static_cast<LastLaunch *>(rec_);
+    if (launched && r) { // this launch as the next one's predecessor
+        r->tma = family_ == TMA && chain_feed_ > 0;
+        r->direct = family_ == DIRECT && chain_feed_ > 0;
+        for (int i = 0; i < 3; i++) r->w[i] = plane_range(w_[i]);
+        r->expected += (unsigned long long)chain_feed_;
+    }
     g_last_mu.unlock();
 }
-EarlyScope::~EarlyScope() { done(false); }
 }
 
 static bool tma_dynamic = true; // env B200DCT_TMA_STATIC=1 forces the static tile split
@@ -639,23 +609,22 @@ static bool use_pdl()
     }();
     return v;
 }
+namespace b200dct {
+bool use_factored_inverse_u8(const b200dct_plan *pl) { return use_factored_inverse(pl, MODE_RT, DT_U8); }
+bool stream_capturing(cudaStream_t s)
+{
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    return cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
+}
 // Under stream capture the attribute becomes a programmatic edge of the graph (CUDA >= 12.3);
 // off unless B200DCT_PDL_CAPTURE=1 (experiment).
-static bool pdl_for(bool capturing)
+bool pdl_enabled(bool capturing)
 {
     static const bool cap = [] {
         const char *p = getenv("B200DCT_PDL_CAPTURE");
         return p && atoi(p) == 1;
     }();
     return use_pdl() && (!capturing || cap);
-}
-namespace b200dct {
-bool use_factored_inverse_u8(const b200dct_plan *pl) { return use_factored_inverse(pl, MODE_RT, DT_U8); }
-bool pdl_enabled(cudaStream_t s)
-{
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    const bool capturing = cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
-    return pdl_for(capturing);
 }
 } // namespace b200dct
 static int tma_grid = 0;                          // env B200DCT_TMA_GRID: CTAs (default: one per SM)
@@ -685,6 +654,48 @@ static bool prefers_tma(const b200dct_plan *pl, size_t bytes_per_px, int H, int 
            (bytes_per_px >= 4 && pl->tk == TK_DENSE_SYM && px >= TMA_HUGE_PIXELS);
 }
 
+// The kernel variant a plan runs for (mode, pixel dtype): quantiser, compile-time retained-coefficient mask (kmask
+// = k of the first k zig-zag coefficients, 0: none) and the factored inverse.  runtime_mask: the kernels take the
+// mask as data only (metrics, any size).
+struct Variant {
+    int qm, kmask;
+    bool finv;
+};
+static Variant variant_of(const b200dct_plan *pl, int mode, int pix, bool runtime_mask)
+{
+    Variant v;
+    if (!pl->q_fastdiv) v.qm = Q_PARAM_DIV;
+    else if (pl->sparse && pl->q_default && pl->mask == ~(uint64_t)0) v.qm = Q_IMM;
+    else v.qm = Q_PARAM;
+    // retained-coefficient round trips (first k = 6..10 zig-zag coefficients of the default
+    // tables): kernels with the mask as a compile-time constant
+    v.kmask = 0;
+    if (mode == MODE_RT && !runtime_mask && pl->sparse && pl->q_default && pl->q_fastdiv && compiled_masks())
+        for (int k = 6; k <= 10; k++)
+            if (pl->mask == b200dct_zigzag_mask(k)) v.kmask = k;
+    v.finv = !v.kmask && use_factored_inverse(pl, mode, pix); // compile-time-mask kernels keep the chains
+    return v;
+}
+// ctas_per_sm != NULL: no launch, only the resident-CTA count of the kernel the arguments select
+static cudaError_t launch_direct(int tk, const Variant &v, int mode, int pix, bool metrics, const DirectParams &P, dim3 grid,
+                                 dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm = nullptr)
+{
+    if (v.kmask) return launch_direct_kmask(v.kmask, pix, P, grid, block, s, pdl, ctas_per_sm);
+    return unit_of(tk, v.qm).direct(mode, pix, v.finv, metrics, P, grid, block, s, pdl, ctas_per_sm);
+}
+static cudaError_t launch_tma(int tk, const Variant &v, int mode, int pix, const TmaParams &P, int grid, int block, size_t smem,
+                              cudaStream_t s, bool pdl)
+{
+    if (v.kmask) return launch_tma_kmask(v.kmask, pix, P, grid, block, smem, s, pdl);
+    return unit_of(tk, v.qm).tma(mode, pix, v.finv, P, grid, block, smem, s, pdl);
+}
+// the bytes of one plane of a call (the zig-zag stream: H/8 rows of W/8 blocks of 128 bytes)
+static Span plane_span(const Plane &p, int H, int W)
+{
+    if (p.dt == DT_I16ZZ) return Span{p.ptr, p.pitch, (size_t)(W / 8) * 128, H / 8};
+    return Span{p.ptr, p.pitch, (size_t)W * elem_size(p.dt), H};
+}
+
 static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef, float *shifted, int H, int W,
                cudaStream_t stream, double *partials = nullptr, double *acc = nullptr)
 {
@@ -703,8 +714,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
 
     const int pix = (mode == MODE_INV) ? out.dt : in.dt;
     const int coef_dt = (mode == MODE_FWD) ? out.dt : (mode == MODE_INV ? in.dt : (coef.ptr ? coef.dt : DT_F32));
-    const int qmode = qmode_of(pl);
-    const int qm = (!pl->sparse && qmode == Q_IMM) ? Q_PARAM : qmode;
+    const Variant v = variant_of(pl, mode, pix, partials != nullptr); // the metrics kernels take runtime masks
 
     // AUTO: the TMA family wins where the call is HBM-bound (>= 4 bytes moved per pixel: any
     // f32/i16 plane); all-u8 round trips move 2 B/px, are instruction-issue bound, and run faster
@@ -726,8 +736,8 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     // Under stream capture the launch takes a ticket-counter pair of its own (see SchedRing); when
     // none is left (or the pools do not exist yet) AUTO falls back to the hardware-scheduled
     // direct family (86.9 us at 8192^2), which beats the TMA family's static split (99.8 us).
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    const bool capturing = cudaStreamIsCapturing(stream, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
+    const bool capturing = stream_capturing(stream);
+    const bool pdl = pdl_enabled(capturing);
     static std::once_flag env_once;
     std::call_once(env_once, [] {
         const char *e = getenv("B200DCT_TMA_WARPS");
@@ -749,16 +759,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     if (capturing && tma_dynamic && tma_possible) capture_sched = sched_slot(true);
     const bool use_tma = tma_possible && !(capturing && !capture_sched && pl->path == B200DCT_PATH_AUTO);
     if (pl->path == B200DCT_PATH_TMA && !use_tma) return B200DCT_ERR_ALIGN;
-
-    // retained-coefficient round trips (first k = 6..10 zig-zag coefficients of the default
-    // tables): kernels with the mask as a compile-time constant
-    int kmask = 0;
-    if (mode == MODE_RT && pl->sparse && pl->q_default && pl->q_fastdiv && compiled_masks())
-        for (int k = 6; k <= 10; k++)
-            if (pl->mask == b200dct_zigzag_mask(k)) kmask = k;
-
-    if (partials) kmask = 0; // the metrics kernels take runtime masks
-    const bool finv = !kmask && use_factored_inverse(pl, mode, pix); // compile-time-mask kernels keep the chains
+    const Span rd = plane_span(in, H, W), w0 = plane_span(out, H, W), w1 = plane_span(coef, H, W);
     // the tensor-core arm of the dense variant (opt-in): f32 fused round trips, optional f32 coefficient plane
     if (pl->dense == B200DCT_DENSE_MMA && !pl->sparse && mode == MODE_RT && in.dt == DT_F32 && !partials && !shifted &&
         (!coef.ptr || coef.dt == DT_F32)) {
@@ -771,8 +772,8 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
         M.cp = pl->cp;
         dim3 mblock(32, 4), mgrid((unsigned)((M.by + 3) / 4), (unsigned)((M.bx + 31) / 32));
         if (mgrid.y > 65535u) return B200DCT_ERR_SHAPE;
-        forget_stream(stream);
-        const cudaError_t em = launch_mma(pl->q_fastdiv, M, mgrid, mblock, stream, pdl_for(capturing));
+        LaunchScope order(stream);
+        const cudaError_t em = launch_mma(pl->q_fastdiv, M, mgrid, mblock, stream, pdl);
         if (em != cudaSuccess) return (int)em;
         tl_launches = 1;
         tl_path = "mma";
@@ -818,38 +819,25 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
         P.run_tickets = nt > tail ? (uint32_t)((nt - tail) / P.run) : 0u;
         // Metrics: with the dynamic scheduler the slot owns a zeroed integer accumulator and the last warp out
         // folds it into acc -- one launch.  Static split: the first MACC_WORDS words of the caller's workspace,
-        // zeroed before and folded after the kernel.
-        std::unique_lock<std::mutex> launch_order(g_last_mu); // held until this kernel is in the stream
-        const Range rd = plane_range(in.ptr, in.pitch, (size_t)W * elem_size(in.dt), H);
-        const Range w0 = plane_range(out.ptr, out.pitch, (size_t)W * elem_size(out.dt), H);
-        const Range w1 = plane_range(coef.ptr, coef.pitch, (size_t)W * elem_size(coef.dt), H);
-        // the argument above needs the predecessor to occupy every SM (grid == SM count) and neither
-        // launch to fit beside the other on one SM: both take more than half of its shared memory
-        const bool heavy = smem > (size_t)(di.smem_optin / 2) + 1024;
-        const bool fills = !capturing && pdl_for(capturing) && grid >= di.sms && heavy && P.sched != nullptr;
-        const LaunchTicket ticket = begin_launch_locked(stream, true, fills, !capturing, rd);
-        const bool feeds = fills && ticket.chain != nullptr;
-        P.early_loads = ticket.early ? 1 : 0;
-        P.chain = (feeds || ticket.early) ? ticket.chain : nullptr;
-        P.chain_target = ticket.target;
-        P.chain_feed = feeds ? 1 : 0;
-        bool separate_finish = false;
+        // zeroed before and folded after the kernel by a second one.
         if (partials) {
             P.macc = sched_macc(P.sched);
             P.acc = acc;
-            if (!P.macc) {
-                separate_finish = true;
-                P.acc = nullptr;
-                P.macc = reinterpret_cast<unsigned long long *>(partials);
-                const cudaError_t em = cudaMemsetAsync(P.macc, 0, MACC_WORDS * sizeof(unsigned long long), stream);
-                if (em != cudaSuccess) return (int)em;
-            }
         }
-        cudaError_t e = kmask
-                            ? launch_tma_kmask(kmask, pix, P, grid, nw * 32, smem, stream, pdl_for(capturing))
-                            : launch_tma(pl->tk, mode, qm, pix, finv, P, grid, nw * 32, smem, stream, pdl_for(capturing) && !separate_finish);
-        if (e == cudaSuccess) commit_launch_locked(ticket, true, feeds, 1, w0, w1);
-        launch_order.unlock();
+        const bool separate_finish = partials && !P.macc;
+        // the argument above needs the predecessor to occupy every SM (grid == SM count) and neither
+        // launch to fit beside the other on one SM: both take more than half of its shared memory
+        const bool heavy = smem > (size_t)(di.smem_optin / 2) + 1024;
+        LaunchScope scope(stream, separate_finish ? LaunchScope::NONE : LaunchScope::TMA, pdl && !capturing && heavy && P.sched != nullptr,
+                          (unsigned long long)grid, 1, rd, w0, w1);
+        scope.apply(P);
+        if (separate_finish) {
+            P.acc = nullptr;
+            P.macc = reinterpret_cast<unsigned long long *>(partials);
+            const cudaError_t em = cudaMemsetAsync(P.macc, 0, MACC_WORDS * sizeof(unsigned long long), stream);
+            if (em != cudaSuccess) return (int)em;
+        }
+        cudaError_t e = launch_tma(pl->tk, v, mode, pix, P, grid, nw * 32, smem, stream, pdl && !separate_finish);
         if (e != cudaSuccess) return (int)e;
         tl_launches = 1;
         if (separate_finish) {
@@ -858,6 +846,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
             if (e != cudaSuccess) return (int)e;
             tl_launches = 2;
         }
+        scope.done(true);
         tl_path = "tma";
         return B200DCT_OK;
     }
@@ -879,88 +868,43 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     dim3 block(32, 4);
     dim3 grid((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32));
     if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
-    cudaError_t e;
-    if (partials) {
+    const bool metrics = partials != nullptr;
+    if (metrics) {
         if (mode != MODE_RT || in.ptr == out.ptr) return B200DCT_ERR_ARG;
-        kmask = 0;
         // One launch: integer sums through 64-bit atomics into the triple that belongs to a ticket-counter pair,
         // the last CTA out folds them into acc (the TMA family's scheme).  Dependent launch and the early path apply.
         uint32_t *slot = sched_slot(capturing);
         unsigned long long *macc = sched_macc(slot);
-        if (slot && macc) {
-            const bool pdl = pdl_for(capturing);
-            std::lock_guard<std::mutex> launch_order(g_last_mu); // held until this kernel is in the stream
-            int per_sm = 0;
-            if (pdl && !capturing) launch_direct_metrics(pl->tk, qm, pix, finv, P, grid, block, stream, pdl, &per_sm);
-            const unsigned long long ctas = (unsigned long long)grid.x * grid.y;
-            const unsigned long long machine = (unsigned long long)per_sm * (unsigned long long)di.sms;
-            const bool fills = per_sm > 0 && ctas > machine;
-            const bool eligible = pdl && !capturing && !coef.ptr;
-            const Range rd = eligible ? plane_range(in.ptr, in.pitch, (size_t)W * elem_size(in.dt), H) : Range{};
-            const Range w0 = plane_range(out.ptr, out.pitch, (size_t)W * elem_size(out.dt), H);
-            const Range w1 = plane_range(coef.ptr, coef.pitch, coef_dt == DT_I16ZZ ? (size_t)(W / 8) * 128 : (size_t)W * elem_size(coef.dt),
-                                         coef_dt == DT_I16ZZ ? H / 8 : H);
-            const Range w2 = plane_range(acc, 0, 3 * sizeof(double), 1);
-            const LaunchTicket ticket = begin_launch_locked(stream, false, fills, !capturing, rd);
-            const bool feeds = fills && ticket.chain != nullptr;
-            P.early = ticket.early ? (int)(ctas < machine ? ctas : machine) : 0;
-            P.chain = (feeds || ticket.early) ? ticket.chain : nullptr;
-            P.chain_target = ticket.target;
-            P.chain_feed = feeds ? (int)(ctas < 1024 ? ctas : 1024) : 0;
-            P.macc = macc;
-            P.mdone = slot;
-            P.acc = acc;
-            P.metrics_scale = pix == DT_U8 ? 1.0 : METRICS_FIXED_POINT;
-            e = launch_direct_metrics(pl->tk, qm, pix, finv, P, grid, block, stream, pdl);
-            if (e == cudaSuccess) commit_launch_locked(ticket, false, feeds, (unsigned long long)P.chain_feed, w0, w1, w2);
+        if (!macc) {
+            // no counter pair (capture without a free slot): per-CTA partials, then one fixed-order reduction into acc[0..2]
+            LaunchScope order(stream);
+            P.partials = partials;
+            cudaError_t e = launch_direct(pl->tk, v, mode, pix, true, P, grid, block, stream, false);
             if (e != cudaSuccess) return (int)e;
-            tl_launches = 1;
+            e = reduce_partials_sparse(partials, (size_t)grid.x * grid.y, acc, stream);
+            if (e != cudaSuccess) return (int)e;
+            tl_launches = 2;
             tl_path = "direct";
             return B200DCT_OK;
         }
-        // no counter pair (capture without a free slot): per-CTA partials, then one fixed-order reduction into acc[0..2]
-        forget_stream(stream);
-        P.partials = partials;
-        e = launch_direct_metrics(pl->tk, qm, pix, finv, P, grid, block, stream);
-        if (e != cudaSuccess) return (int)e;
-        e = reduce_partials_sparse(partials, (size_t)grid.x * grid.y, acc, stream);
-        if (e != cudaSuccess) return (int)e;
-        tl_launches = 2;
-        tl_path = "direct";
-        return B200DCT_OK;
+        P.macc = macc;
+        P.mdone = slot;
+        P.acc = acc;
+        P.metrics_scale = pix == DT_U8 ? 1.0 : METRICS_FIXED_POINT;
     }
-    const bool pdl = pdl_for(capturing);
-    {
-        // early loads (see record_launch_locked): this launch as a successor, and as the next one's predecessor
-        std::lock_guard<std::mutex> launch_order(g_last_mu); // held until this kernel is in the stream
-        int per_sm = 0;
-        if (pdl && !capturing) {
-            if (kmask) launch_direct_kmask(kmask, pix, P, grid, block, stream, pdl, &per_sm);
-            else launch_direct(pl->tk, mode, qm, pix, finv, P, grid, block, stream, pdl, &per_sm);
-        }
-        const unsigned long long ctas = (unsigned long long)grid.x * grid.y;
-        const bool fills = per_sm > 0 && ctas > (unsigned long long)per_sm * (unsigned long long)di.sms;
-        // the early path: fused round trips without a coefficient plane, forward calls without the X-128 write-back,
-        // inverse calls whose coefficients are a plane (not the zig-zag stream)
-        const bool eligible = pdl && !capturing && !coef.ptr && !shifted && !(mode == MODE_INV && in.dt == DT_I16ZZ);
-        const Range rd = eligible ? plane_range(in.ptr, in.pitch, (size_t)W * elem_size(in.dt), H) : Range{};
-        const Range w0 = out.dt == DT_I16ZZ ? plane_range(out.ptr, out.pitch, (size_t)(W / 8) * 128, H / 8)
-                                            : plane_range(out.ptr, out.pitch, (size_t)W * elem_size(out.dt), H);
-        const Range w1 = plane_range(coef.ptr, coef.pitch, coef_dt == DT_I16ZZ ? (size_t)(W / 8) * 128 : (size_t)W * elem_size(coef.dt),
-                                     coef_dt == DT_I16ZZ ? H / 8 : H);
-        const Range w2 = plane_range(shifted, in.pitch, (size_t)W * 4, H);
-        const LaunchTicket ticket = begin_launch_locked(stream, false, fills, !capturing, rd);
-        const bool feeds = fills && ticket.chain != nullptr;
-        const unsigned long long machine = (unsigned long long)per_sm * (unsigned long long)di.sms;
-        P.early = ticket.early ? (int)(ctas < machine ? ctas : machine) : 0; // CTAs beyond one machine-full start after the predecessor anyway
-        P.chain = (feeds || ticket.early) ? ticket.chain : nullptr;
-        P.chain_target = ticket.target;
-        P.chain_feed = feeds ? (int)(ctas < 1024 ? ctas : 1024) : 0;         // the last CTAs of the grid feed the counter
-        if (kmask) e = launch_direct_kmask(kmask, pix, P, grid, block, stream, pdl);
-        else e = launch_direct(pl->tk, mode, qm, pix, finv, P, grid, block, stream, pdl);
-        if (e == cudaSuccess) commit_launch_locked(ticket, false, feeds, (unsigned long long)P.chain_feed, w0, w1, w2);
-    }
+    const bool usable = pdl && !capturing;
+    int per_sm = 0;
+    if (usable) launch_direct(pl->tk, v, mode, pix, metrics, P, grid, block, stream, pdl, &per_sm);
+    // the early path: fused round trips without a coefficient plane, forward calls without the X-128 write-back,
+    // inverse calls whose coefficients are a plane (not the zig-zag stream)
+    const bool may_load_early = !coef.ptr && !shifted && !(mode == MODE_INV && in.dt == DT_I16ZZ);
+    const Span w2 = metrics ? Span{acc, 0, 3 * sizeof(double), 1} : Span{shifted, in.pitch, (size_t)W * 4, H};
+    LaunchScope scope(stream, LaunchScope::DIRECT, usable, (unsigned long long)grid.x * grid.y, per_sm, may_load_early ? rd : Span{}, w0,
+                      w1, w2);
+    scope.apply(P);
+    const cudaError_t e = launch_direct(pl->tk, v, mode, pix, metrics, P, grid, block, stream, pdl);
     if (e != cudaSuccess) return (int)e;
+    scope.done(true);
     tl_launches = 1;
     tl_path = "direct";
     return B200DCT_OK;
@@ -1028,15 +972,8 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
         tl_path = path;
         return B200DCT_OK;
     }
-    const int qmode = qmode_of(plan);
-    const int qm = (!plan->sparse && qmode == Q_IMM) ? Q_PARAM : qmode;
-    int kmask = 0;
-    if (plan->sparse && plan->q_default && plan->q_fastdiv && compiled_masks())
-        for (int k = 6; k <= 10; k++)
-            if (plan->mask == b200dct_zigzag_mask(k)) kmask = k;
-    const bool finv = !kmask && use_factored_inverse(plan, MODE_RT, (int)dt);
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    const bool capturing = cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
+    const Variant v = variant_of(plan, MODE_RT, (int)dt, false);
+    const bool pdl = pdl_enabled(stream_capturing(s));
     DirectParams P;
     memset(&P, 0, sizeof(P));
     P.in_pitch = in_pitch; P.out_pitch = out_pitch;
@@ -1049,7 +986,7 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
     dim3 block(32, 4);
     dim3 grid((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32), 1);
     if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
-    forget_stream(s);
+    LaunchScope order(s);
     int launches = 0;
     for (int first = 0; first < n_images; first += DIRECT_BATCH_MAX) {
         const int n = n_images - first < DIRECT_BATCH_MAX ? n_images - first : DIRECT_BATCH_MAX;
@@ -1060,8 +997,7 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
         }
         P.in = P.img_in[0]; P.out = P.img_out[0];
         grid.z = (unsigned)n;
-        const cudaError_t e = kmask ? launch_direct_kmask(kmask, (int)dt, P, grid, block, s, pdl_for(capturing))
-                                    : launch_direct(plan->tk, MODE_RT, qm, (int)dt, finv, P, grid, block, s, pdl_for(capturing));
+        const cudaError_t e = launch_direct(plan->tk, v, MODE_RT, (int)dt, false, P, grid, block, s, pdl);
         if (e != cudaSuccess) return (int)e;
         launches++;
     }
@@ -1094,17 +1030,13 @@ extern "C" int b200dct_roundtrip_any(const b200dct_plan *plan, const void *img, 
     P.out = out; P.out_pitch = out_pitch;
     P.H = H; P.W = W;
     P.cp = plan->cp;
-    const int qmode = qmode_of(plan);
-    const int qm = (!plan->sparse && qmode == Q_IMM) ? Q_PARAM : qmode;
+    const Variant v = variant_of(plan, MODE_RT, (int)dt, true); // finv only for 8-bit pixels
     const unsigned nby = (unsigned)((H + 7) / 8), nbx = (unsigned)((W + 7) / 8);
     dim3 block(32, 4), grid((nby + 3) / 4, (nbx + 31) / 32);
     if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    const bool capturing = cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
-    const bool finv = use_factored_inverse(plan, MODE_RT, (int)dt);
-    forget_stream(s);
-    cudaError_t e = dt == B200DCT_F32 ? launch_any_f32(plan->tk, qm, false, P, grid, block, s, pdl_for(capturing))
-                                      : launch_any_u8(plan->tk, qm, finv, P, grid, block, s, pdl_for(capturing));
+    const bool pdl = pdl_enabled(stream_capturing(s));
+    LaunchScope order(s);
+    const cudaError_t e = (dt == B200DCT_F32 ? launch_any_f32 : launch_any_u8)(plan->tk, v.qm, v.finv, P, grid, block, s, pdl);
     if (e != cudaSuccess) return (int)e;
     tl_launches = 1;
     tl_path = "any";

@@ -7,48 +7,8 @@
 
 using namespace b200dct;
 
-// ctas_per_sm != NULL: no launch, only the occupancy of kernel k (`occupancy`: the caller's cache of it)
-static cudaError_t launch_rgb_kernel(void (*k)(RgbParams), int &occupancy, const RgbParams &P, dim3 grid, cudaStream_t s,
-                                     bool pdl, int *ctas_per_sm)
-{
-    if (ctas_per_sm) {
-        if (occupancy < 0) {
-            int n = 0;
-            occupancy = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k, 128, 0) == cudaSuccess ? n : 0;
-        }
-        *ctas_per_sm = occupancy;
-        return cudaSuccess;
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(32, 4);
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, k, P);
-}
-using RgbLauncher = cudaError_t (*)(const RgbParams &, dim3, cudaStream_t, bool, int *);
-template <int QK, bool FINV, bool ZZ>
-static cudaError_t launch_rgb3(const RgbParams &P, dim3 grid, cudaStream_t s, bool pdl, int *ctas_per_sm)
-{
-    static int occupancy = -1;
-    return launch_rgb_kernel(k_rgb<QK, FINV, ZZ>, occupancy, P, grid, s, pdl, ctas_per_sm);
-}
-template <int QK>
-static cudaError_t launch_rgb_forward(const RgbParams &P, dim3 grid, cudaStream_t s, bool pdl, int *ctas_per_sm)
-{
-    static int occupancy = -1;
-    return launch_rgb_kernel(k_rgb_forward<QK>, occupancy, P, grid, s, pdl, ctas_per_sm);
-}
-template <bool FINV>
-static cudaError_t launch_rgb_inverse(const RgbParams &P, dim3 grid, cudaStream_t s, bool pdl, int *ctas_per_sm)
-{
-    static int occupancy = -1;
-    return launch_rgb_kernel(k_rgb_inverse<FINV>, occupancy, P, grid, s, pdl, ctas_per_sm);
-}
+// launch_kernel (dct_core.cuh) of one colour kernel
+using RgbLauncher = cudaError_t (*)(const RgbParams &, dim3, dim3, size_t, cudaStream_t, bool, int *);
 
 // The argument rules of the colour entry points and the parameters their kernels share.  rgb_in / rgb_out: the pixel
 // planes the call has (NULL where it has none), interleaved RGB with 8-byte aligned rows; zz: the three streams
@@ -93,22 +53,15 @@ static int rgb_qk(const b200dct_plan *plan)
 // before it waits (rd.ptr NULL: never); w0 / w1 are what the launch writes.
 static int run_rgb(RgbLauncher launch, RgbParams &P, dim3 grid, cudaStream_t s, Span rd, Span w0, Span w1)
 {
-    const bool pdl = pdl_enabled(s);
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    const bool capturing = cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
+    const bool capturing = stream_capturing(s), pdl = pdl_enabled(capturing), usable = pdl && !capturing;
+    const dim3 block(32, 4);
     int per_sm = 0;
-    if (pdl && !capturing) launch(P, grid, s, pdl, &per_sm);
-    cudaError_t e;
-    {
-        EarlyScope scope(s, pdl && !capturing, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1);
-        P.early = scope.params().early;
-        P.chain_feed = scope.params().chain_feed;
-        P.chain = scope.params().chain;
-        P.chain_target = scope.params().chain_target;
-        e = launch(P, grid, s, pdl, nullptr);
-        scope.done(e == cudaSuccess);
-    }
+    if (usable) launch(P, grid, block, 0, s, pdl, &per_sm);
+    LaunchScope scope(s, LaunchScope::DIRECT, usable, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1);
+    scope.apply(P);
+    const cudaError_t e = launch(P, grid, block, 0, s, pdl, nullptr);
     if (e != cudaSuccess) return (int)e;
+    scope.done(true);
     note_launch(1, "rgb");
     return B200DCT_OK;
 }
@@ -124,9 +77,12 @@ extern "C" int b200dct_roundtrip_rgb(const b200dct_plan *plan, const void *rgb, 
     const int rc = rgb_params(plan, rgb, in_pitch, out, out_pitch, zz3_or_null, zz_plane_bytes, H, W, P, grid);
     if (rc != B200DCT_OK) return rc;
     static const RgbLauncher launchers[3][2][2] = {
-        {{launch_rgb3<0, false, false>, launch_rgb3<0, false, true>}, {launch_rgb3<0, true, false>, launch_rgb3<0, true, true>}},
-        {{launch_rgb3<1, false, false>, launch_rgb3<1, false, true>}, {launch_rgb3<1, true, false>, launch_rgb3<1, true, true>}},
-        {{launch_rgb3<2, false, false>, launch_rgb3<2, false, true>}, {launch_rgb3<2, true, false>, launch_rgb3<2, true, true>}}};
+        {{launch_kernel<k_rgb<0, false, false>>, launch_kernel<k_rgb<0, false, true>>},
+         {launch_kernel<k_rgb<0, true, false>>, launch_kernel<k_rgb<0, true, true>>}},
+        {{launch_kernel<k_rgb<1, false, false>>, launch_kernel<k_rgb<1, false, true>>},
+         {launch_kernel<k_rgb<1, true, false>>, launch_kernel<k_rgb<1, true, true>>}},
+        {{launch_kernel<k_rgb<2, false, false>>, launch_kernel<k_rgb<2, false, true>>},
+         {launch_kernel<k_rgb<2, true, false>>, launch_kernel<k_rgb<2, true, true>>}}};
     // with streams every CTA writes mid-kernel, so that kernel never takes the early path
     return run_rgb(launchers[rgb_qk(plan)][use_factored_inverse_u8(plan)][zz3_or_null != nullptr], P, grid, (cudaStream_t)stream,
                    rgb_span(zz3_or_null ? nullptr : rgb, in_pitch, H, W), rgb_span(out, out_pitch, H, W),
@@ -142,7 +98,8 @@ extern "C" int b200dct_forward_rgb(const b200dct_plan *plan, const void *rgb, si
     dim3 grid;
     const int rc = rgb_params(plan, rgb, in_pitch, nullptr, 0, zz3, zz_plane_bytes, H, W, P, grid);
     if (rc != B200DCT_OK) return rc;
-    static const RgbLauncher launchers[3] = {launch_rgb_forward<0>, launch_rgb_forward<1>, launch_rgb_forward<2>};
+    static const RgbLauncher launchers[3] = {launch_kernel<k_rgb_forward<0>>, launch_kernel<k_rgb_forward<1>>,
+                                             launch_kernel<k_rgb_forward<2>>};
     return run_rgb(launchers[rgb_qk(plan)], P, grid, (cudaStream_t)stream, rgb_span(rgb, in_pitch, H, W),
                    zz_span(zz3, zz_plane_bytes, H, W), Span{nullptr, 0, 0, 0});
 }
@@ -156,7 +113,7 @@ extern "C" int b200dct_inverse_rgb(const b200dct_plan *plan, const void *zz3, si
     dim3 grid;
     const int rc = rgb_params(plan, nullptr, 0, out, out_pitch, const_cast<void *>(zz3), zz_plane_bytes, H, W, P, grid);
     if (rc != B200DCT_OK) return rc;
-    static const RgbLauncher launchers[2] = {launch_rgb_inverse<false>, launch_rgb_inverse<true>};
+    static const RgbLauncher launchers[2] = {launch_kernel<k_rgb_inverse<false>>, launch_kernel<k_rgb_inverse<true>>};
     return run_rgb(launchers[use_factored_inverse_u8(plan)], P, grid, (cudaStream_t)stream, zz_span(zz3, zz_plane_bytes, H, W),
                    rgb_span(out, out_pitch, H, W), Span{nullptr, 0, 0, 0});
 }

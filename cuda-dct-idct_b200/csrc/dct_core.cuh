@@ -589,4 +589,37 @@ __device__ __forceinline__ float &zigzag_elem(float2 (&p)[8][4])
 __device__ __forceinline__ float i16_lo(uint32_t w) { return (float)(short)(w & 0xffffu); }
 __device__ __forceinline__ float i16_hi(uint32_t w) { return (float)((int)w >> 16); }
 
+// ---------------------------------------------------------------- host: kernel launch
+// One launch of KERNEL with programmatic dependent launch when pdl is set: the kernel may start
+// while the previous kernel of the stream drains (every kernel of the library executes
+// griddepcontrol.wait before it touches memory its predecessor may write).
+// ctas_per_sm != NULL: no launch, only the resident CTAs per SM of KERNEL at this block size and
+// dynamic shared memory (cached; a kernel is launched with at most one size besides 0).
+template <auto KERNEL, class Params>
+inline cudaError_t launch_kernel(const Params &P, dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool pdl,
+                                 int *ctas_per_sm = nullptr)
+{
+    if (ctas_per_sm) {
+        static int cached[2] = {-1, -1};
+        int &v = cached[smem ? 1 : 0];
+        if (v < 0) {
+            int n = 0;
+            v = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, KERNEL, (int)(block.x * block.y * block.z), smem) == cudaSuccess ? n : 0;
+        }
+        *ctas_per_sm = v;
+        return cudaSuccess;
+    }
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, KERNEL, P);
+}
+
 } // namespace b200dct

@@ -557,20 +557,6 @@ __global__ void __launch_bounds__(128, METRICS ? B200DCT_METRICS_MIN_BLOCKS : B2
     }
 }
 
-// Resident CTAs per SM of one instantiation (cached): the host needs it to decide whether a launch
-// has more CTAs than the machine holds at once (early loads of its successor, b200dct.cu).
-template <void (*KERNEL)(DirectParams)>
-inline int direct_ctas_per_sm(size_t smem)
-{
-    static int cached[2] = {-1, -1};
-    int &v = cached[smem ? 1 : 0];
-    if (v < 0) {
-        int n = 0;
-        v = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, KERNEL, 128, smem) == cudaSuccess ? n : 0;
-    }
-    return v;
-}
-
 // ============================================================== TMA family
 // Tile = 8 image rows x 32 blocks (256 pixels).  Shared-memory images of a tile:
 //   f32 : 8 KiB, rows of 1 KiB = 8 segments of 128 B, hardware SWIZZLE_128B: the 16-byte
@@ -599,7 +585,7 @@ struct TmaParams {
     unsigned long long *macc;
     double *acc;          // METRICS with the dynamic scheduler: the last warp out adds macc into acc[0..2] and re-zeroes macc
     // 1: the host has established that nothing this launch READS is written by the launch it may
-    // overlap with (see early_loads_ok in b200dct.cu): tile loads start before griddepcontrol.wait,
+    // overlap with (see LaunchScope in b200dct.cu): tile loads start before griddepcontrol.wait,
     // every global write (TMA stores, metrics atomics) still waits for the predecessor to complete
     int early_loads;
     // completion counter of the (device, stream) record: chain_feed = 1: the last warp out adds 1; early_loads = 1:

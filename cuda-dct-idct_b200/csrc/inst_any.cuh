@@ -10,17 +10,8 @@ namespace b200dct {
 template <int TK, int QM, int PIX, bool FINV = false>
 static cudaError_t launch_one(const AnyParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl)
 {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    if constexpr (PIX == DT_U8) return cudaLaunchKernelEx(&cfg, k_any_u8<TK, QM, FINV>, P); // word-packed, no shared-memory stage
-    else return cudaLaunchKernelEx(&cfg, k_any<TK, QM, PIX, FINV>, P);
+    if constexpr (PIX == DT_U8) return launch_kernel<k_any_u8<TK, QM, FINV>>(P, grid, block, 0, s, pdl); // word-packed, no shared-memory stage
+    else return launch_kernel<k_any<TK, QM, PIX, FINV>>(P, grid, block, 0, s, pdl);
 }
 
 template <int PIX>

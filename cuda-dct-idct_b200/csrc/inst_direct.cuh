@@ -8,81 +8,39 @@ namespace b200dct {
 #define B200_CAT_(a, b) a##b
 #define B200_CAT(a, b) B200_CAT_(a, b)
 
-#define B200_DIRECT_CASE(M, X, F)                                                   \
-    if (mode == (M) && pix == (X) && finv == (F)) {                                 \
-        if (ctas_per_sm) {                                                          \
-            *ctas_per_sm = direct_ctas_per_sm<k_direct<M, INST_SPARSE, INST_Q, X, false, F>>(P.zz_smem ? ZZ_SMEM_BYTES : 0); \
-            return cudaSuccess;                                                     \
-        }                                                                           \
-        cudaLaunchConfig_t cfg = {};                                                \
-        cfg.gridDim = grid;                                                         \
-        cfg.blockDim = block;                                                       \
-        cfg.stream = s;                                                             \
-        cfg.dynamicSmemBytes = P.zz_smem ? ZZ_SMEM_BYTES : 0;                       \
-        cudaLaunchAttribute attr[1];                                                \
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;            \
-        attr[0].val.programmaticStreamSerializationAllowed = 1;                     \
-        cfg.attrs = attr;                                                           \
-        cfg.numAttrs = pdl ? 1 : 0;                                                 \
-        return cudaLaunchKernelEx(&cfg, k_direct<M, INST_SPARSE, INST_Q, X, false, F>, P); \
-    }
+#define B200_DIRECT_CASE(M, X, F, MET)                                              \
+    if (mode == (M) && pix == (X) && finv == (F) && metrics == (MET))               \
+        return launch_kernel<k_direct<M, INST_SPARSE, INST_Q, X, MET, F>>(P, grid, block, smem, s, pdl, ctas_per_sm);
 
 // ctas_per_sm != NULL: no launch, only the occupancy of the kernel the arguments select
-cudaError_t B200_CAT(launch_direct_, INST_TAG)(int mode, int pix, bool finv, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm)
+cudaError_t B200_CAT(launch_direct_, INST_TAG)(int mode, int pix, bool finv, bool metrics, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm)
 {
+    const size_t smem = P.zz_smem ? ZZ_SMEM_BYTES : 0;
     // finv: factored +-1 LSB inverse (Haweel's T, 8-bit pixel output only)
-    B200_DIRECT_CASE(MODE_RT, DT_F32, false)
-    B200_DIRECT_CASE(MODE_RT, DT_U8, false)
+    B200_DIRECT_CASE(MODE_RT, DT_F32, false, false)
+    B200_DIRECT_CASE(MODE_RT, DT_U8, false, false)
 #if INST_SPARSE == 1
-    B200_DIRECT_CASE(MODE_RT, DT_U8, true)
+    B200_DIRECT_CASE(MODE_RT, DT_U8, true, false)
 #endif
 #ifdef B200DCT_FAST_BUILD /* experiment builds: round trip only (+ f32 split for the default quantiser) */
 #if INST_Q == 0
-    B200_DIRECT_CASE(MODE_FWD, DT_F32, false)
-    B200_DIRECT_CASE(MODE_INV, DT_F32, false)
+    B200_DIRECT_CASE(MODE_FWD, DT_F32, false, false)
+    B200_DIRECT_CASE(MODE_INV, DT_F32, false, false)
 #endif
     return cudaErrorInvalidValue;
 #else
-    B200_DIRECT_CASE(MODE_FWD, DT_F32, false)
-    B200_DIRECT_CASE(MODE_FWD, DT_U8, false)
-    B200_DIRECT_CASE(MODE_INV, DT_F32, false)
-    B200_DIRECT_CASE(MODE_INV, DT_U8, false)
+    B200_DIRECT_CASE(MODE_FWD, DT_F32, false, false)
+    B200_DIRECT_CASE(MODE_FWD, DT_U8, false, false)
+    B200_DIRECT_CASE(MODE_INV, DT_F32, false, false)
+    B200_DIRECT_CASE(MODE_INV, DT_U8, false, false)
 #if INST_SPARSE == 1
-    B200_DIRECT_CASE(MODE_INV, DT_U8, true)
+    B200_DIRECT_CASE(MODE_INV, DT_U8, true, false)
+    B200_DIRECT_CASE(MODE_RT, DT_U8, true, true)
 #endif
+    B200_DIRECT_CASE(MODE_RT, DT_F32, false, true)
+    B200_DIRECT_CASE(MODE_RT, DT_U8, false, true)
     return cudaErrorInvalidValue;
 #endif
-}
-
-#define B200_METRICS_CASE(X, F)                                                     \
-    if (pix == (X) && finv == (F)) {                                                \
-        if (ctas_per_sm) {                                                          \
-            *ctas_per_sm = direct_ctas_per_sm<k_direct<MODE_RT, INST_SPARSE, INST_Q, X, true, F>>(0); \
-            return cudaSuccess;                                                     \
-        }                                                                           \
-        cudaLaunchConfig_t cfg = {};                                                \
-        cfg.gridDim = grid;                                                         \
-        cfg.blockDim = block;                                                       \
-        cfg.stream = s;                                                             \
-        cudaLaunchAttribute attr[1];                                                \
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;            \
-        attr[0].val.programmaticStreamSerializationAllowed = 1;                     \
-        cfg.attrs = attr;                                                           \
-        cfg.numAttrs = pdl ? 1 : 0;                                                 \
-        return cudaLaunchKernelEx(&cfg, k_direct<MODE_RT, INST_SPARSE, INST_Q, X, true, F>, P); \
-    }
-
-// ctas_per_sm != NULL: no launch, only the occupancy of the kernel the arguments select
-cudaError_t B200_CAT(launch_direct_metrics_, INST_TAG)(int pix, bool finv, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm)
-{
-#ifndef B200DCT_FAST_BUILD
-#if INST_SPARSE == 1
-    B200_METRICS_CASE(DT_U8, true)
-#endif
-    B200_METRICS_CASE(DT_F32, false)
-    B200_METRICS_CASE(DT_U8, false)
-#endif
-    return cudaErrorInvalidValue;
 }
 
 } // namespace b200dct

@@ -9,21 +9,7 @@ namespace b200dct {
 template <int QM, int PIX>
 static cudaError_t launch_one(const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm)
 {
-    if (ctas_per_sm) { // no launch, only the occupancy of this kernel
-        *ctas_per_sm = direct_ctas_per_sm<k_direct<MODE_RT, TK_HAWEEL, QM, PIX>>(P.zz_smem ? ZZ_SMEM_BYTES : 0);
-        return cudaSuccess;
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.stream = s;
-    cfg.dynamicSmemBytes = P.zz_smem ? ZZ_SMEM_BYTES : 0;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, k_direct<MODE_RT, TK_HAWEEL, QM, PIX>, P);
+    return launch_kernel<k_direct<MODE_RT, TK_HAWEEL, QM, PIX>>(P, grid, block, P.zz_smem ? ZZ_SMEM_BYTES : 0, s, pdl, ctas_per_sm);
 }
 
 template <int PIX>

@@ -5,16 +5,7 @@ namespace b200dct {
 
 cudaError_t launch_mma(bool fastdiv, const MmaParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl)
 {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    return fastdiv ? cudaLaunchKernelEx(&cfg, k_mma<true>, P) : cudaLaunchKernelEx(&cfg, k_mma<false>, P);
+    return fastdiv ? launch_kernel<k_mma<true>>(P, grid, block, 0, s, pdl) : launch_kernel<k_mma<false>>(P, grid, block, 0, s, pdl);
 }
 
 } // namespace b200dct

@@ -9,20 +9,10 @@ namespace b200dct {
 #define B200_TMA_CASE(M, X, F) B200_TMA_CASE_M(M, X, F, false)
 #define B200_TMA_CASE_M(M, X, F, MET)                                                                 \
     if (mode == (M) && pix == (X) && finv == (F) && (P.macc != nullptr) == (MET)) {                   \
-        auto kern = k_tma<M, INST_SPARSE, INST_Q, X, F, MET>;                                         \
+        constexpr auto kern = k_tma<M, INST_SPARSE, INST_Q, X, F, MET>;                               \
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         if (e != cudaSuccess) return e;                                                               \
-        cudaLaunchConfig_t cfg = {};                                                                  \
-        cfg.gridDim = dim3((unsigned)grid);                                                           \
-        cfg.blockDim = dim3((unsigned)block);                                                         \
-        cfg.dynamicSmemBytes = smem;                                                                  \
-        cfg.stream = s;                                                                               \
-        cudaLaunchAttribute attr[1];                                                                  \
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                              \
-        attr[0].val.programmaticStreamSerializationAllowed = 1;                                       \
-        cfg.attrs = attr;                                                                             \
-        cfg.numAttrs = pdl ? 1 : 0;                                                                   \
-        return cudaLaunchKernelEx(&cfg, kern, P);                                                     \
+        return launch_kernel<kern>(P, dim3((unsigned)grid), dim3((unsigned)block), smem, s, pdl);     \
     }
 
 cudaError_t B200_CAT(launch_tma_, INST_TAG)(int mode, int pix, bool finv, const TmaParams &P, int grid, int block, size_t smem, cudaStream_t s, bool pdl)

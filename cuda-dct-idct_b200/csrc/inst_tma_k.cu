@@ -8,20 +8,10 @@ namespace b200dct {
 template <int QM, int PIX>
 static cudaError_t launch_one(const TmaParams &P, int grid, int block, size_t smem, cudaStream_t s, bool pdl)
 {
-    auto kern = k_tma<MODE_RT, TK_HAWEEL, QM, PIX>;
+    constexpr auto kern = k_tma<MODE_RT, TK_HAWEEL, QM, PIX>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3((unsigned)block);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kern, P);
+    return launch_kernel<kern>(P, dim3((unsigned)grid), dim3((unsigned)block), smem, s, pdl);
 }
 
 template <int PIX>

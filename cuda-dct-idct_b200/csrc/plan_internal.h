@@ -24,31 +24,54 @@ struct b200dct_plan {
 
 
 namespace b200dct {
-// Early path of a hardware-scheduled (direct-style) kernel across a launch boundary, see "early loads" in
-// b200dct.cu: the scope holds the per-stream launch-order lock from the decision until done().
-struct EarlyParams {
-    int early = 0;                       // leading CTAs that may load and compute before griddepcontrol.wait
-    int chain_feed = 0;                  // trailing CTAs that add 1 to the completion counter at their end
-    unsigned long long *chain = nullptr; // completion counter of the (device, stream) record
-    unsigned long long chain_target = 0; // its value once the predecessor is complete
-};
-struct Span { const void *ptr; size_t pitch, row_bytes; int rows; };
-class EarlyScope {
+struct Span { const void *ptr; size_t pitch, row_bytes; int rows; }; // rows of row_bytes, pitch bytes apart
+// Every launch of a library kernel happens inside one of these (see "early loads" in b200dct.cu).  The scope
+// holds the launch-order lock from its decision until done() or its end, so that the per-(device, stream)
+// record of the last launch follows stream order even when several host threads launch on one stream.
+class LaunchScope {
 public:
-    // usable: programmatic dependent launch is on for this launch and the stream is not capturing;
-    // ctas_per_sm: occupancy of the kernel about to be launched; rd: the plane it reads (ptr NULL: never early)
-    EarlyScope(cudaStream_t s, bool usable, unsigned long long ctas, int ctas_per_sm, Span rd, Span w0, Span w1);
-    ~EarlyScope();
-    const EarlyParams &params() const { return p_; }
+    // DIRECT: hardware-scheduled 128-thread CTAs (direct family, colour), ctas_per_sm = the kernel's occupancy;
+    // TMA: persistent kernel, ctas_per_sm = 1.  usable: programmatic dependent launch is on for this launch, the
+    // stream is not capturing, and (TMA) the kernel feeds the completion counter and no two of its CTAs fit on
+    // one SM.  rd: the plane the launch reads (ptr NULL: never early); w0..w2: the planes it writes.
+    enum Family { NONE, DIRECT, TMA };
+    LaunchScope(cudaStream_t s, Family family, bool usable, unsigned long long ctas, int ctas_per_sm, Span rd, Span w0,
+                Span w1 = Span{}, Span w2 = Span{});
+    // a launch (or several) that does not take part in the early path: the record is left cleared
+    explicit LaunchScope(cudaStream_t s) : LaunchScope(s, NONE, false, 0, 0, Span{}, Span{}) {}
+    ~LaunchScope() { done(false); }
+    LaunchScope(const LaunchScope &) = delete;
+    LaunchScope &operator=(const LaunchScope &) = delete;
+    // the decision in the kernel's parameters
+    template <class DirectStyleParams> // DirectParams, RgbParams
+    void apply(DirectStyleParams &P) const
+    {
+        P.early = early_;
+        P.chain_feed = chain_feed_;
+        P.chain = chain_;
+        P.chain_target = chain_target_;
+    }
+    void apply(TmaParams &P) const
+    {
+        P.early_loads = early_;
+        P.chain_feed = chain_feed_;
+        P.chain = chain_;
+        P.chain_target = chain_target_;
+    }
+    // launched: the scope's kernels are in the stream and the record describes them from now on; releases the lock
     void done(bool launched);
 private:
-    EarlyParams p_;
-    void *rec_;    // the (device, stream) record of b200dct.cu
-    Span w_[2];
-    bool feeds_, finished_;
+    Family family_;
+    int early_ = 0;                       // leading CTAs that may load before griddepcontrol.wait (TMA: 1 = early tile loads)
+    int chain_feed_ = 0;                  // what the kernel adds to the completion counter in total
+    unsigned long long *chain_ = nullptr; // completion counter of the (device, stream) record
+    unsigned long long chain_target_ = 0; // its value once the predecessor is complete
+    void *rec_ = nullptr;                 // the (device, stream) record of b200dct.cu
+    Span w_[3];
+    bool finished_ = false;
 };
 void note_launch(int launches, const char *path); // b200dct_last_launch_count / b200dct_last_path of this thread
 bool use_factored_inverse_u8(const b200dct_plan *pl);
-bool pdl_enabled(cudaStream_t s);
-void forget_stream(cudaStream_t s); // a non-TMA kernel of the library was launched on s (see early loads, b200dct.cu)
+bool stream_capturing(cudaStream_t s);
+bool pdl_enabled(bool capturing); // programmatic dependent launch for a launch on a (non-)capturing stream
 }
