@@ -48,51 +48,6 @@ static Unit unit_of(int tk, int q)
 
 using namespace b200dct;
 
-// Sums n CTA partial triples in a fixed order and ADDS the totals into acc[0..2].  One CTA (the
-// order of the additions must not depend on scheduling); latency-bound, so every thread issues
-// the loads of 8 strided triples before it adds them.
-constexpr int REDUCE_THREADS = 1024;
-static __global__ void __launch_bounds__(REDUCE_THREADS) k_reduce_partials(const double *__restrict__ partials, size_t n, double *acc)
-{
-    __shared__ double red[3][REDUCE_THREADS];
-    double v[3] = {0.0, 0.0, 0.0};
-    size_t i = threadIdx.x;
-    for (; i + 7 * REDUCE_THREADS < n; i += 8 * REDUCE_THREADS) {
-        double t[8][3];
-#pragma unroll
-        for (int u = 0; u < 8; u++)
-#pragma unroll
-            for (int q = 0; q < 3; q++) t[u][q] = partials[(i + (size_t)u * REDUCE_THREADS) * 3 + q];
-#pragma unroll
-        for (int u = 0; u < 8; u++)
-#pragma unroll
-            for (int q = 0; q < 3; q++) v[q] += t[u][q];
-    }
-    for (; i < n; i += REDUCE_THREADS)
-        for (int q = 0; q < 3; q++) v[q] += partials[i * 3 + q];
-    for (int q = 0; q < 3; q++) red[q][threadIdx.x] = v[q];
-    __syncthreads();
-    for (int s = REDUCE_THREADS / 2; s > 0; s >>= 1) {
-        if ((int)threadIdx.x < s)
-            for (int q = 0; q < 3; q++) red[q][threadIdx.x] += red[q][threadIdx.x + s];
-        __syncthreads();
-    }
-    if (threadIdx.x < 3) acc[threadIdx.x] += red[threadIdx.x][0];
-}
-
-// TMA-family metrics: the kernel leaves exact integer sums in macc[0..MACC_WORDS) (128-bit fixed point, dct_kernels.cuh)
-static __global__ void k_finish_fixed_point(const unsigned long long *macc, double *acc)
-{
-    if (threadIdx.x < 2) acc[threadIdx.x] += u128_to_double(macc[2 * threadIdx.x], macc[2 * threadIdx.x + 1]) / METRICS_FIXED_POINT;
-    if (threadIdx.x == 2) acc[2] += (double)macc[4];
-}
-
-static cudaError_t reduce_partials_sparse(const double *partials, size_t n, double *acc, cudaStream_t s)
-{
-    k_reduce_partials<<<1, REDUCE_THREADS, 0, s>>>(partials, n, acc);
-    return cudaGetLastError();
-}
-
 #include "plan_internal.h"
 
 static thread_local int tl_launches = 0;
@@ -433,6 +388,24 @@ unsigned long long *sched_macc(const uint32_t *slot)
     if (!slot || cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64 || !g_sched.base[dev]) return nullptr;
     return g_sched.macc[dev] + MACC_WORDS * ((slot - g_sched.base[dev]) / 2);
 }
+// The counters of a fused-metrics launch: those of its scheduler slot, or without one (capture pool used up,
+// B200DCT_TMA_STATIC=1, failed ring allocation) the caller's workspace, laid out as
+// {u64 macc[MACC_WORDS]; u32 pair[2]}.  The kernel leaves either zeroed; the workspace starts unknown, so a launch on it
+// is preceded by a memset on its stream and takes no part in the early path.
+constexpr size_t METRICS_WORKSPACE_BYTES = MACC_WORDS * sizeof(unsigned long long) + 2 * sizeof(uint32_t);
+struct MetricsCounters {
+    uint32_t *pair; // {next ticket, finished CTAs / warps}
+    unsigned long long *macc;
+    bool in_workspace;
+    // inside the launch's scope, ahead of the kernel
+    cudaError_t zero(cudaStream_t s) const { return in_workspace ? cudaMemsetAsync(macc, 0, METRICS_WORKSPACE_BYTES, s) : cudaSuccess; }
+};
+MetricsCounters metrics_counters(uint32_t *slot, void *workspace)
+{
+    if (unsigned long long *macc = sched_macc(slot)) return MetricsCounters{slot, macc, false};
+    auto *macc = static_cast<unsigned long long *>(workspace);
+    return MetricsCounters{reinterpret_cast<uint32_t *>(macc + MACC_WORDS), macc, true};
+}
 } // namespace
 
 // ---- early tile loads across launch boundaries
@@ -697,7 +670,7 @@ static Span plane_span(const Plane &p, int H, int W)
 }
 
 static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef, float *shifted, int H, int W,
-               cudaStream_t stream, double *partials = nullptr, double *acc = nullptr)
+               cudaStream_t stream, void *workspace = nullptr, double *acc = nullptr)
 {
     tl_launches = 0;
     if (!pl) return B200DCT_ERR_ARG;
@@ -714,7 +687,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
 
     const int pix = (mode == MODE_INV) ? out.dt : in.dt;
     const int coef_dt = (mode == MODE_FWD) ? out.dt : (mode == MODE_INV ? in.dt : (coef.ptr ? coef.dt : DT_F32));
-    const Variant v = variant_of(pl, mode, pix, partials != nullptr); // the metrics kernels take runtime masks
+    const Variant v = variant_of(pl, mode, pix, workspace != nullptr); // the metrics kernels take runtime masks
 
     // AUTO: the TMA family wins where the call is HBM-bound (>= 4 bytes moved per pixel: any
     // f32/i16 plane); all-u8 round trips move 2 B/px, are instruction-issue bound, and run faster
@@ -751,7 +724,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     });
     // fused metrics on the TMA family: f32 round trips of Haweel's T (the input tile is compared where it
     // already is, in shared memory); everything else takes the direct family's metrics kernels
-    const bool metrics_tma_ok = !partials || (mode == MODE_RT && in.dt == DT_F32 && pl->tk == TK_HAWEEL && in.ptr != out.ptr);
+    const bool metrics_tma_ok = !workspace || (mode == MODE_RT && in.dt == DT_F32 && pl->tk == TK_HAWEEL && in.ptr != out.ptr);
     const bool tma_possible = pl->path != B200DCT_PATH_DIRECT && prefer_tma && !shifted && metrics_tma_ok && get_encode() != nullptr &&
                               tma_plane_ok(in.ptr, in.dt, in.pitch, W) && tma_plane_ok(out.ptr, out.dt, out.pitch, W) &&
                               (!coef.ptr || tma_plane_ok(coef.ptr, coef.dt, coef.pitch, W));
@@ -761,7 +734,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     if (pl->path == B200DCT_PATH_TMA && !use_tma) return B200DCT_ERR_ALIGN;
     const Span rd = plane_span(in, H, W), w0 = plane_span(out, H, W), w1 = plane_span(coef, H, W);
     // the tensor-core arm of the dense variant (opt-in): f32 fused round trips, optional f32 coefficient plane
-    if (pl->dense == B200DCT_DENSE_MMA && !pl->sparse && mode == MODE_RT && in.dt == DT_F32 && !partials && !shifted &&
+    if (pl->dense == B200DCT_DENSE_MMA && !pl->sparse && mode == MODE_RT && in.dt == DT_F32 && !workspace && !shifted &&
         (!coef.ptr || coef.dt == DT_F32)) {
         MmaParams M;
         memset(&M, 0, sizeof(M));
@@ -803,10 +776,10 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
         P.buf_bytes = buf;
         // warps per CTA: the flavour's CTA size (8 for sparse-T f32; all the CTA holds for the
         // FP32-bound u8 and dense-T flavours), limited by 227 KiB of shared memory
-        const int max_w = (partials ? B200DCT_TMA_CTA_THREADS_METRICS : tma_cta_threads(pix, pl->tk)) / 32;
-        int nw = tma_warps > 0 ? tma_warps : (pix == DT_U8 || !pl->sparse || partials ? max_w : B200DCT_TMA_DEFAULT_WARPS);
+        const int max_w = (workspace ? B200DCT_TMA_CTA_THREADS_METRICS : tma_cta_threads(pix, pl->tk)) / 32;
+        int nw = tma_warps > 0 ? tma_warps : (pix == DT_U8 || !pl->sparse || workspace ? max_w : B200DCT_TMA_DEFAULT_WARPS);
         if (nw > max_w) nw = max_w;
-        const unsigned nbuf = partials ? 3u : 2u; // metrics: two input buffers per warp
+        const unsigned nbuf = workspace ? 3u : 2u; // metrics: two input buffers per warp
         const int smem_w = (int)((227u * 1024u - 1024u) / (nbuf * buf + 16u));
         if (nw > smem_w) nw = smem_w;
         const size_t smem = (size_t)nw * nbuf * buf + (size_t)nw * 16 + 1024;
@@ -817,36 +790,27 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
         P.run = (uint32_t)tma_max_run;
         const unsigned long long tail = 2ull * (unsigned long long)grid * nw;
         P.run_tickets = nt > tail ? (uint32_t)((nt - tail) / P.run) : 0u;
-        // Metrics: with the dynamic scheduler the slot owns a zeroed integer accumulator and the last warp out
-        // folds it into acc -- one launch.  Static split: the first MACC_WORDS words of the caller's workspace,
-        // zeroed before and folded after the kernel by a second one.
-        if (partials) {
-            P.macc = sched_macc(P.sched);
+        // Metrics: the dynamic scheduler always, on the counters of the slot or of the workspace; the last warp out
+        // folds the integer sums into acc -- one launch
+        MetricsCounters mc{};
+        if (workspace) {
+            mc = metrics_counters(P.sched, workspace);
+            P.sched = mc.pair;
+            P.macc = mc.macc;
             P.acc = acc;
         }
-        const bool separate_finish = partials && !P.macc;
         // the argument above needs the predecessor to occupy every SM (grid == SM count) and neither
         // launch to fit beside the other on one SM: both take more than half of its shared memory
         const bool heavy = smem > (size_t)(di.smem_optin / 2) + 1024;
-        LaunchScope scope(stream, separate_finish ? LaunchScope::NONE : LaunchScope::TMA, pdl && !capturing && heavy && P.sched != nullptr,
+        LaunchScope scope(stream, mc.in_workspace ? LaunchScope::NONE : LaunchScope::TMA, pdl && !capturing && heavy && P.sched != nullptr,
                           (unsigned long long)grid, 1, rd, w0, w1);
         scope.apply(P);
-        if (separate_finish) {
-            P.acc = nullptr;
-            P.macc = reinterpret_cast<unsigned long long *>(partials);
-            const cudaError_t em = cudaMemsetAsync(P.macc, 0, MACC_WORDS * sizeof(unsigned long long), stream);
-            if (em != cudaSuccess) return (int)em;
-        }
-        cudaError_t e = launch_tma(pl->tk, v, mode, pix, P, grid, nw * 32, smem, stream, pdl && !separate_finish);
+        const cudaError_t em = mc.zero(stream);
+        if (em != cudaSuccess) return (int)em;
+        const cudaError_t e = launch_tma(pl->tk, v, mode, pix, P, grid, nw * 32, smem, stream, pdl && !mc.in_workspace);
         if (e != cudaSuccess) return (int)e;
-        tl_launches = 1;
-        if (separate_finish) {
-            k_finish_fixed_point<<<1, 32, 0, stream>>>(P.macc, acc);
-            e = cudaGetLastError();
-            if (e != cudaSuccess) return (int)e;
-            tl_launches = 2;
-        }
         scope.done(true);
+        tl_launches = 1;
         tl_path = "tma";
         return B200DCT_OK;
     }
@@ -859,7 +823,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     P.shifted = shifted; P.shifted_pitch = in.pitch;
     P.bx = W / 8; P.by = H / 8;
     P.coef_dt = coef_dt;
-    P.zz_smem = (coef_dt == DT_I16ZZ && !partials) ? 1 : 0; // the metrics kernels are launched without dynamic smem
+    P.zz_smem = (coef_dt == DT_I16ZZ && !workspace) ? 1 : 0; // the metrics kernels are launched without dynamic smem
     if (direct_v8()) { // f32 planes aligned to 32 bytes move with 256-bit accesses
         auto aligned32 = [](const Plane &pl) { return pl.ptr && pl.dt == DT_F32 && !((uintptr_t)pl.ptr & 31) && !(pl.pitch & 31); };
         P.v8 = (aligned32(in) ? 1 : 0) | (aligned32(out) ? 2 : 0) | (aligned32(coef) ? 4 : 0);
@@ -868,41 +832,30 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     dim3 block(32, 4);
     dim3 grid((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32));
     if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
-    const bool metrics = partials != nullptr;
+    const bool metrics = workspace != nullptr;
+    MetricsCounters mc{};
     if (metrics) {
         if (mode != MODE_RT || in.ptr == out.ptr) return B200DCT_ERR_ARG;
-        // One launch: integer sums through 64-bit atomics into the triple that belongs to a ticket-counter pair,
-        // the last CTA out folds them into acc (the TMA family's scheme).  Dependent launch and the early path apply.
-        uint32_t *slot = sched_slot(capturing);
-        unsigned long long *macc = sched_macc(slot);
-        if (!macc) {
-            // no counter pair (capture without a free slot): per-CTA partials, then one fixed-order reduction into acc[0..2]
-            LaunchScope order(stream);
-            P.partials = partials;
-            cudaError_t e = launch_direct(pl->tk, v, mode, pix, true, P, grid, block, stream, false);
-            if (e != cudaSuccess) return (int)e;
-            e = reduce_partials_sparse(partials, (size_t)grid.x * grid.y, acc, stream);
-            if (e != cudaSuccess) return (int)e;
-            tl_launches = 2;
-            tl_path = "direct";
-            return B200DCT_OK;
-        }
-        P.macc = macc;
-        P.mdone = slot;
+        // One launch: integer sums through 64-bit atomics into the accumulator of a ticket-counter pair, the last
+        // CTA out folds them into acc (the TMA family's scheme).  Dependent launch and the early path apply on a slot.
+        mc = metrics_counters(sched_slot(capturing), workspace);
+        P.macc = mc.macc;
+        P.mdone = mc.pair;
         P.acc = acc;
-        P.metrics_scale = pix == DT_U8 ? 1.0 : METRICS_FIXED_POINT;
     }
-    const bool usable = pdl && !capturing;
+    const bool usable = pdl && !capturing && !mc.in_workspace;
     int per_sm = 0;
     if (usable) launch_direct(pl->tk, v, mode, pix, metrics, P, grid, block, stream, pdl, &per_sm);
     // the early path: fused round trips without a coefficient plane, forward calls without the X-128 write-back,
     // inverse calls whose coefficients are a plane (not the zig-zag stream)
     const bool may_load_early = !coef.ptr && !shifted && !(mode == MODE_INV && in.dt == DT_I16ZZ);
     const Span w2 = metrics ? Span{acc, 0, 3 * sizeof(double), 1} : Span{shifted, in.pitch, (size_t)W * 4, H};
-    LaunchScope scope(stream, LaunchScope::DIRECT, usable, (unsigned long long)grid.x * grid.y, per_sm, may_load_early ? rd : Span{}, w0,
-                      w1, w2);
+    LaunchScope scope(stream, mc.in_workspace ? LaunchScope::NONE : LaunchScope::DIRECT, usable, (unsigned long long)grid.x * grid.y,
+                      per_sm, may_load_early ? rd : Span{}, w0, w1, w2);
     scope.apply(P);
-    const cudaError_t e = launch_direct(pl->tk, v, mode, pix, metrics, P, grid, block, stream, pdl);
+    const cudaError_t em = mc.zero(stream);
+    if (em != cudaSuccess) return (int)em;
+    const cudaError_t e = launch_direct(pl->tk, v, mode, pix, metrics, P, grid, block, stream, pdl && !mc.in_workspace);
     if (e != cudaSuccess) return (int)e;
     scope.done(true);
     tl_launches = 1;
@@ -1045,11 +998,7 @@ extern "C" int b200dct_roundtrip_any(const b200dct_plan *plan, const void *img, 
 
 extern "C" size_t b200dct_metrics_workspace_bytes(int H, int W)
 {
-    if (H <= 0 || W <= 0) return 0;
-    const size_t ctas = (size_t)((H / 8 + 3) / 4) * (size_t)((W / 8 + 31) / 32);
-    // per-CTA partials of the direct family, or the TMA family's integer accumulator
-    const size_t partials = ctas * 3 * sizeof(double), fixed = MACC_WORDS * sizeof(unsigned long long);
-    return partials > fixed ? partials : fixed;
+    return H > 0 && W > 0 ? METRICS_WORKSPACE_BYTES : 0;
 }
 
 extern "C" int b200dct_roundtrip_metrics(const b200dct_plan *plan, const void *img, b200dct_dtype in_dt, size_t in_pitch,
@@ -1060,7 +1009,7 @@ extern "C" int b200dct_roundtrip_metrics(const b200dct_plan *plan, const void *i
     if (!d_acc3 || !workspace || workspace_bytes < b200dct_metrics_workspace_bytes(H, W) || ((uintptr_t)workspace & 7))
         return B200DCT_ERR_ARG;
     return run(plan, MODE_RT, Plane{img, (int)in_dt, in_pitch}, Plane{out, (int)out_dt, out_pitch},
-               Plane{coef_or_null, (int)coef_dt, coef_pitch}, nullptr, H, W, (cudaStream_t)stream, (double *)workspace,
+               Plane{coef_or_null, (int)coef_dt, coef_pitch}, nullptr, H, W, (cudaStream_t)stream, workspace,
                d_acc3);
 }
 

@@ -145,6 +145,17 @@ __host__ __device__ __forceinline__ double u128_to_double(unsigned long long lo,
 {
     return (double)hi * 0x1p64 + (double)lo;
 }
+// the last CTA / warp out of a metrics launch, once every other one's sums are in: takes the totals out of
+// macc[0..MACC_WORDS) (leaving it zeroed for the next launch) and adds them into acc[0..2], the two sums divided by scale
+__device__ __forceinline__ void metrics_fold(unsigned long long *macc, double *acc, double scale)
+{
+    __threadfence();
+    unsigned long long t[MACC_WORDS];
+    sfor<MACC_WORDS>([&](auto q) { t[IC(q)] = atomicExch(&macc[IC(q)], 0ull); });
+    acc[0] += u128_to_double(t[0], t[1]) / scale;
+    acc[1] += u128_to_double(t[2], t[3]) / scale;
+    acc[2] += (double)t[4];
+}
 constexpr int DIRECT_BATCH_MAX = 64; // images per launch of the batch entry point (1 KiB of kernel parameters)
 struct DirectParams {
     const void *in;   // FWD/RT: pixels (PIX dtype); INV: coefficients (coef_dt)
@@ -154,15 +165,13 @@ struct DirectParams {
     size_t in_pitch, out_pitch, coef_pitch, shifted_pitch; // bytes
     int bx, by;       // blocks per row / block rows
     int coef_dt;      // DT_F32 / DT_I16
-    double *partials; // METRICS kernels, two-launch form: 3 doubles per CTA {sum (x-y)^2, sum x^2, non-zero coefficients}
-    // METRICS kernels, one-launch form (macc != NULL): every CTA adds its integer sums {sum (x-y)^2, sum x^2} (u8: exact
+    // METRICS kernels: every CTA adds its integer sums {sum (x-y)^2, sum x^2} (u8: exact
     // integers; f32: per-block float sums as 128-bit fixed point in units of 2^-50, the TMA family's convention) and its
     // non-zero count to macc[0..MACC_WORDS) with 64-bit atomics (order-independent => deterministic); the last CTA out
-    // (mdone[1] counts them) adds the totals, divided by metrics_scale, into acc[0..2] and leaves macc and the counter zeroed
+    // (mdone[1] counts them) adds the totals (f32: divided by 2^50) into acc[0..2] and leaves macc and the counter zeroed
     unsigned long long *macc;
     uint32_t *mdone;
     double *acc;
-    double metrics_scale;
     int zz_smem;      // 1: the launch carries ZZ_SMEM_BYTES of dynamic shared memory for the zig-zag stream transpose
     // batch of separately allocated images of one shape (b200dct_roundtrip_batch): image z of the launch
     // is blockIdx.z, its planes come from these tables instead of in / out (pixels only: no coefficient
@@ -326,8 +335,8 @@ __device__ __forceinline__ void shift_row(float2 (&r)[4], float s)
 
 // METRICS (round trip only): the kernel also accumulates, per CTA, the squared error and the
 // signal energy between the pixels it read and the pixels it wrote (as stored: u8 after
-// clamp+truncate) and the number of non-zero quantised coefficients, and writes them to
-// P.partials[cta]; k_reduce_partials then adds them up in a fixed order (deterministic).
+// clamp+truncate) and the number of non-zero quantised coefficients, adds them to P.macc as
+// integers, and its last CTA out folds the totals into P.acc (see DirectParams).
 // The input row is re-read at the end (an L2 hit) instead of being kept in 64 registers.
 // Occupancy of the direct family: 5 CTAs of 128 threads per SM (<= 96 registers, 24-40 bytes of
 // spill) instead of the 4 that the unconstrained 128 registers allow.  Same box, 8192^2
@@ -491,68 +500,44 @@ __global__ void __launch_bounds__(128, METRICS ? B200DCT_METRICS_MIN_BLOCKS : B2
         (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x + (unsigned)P.chain_feed >= gridDim.x * gridDim.y * gridDim.z)
         atomicAdd(P.chain, 1ull); // one of the last CTAs of the grid is (as good as) done
     if constexpr (METRICS) {
-        if (P.macc) { // one-launch form
-            using Acc = std::conditional_t<PIX == DT_U8, unsigned long long, U128>;
-            Acc v[2] = {Acc{}, Acc{}};
-            unsigned long long nz = 0;
-            if (valid) {
-                if constexpr (PIX == DT_U8) {
-                    v[0] = i_xx + i_yy - 2u * i_xy;
-                    v[1] = i_xx;
-                } else {
-                    v[0] = metrics_fixed(m_sse);
-                    v[1] = metrics_fixed(m_en);
-                }
-                nz = (unsigned long long)m_nnz;
+        using Acc = std::conditional_t<PIX == DT_U8, unsigned long long, U128>;
+        Acc v[2] = {Acc{}, Acc{}};
+        unsigned long long nz = 0;
+        if (valid) {
+            if constexpr (PIX == DT_U8) {
+                v[0] = i_xx + i_yy - 2u * i_xy;
+                v[1] = i_xx;
+            } else {
+                v[0] = metrics_fixed(m_sse);
+                v[1] = metrics_fixed(m_en);
             }
-            __shared__ Acc ired[2][4];
-            __shared__ unsigned long long inz[4];
-            const int lane = threadIdx.x, w = threadIdx.y;
-            for (int o = 16; o > 0; o >>= 1) {
-                v[0] = acc_add(v[0], acc_shfl_xor(v[0], o));
-                v[1] = acc_add(v[1], acc_shfl_xor(v[1], o));
-                nz += __shfl_xor_sync(0xffffffffu, nz, o);
-            }
-            if (lane == 0) {
-                ired[0][w] = v[0];
-                ired[1][w] = v[1];
-                inz[w] = nz;
-            }
-            __syncthreads();
-            if (w == 0 && lane == 0) {
-                sfor<2>([&](auto q) {
-                    atomic_add_u128(&P.macc[2 * IC(q)], acc_wide(acc_add(acc_add(ired[IC(q)][0], ired[IC(q)][1]), acc_add(ired[IC(q)][2], ired[IC(q)][3]))));
-                });
-                atomicAdd(&P.macc[4], (inz[0] + inz[1]) + (inz[2] + inz[3]));
-                __threadfence();
-                if (atomicAdd(&P.mdone[1], 1u) == gridDim.x * gridDim.y - 1u) { // every other CTA's sums are in
-                    __threadfence();
-                    unsigned long long t[MACC_WORDS];
-                    sfor<MACC_WORDS>([&](auto q) { t[IC(q)] = atomicExch(&P.macc[IC(q)], 0ull); });
-                    P.acc[0] += u128_to_double(t[0], t[1]) / P.metrics_scale;
-                    P.acc[1] += u128_to_double(t[2], t[3]) / P.metrics_scale;
-                    P.acc[2] += (double)t[4];
-                    P.mdone[1] = 0;
-                    __threadfence();
-                }
-            }
-            return;
+            nz = (unsigned long long)m_nnz;
         }
-        if constexpr (PIX == DT_U8) {
-            m_sse = (float)(i_xx + i_yy - 2u * i_xy);
-            m_en = (float)i_xx;
-        }
-        double v[3] = {valid ? (double)m_sse : 0.0, valid ? (double)m_en : 0.0, valid ? (double)m_nnz : 0.0};
-        __shared__ double red[3][4];
+        __shared__ Acc ired[2][4];
+        __shared__ unsigned long long inz[4];
         const int lane = threadIdx.x, w = threadIdx.y;
-        sfor<3>([&](auto q) {
-            for (int o = 16; o > 0; o >>= 1) v[IC(q)] += __shfl_xor_sync(0xffffffffu, v[IC(q)], o);
-            if (lane == 0) red[IC(q)][w] = v[IC(q)];
-        });
+        for (int o = 16; o > 0; o >>= 1) {
+            v[0] = acc_add(v[0], acc_shfl_xor(v[0], o));
+            v[1] = acc_add(v[1], acc_shfl_xor(v[1], o));
+            nz += __shfl_xor_sync(0xffffffffu, nz, o);
+        }
+        if (lane == 0) {
+            ired[0][w] = v[0];
+            ired[1][w] = v[1];
+            inz[w] = nz;
+        }
         __syncthreads();
-        if (w == 0 && lane < 3) {
-            const size_t cta = (size_t)blockIdx.y * gridDim.x + blockIdx.x;
-            P.partials[cta * 3 + lane] = (red[lane][0] + red[lane][1]) + (red[lane][2] + red[lane][3]);
+        if (w == 0 && lane == 0) {
+            sfor<2>([&](auto q) {
+                atomic_add_u128(&P.macc[2 * IC(q)], acc_wide(acc_add(acc_add(ired[IC(q)][0], ired[IC(q)][1]), acc_add(ired[IC(q)][2], ired[IC(q)][3]))));
+            });
+            atomicAdd(&P.macc[4], (inz[0] + inz[1]) + (inz[2] + inz[3]));
+            __threadfence();
+            if (atomicAdd(&P.mdone[1], 1u) == gridDim.x * gridDim.y - 1u) { // every other CTA's sums are in
+                metrics_fold(P.macc, P.acc, PIX == DT_U8 ? 1.0 : METRICS_FIXED_POINT);
+                P.mdone[1] = 0;
+                __threadfence();
+            }
         }
     }
 }
@@ -574,7 +559,7 @@ struct TmaParams {
     int coef_dt;          // DT_F32 / DT_I16
     int has_coef;         // RT: also emit the coefficient plane
     // Dynamic tile scheduler: {next ticket, finished warps}, both 0 at launch and reset to 0
-    // by the last warp to leave; NULL = static round-robin (used under stream capture).
+    // by the last warp to leave; NULL = static round-robin (launches without metrics only).
     uint32_t *sched;
     uint32_t run;         // tiles per ticket for the first run_tickets tickets, then 1
     uint32_t run_tickets;
@@ -583,7 +568,7 @@ struct TmaParams {
     // non-zero coefficients (MACC_WORDS words), accumulated with 64-bit integer atomics (order-independent
     // => deterministic)
     unsigned long long *macc;
-    double *acc;          // METRICS with the dynamic scheduler: the last warp out adds macc into acc[0..2] and re-zeroes macc
+    double *acc;          // METRICS (always with the dynamic scheduler): the last warp out adds macc into acc[0..2] and re-zeroes macc
     // 1: the host has established that nothing this launch READS is written by the launch it may
     // overlap with (see LaunchScope in b200dct.cu): tile loads start before griddepcontrol.wait,
     // every global write (TMA stores, metrics atomics) still waits for the predecessor to complete
@@ -980,16 +965,8 @@ __global__ void B200DCT_TMA_BOUNDS k_tma(const __grid_constant__ TmaParams P)
             // every warp ends on exactly one losing ticket; the last warp out re-zeroes both counters
             __threadfence();
             if (atomicAdd(&sched[1], 1u) == stride - 1) {
-                if constexpr (METRICS) {
-                    if (P.acc) { // every other warp's sums are in (its atomics precede its fence + ticket)
-                        __threadfence();
-                        unsigned long long t[MACC_WORDS];
-                        sfor<MACC_WORDS>([&](auto q) { t[IC(q)] = atomicExch(&P.macc[IC(q)], 0ull); });
-                        P.acc[0] += u128_to_double(t[0], t[1]) / METRICS_FIXED_POINT;
-                        P.acc[1] += u128_to_double(t[2], t[3]) / METRICS_FIXED_POINT;
-                        P.acc[2] += (double)t[4];
-                    }
-                }
+                // every other warp's sums are in (its atomics precede its fence + ticket)
+                if constexpr (METRICS) metrics_fold(P.macc, P.acc, METRICS_FIXED_POINT);
                 sched[0] = 0;
                 sched[1] = 0;
                 if (P.chain_feed) atomicAdd(P.chain, 1ull); // this launch is (as good as) complete

@@ -225,20 +225,20 @@ int b200dct_roundtrip_any(const b200dct_plan *plan, const void *img, b200dct_dty
  *   d_acc3[0] += sum (x - y)^2     d_acc3[1] += sum x^2     d_acc3[2] += non-zero quantised coefficients
  * so MSE = acc[0]/(H*W), PEEN% = 100*sqrt(acc[0]/acc[1]) (the definitions recovered from
  * README.md:67-68 of the reference) and the coefficient density need no second pass over the
- * images.  `workspace`: device, >= b200dct_metrics_workspace_bytes, caller-owned, 8-byte aligned.
+ * images.  `workspace`: device, >= b200dct_metrics_workspace_bytes, caller-owned, 8-byte aligned.  It holds
+ * the call's counters when no scheduler slot is free (under stream capture with the capture pool used up,
+ * or B200DCT_TMA_STATIC=1), so one workspace must not serve two calls that are in flight at once.
  * `out` must not alias `img`.  Large f32 images of Haweel's T run the TMA family's metrics kernel (the
- * error is taken from the input tile in shared memory); everything else the direct family's.
+ * error is taken from the input tile in shared memory); everything else the direct family's.  Every call
+ * is one launch, and its result is the same bit for bit on every path, including capture with an empty pool.
  * Range and accuracy:
- *   u8 images: exact integers, in one launch (or, under stream capture without a free scheduler slot,
- *     per-CTA partials in `workspace` reduced in a fixed order).
+ *   u8 images: exact integers.
  *   f32 images: each 8x8 block's two sums are taken in f32 in a fixed order, converted exactly to 128-bit
  *     fixed point in units of 2^-50 and added as integers, so the result does not depend on scheduling:
  *     run to run and between the two kernel families it is the same bit for bit.  The sums are exact
  *     to within 2^-50 per block, and the totals may reach 2^78 (2^22 blocks, a 16384^2 image, of pixels
  *     up to 2^20 sum to 2^68).  The relative error is that of the per-block f32 sums (measured <= 1e-6 for
- *     pixels of magnitude 2^-10 .. 2^20 with the quantiser scaled alike, tests/test_gpu_range.py).
- *     Without a free scheduler slot under capture the f32 direct path falls back to per-CTA double
- *     partials reduced in a fixed order: deterministic too, but its last bits can differ. */
+ *     pixels of magnitude 2^-10 .. 2^20 with the quantiser scaled alike, tests/test_gpu_range.py). */
 size_t b200dct_metrics_workspace_bytes(int H, int W);
 int b200dct_roundtrip_metrics(const b200dct_plan *plan,
                               const void *img, b200dct_dtype in_dt, size_t in_pitch,

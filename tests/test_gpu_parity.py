@@ -239,7 +239,7 @@ def test_host_roundtrip_and_metrics(dct, oracle):
 def test_fused_metrics(dct, oracle, shape):
     """b200dct_roundtrip_metrics: pixels identical to the plain round trip; MSE/PEEN equal the
     oracle's double-precision values (u8: exactly, the in-kernel sums are integers;
-    f32: to 1e-6 relative, the in-kernel partials are float) -- spec tolerance is 1e-3;
+    f32: to 1e-6 relative, the in-kernel per-block sums are float) -- spec tolerance is 1e-3;
     non-zero count equals the coefficient plane's."""
     img8 = oracle.rand_image_u8(*shape, 7)
     want8, wcoef = oracle.roundtrip(img8, want_coef=True)
@@ -605,7 +605,7 @@ def test_fused_metrics_tma_family(dct, oracle, shape):
         assert m1 == pytest.approx(oracle.metrics(img, oracle.roundtrip(img))[0], rel=1e-6)
         assert dct.api.last_path() == path and dct.api.last_launch_count() == 1   # one launch on both families
         both[path] = (m1, p1, n1)
-    # same per-block float sums, same 2^-12 fixed point, integer accumulation: the families agree bit for bit
+    # same per-block float sums, same 2^-50 fixed point, integer accumulation: the families agree bit for bit
     assert both["tma"] == both["direct"]
     # and the direct family's integer accumulation does not depend on the CTA schedule either
     seen = {dct.roundtrip_with_metrics(x, plan=dct.Plan(path=PATHS["direct"]))[1] for _ in range(4)}
