@@ -2,7 +2,7 @@
 """The reference README's accuracy table (README.md:62-69: PEEN, MSE and compression factor for 6..10
 retained coefficients and for the standard quantisation matrix), regenerated on the GPU.
 
-    python benchmarks/readme_table.py [--size 2048] [--image file] [--colour]
+    python benchmarks/readme_table.py [--size 2048] [--image file] [--colour] [--subsampling 420]
 
 The README's "Circuit" image is not in the reference repository, so the default input is a
 deterministic synthetic stand-in with the same character (dark background, straight traces and
@@ -47,10 +47,14 @@ def main():
     ap.add_argument("--size", type=int, default=2048)
     ap.add_argument("--image", default=None, help="grayscale image file instead of the synthetic one")
     ap.add_argument("--colour", action="store_true", help="RGB version (three planes, chroma table)")
+    ap.add_argument("--subsampling", choices=["444", "420"], default="444",
+                    help="chroma of the RGB version: full resolution, or 4:2:0 as JPEG encoders do by default (implies --colour)")
     args = ap.parse_args()
+    args.colour = args.colour or args.subsampling == "420"
     if args.image:
         img = m.imageio.load_gray(args.image)
-        img = np.ascontiguousarray(img[: img.shape[0] // 8 * 8, : img.shape[1] // 8 * 8])
+        b = 16 if args.subsampling == "420" else 8
+        img = np.ascontiguousarray(img[: img.shape[0] // b * b, : img.shape[1] // b * b])
     else:
         img = circuit_like(args.size)
     H, W = img.shape
@@ -71,14 +75,21 @@ def main():
         d = torch.from_numpy(rgb).cuda()
         for k in cols:
             plan = m.Plan(keep=m.zigzag_mask(k), inverse=m.api.INVERSE_EXACT)
-            zz = torch.empty(3, H // 8, W // 8, 64, dtype=torch.int16, device=d.device)
-            out = m.roundtrip_rgb(d, streams=zz, plan=plan)
+            if args.subsampling == "420":
+                zz = m.forward_rgb420(d, plan=plan)
+                out = m.inverse_rgb420(zz, plan=plan)
+                nnz, blocks = sum(float((s != 0).sum().item()) for s in zz), 1.5 * H * W / 64
+            else:
+                zz = torch.empty(3, H // 8, W // 8, 64, dtype=torch.int16, device=d.device)
+                out = m.roundtrip_rgb(d, streams=zz, plan=plan)
+                nnz, blocks = float((zz != 0).sum().item()), 3 * H * W / 64
             mse, peen = m.metrics(d.view(H, W * 3), out.view(H, W * 3))
             rows["PEEN (%)"].append(peen)
             rows["MSE"].append(mse)
             rows["Compr. Factor"].append(m.compression_factor(zz))
-            rows["non-zero coeff. / block"].append(float((zz != 0).sum().item()) / (3 * H * W / 64))
-    print(f"Input: {'synthetic circuit-like' if not args.image else args.image} {H}x{W} {'RGB' if args.colour else 'grayscale'} u8; "
+            rows["non-zero coeff. / block"].append(nnz / blocks)
+    kind = ("RGB 4:2:0" if args.subsampling == "420" else "RGB 4:4:4") if args.colour else "grayscale"
+    print(f"Input: {'synthetic circuit-like' if not args.image else args.image} {H}x{W} {kind} u8; "
           "HpApprDCT (Haweel T), JPEG tables; CF = 8*H*W*channels / baseline-JPEG coded bits\n")
     print("| Metric / Coefficients | 6 | 7 | 8 | 9 | 10 | Standard |")
     print("| :--- | :---: | :---: | :---: | :---: | :---: | :---: |")

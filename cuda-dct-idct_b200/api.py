@@ -75,6 +75,8 @@ def lib() -> C.CDLL:
         L.b200dct_roundtrip_rgb.argtypes = [vp, vp, sz, vp, sz, vp, sz, i, i, vp]
         L.b200dct_forward_rgb.argtypes = [vp, vp, sz, vp, sz, i, i, vp]
         L.b200dct_inverse_rgb.argtypes = [vp, vp, sz, vp, sz, i, i, vp]
+        L.b200dct_forward_rgb420.argtypes = [vp, vp, sz, vp, vp, vp, i, i, vp]
+        L.b200dct_inverse_rgb420.argtypes = [vp, vp, vp, vp, vp, sz, i, i, vp]
         L.b200dct_zigzag_coded_bits.argtypes = [vp, sz, i, i, i, vp, vp]
         L.b200dct_host_pipeline_create.argtypes = [C.POINTER(vp), sz, i]
         L.b200dct_host_pipeline_destroy.argtypes = [vp]
@@ -518,6 +520,59 @@ def inverse_rgb(streams, out=None, plan: Plan | None = None, stream=None):
     return out
 
 
+def _rgb420_streams(streams, H, W):
+    """Pointers of the 4:2:0 streams (y, cb, cr): tightly packed int16 CUDA tensors of shapes (H/8, W/8, 64) and
+    (H/16, W/16, 64) twice, on one device (H, W None: taken from y)."""
+    import torch
+
+    if not (isinstance(streams, (tuple, list)) and len(streams) == 3):
+        raise B200DCTError("4:2:0 streams are a (y, cb, cr) tuple")
+    y = streams[0]
+    if H is None and isinstance(y, torch.Tensor) and y.dim() == 3:
+        H, W = int(y.shape[0]) * 8, int(y.shape[1]) * 8
+    shapes = ((H // 8, W // 8, 64), (H // 16, W // 16, 64), (H // 16, W // 16, 64))
+    for t, shape in zip(streams, shapes):
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.int16 and tuple(t.shape) == shape
+                and t.is_contiguous() and t.device == y.device):
+            raise B200DCTError("4:2:0 streams must be tightly packed int16 CUDA tensors of shapes (H/8, W/8, 64), "
+                               "(H/16, W/16, 64), (H/16, W/16, 64) on one device")
+    return H, W, [t.data_ptr() for t in streams]
+
+
+def forward_rgb420(rgb, streams=None, plan: Plan | None = None, stream=None):
+    """RGB with 4:2:0 chroma subsampling (b200dct_forward_rgb420): an (H, W, 3) uint8 CUDA tensor, H and W
+    multiples of 16 -> YCbCr -> Cb and Cr downsampled 2x2 as libjpeg does -> per-plane DCT / quantise -> the
+    zig-zag streams (y, cb, cr), int16 tensors of shapes (H/8, W/8, 64), (H/16, W/16, 64) and (H/16, W/16, 64)
+    (written into `streams` when given)."""
+    import torch
+
+    _rgb_image(rgb, None, None, "rgb")
+    H, W = int(rgb.shape[0]), int(rgb.shape[1])
+    with _on(rgb, stream):
+        if streams is None:
+            streams = (torch.empty((H // 8, W // 8, 64), dtype=torch.int16, device=rgb.device),
+                       torch.empty((H // 16, W // 16, 64), dtype=torch.int16, device=rgb.device),
+                       torch.empty((H // 16, W // 16, 64), dtype=torch.int16, device=rgb.device))
+        _, _, (py, pb, pr) = _rgb420_streams(streams, H, W)
+        _check(lib().b200dct_forward_rgb420(_plan(plan)._h, rgb.data_ptr(), rgb.stride(0), py, pb, pr, H, W, _stream(stream)))
+    return tuple(streams)
+
+
+def inverse_rgb420(streams, out=None, plan: Plan | None = None, stream=None):
+    """The 4:2:0 streams (y, cb, cr) -> per-plane dequantise / IDCT -> Cb and Cr upsampled as libjpeg's
+    decoder does by default ('fancy' triangle filter) -> RGB, an (H, W, 3) uint8 CUDA tensor (written into
+    `out` when given) (b200dct_inverse_rgb420)."""
+    import torch
+
+    H, W, (py, pb, pr) = _rgb420_streams(streams, None, None)
+    with _on(streams[0], stream):
+        if out is None:
+            out = torch.empty((H, W, 3), dtype=torch.uint8, device=streams[0].device)
+        _rgb_image(out, H, W, "out")
+        _check(lib().b200dct_inverse_rgb420(_plan(plan)._h, py, pb, pr, out.data_ptr(), out.stride(0), H, W, _stream(stream)))
+    return out
+
+
 CODED_OUT_OF_RANGE = 1 << 63   # B200DCT_CODED_OUT_OF_RANGE: the stream holds a symbol baseline JPEG cannot code
 
 
@@ -544,7 +599,13 @@ def compression_factor(zz, table: int = 0, stream=None) -> float:
     """8*H*W / coded_bits: the README's 'Compr. Factor' (README.md:62-69) under the baseline-JPEG
     entropy coder.  `zz`: one plane's stream, or a (3, ...) stack (Y with the luminance codes,
     Cb and Cr with the chrominance codes; CF of the whole colour image).  Raises B200DCTError for a
-    stream that baseline JPEG cannot code (see coded_bits)."""
+    stream that baseline JPEG cannot code (see coded_bits).  `zz` may also be the (y, cb, cr) streams of
+    forward_rgb420: their bits add up (Y with the luminance codes), over the same 8*3*H*W bits of the RGB image,
+    H and W from y, so the factor compares directly with the 4:4:4 stack's."""
+    if isinstance(zz, (tuple, list)):
+        y, cb, cr = zz
+        bits = coded_bits(y, 0, stream) + coded_bits(cb, 1, stream) + coded_bits(cr, 1, stream)
+        return 8.0 * 3 * y.shape[0] * y.shape[1] * 64 / bits
     if zz.dim() == 4:
         bits = sum(coded_bits(zz[c], 0 if c == 0 else 1, stream) for c in range(zz.shape[0]))
         return 8.0 * zz.shape[0] * zz.shape[1] * zz.shape[2] * 64 / bits

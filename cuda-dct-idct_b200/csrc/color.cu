@@ -1,9 +1,11 @@
 // color.cu -- host side of the colour entry points (b200dct_roundtrip_rgb, b200dct_forward_rgb,
-// b200dct_inverse_rgb) and of the coded-size / compression-factor kernel (b200dct_zigzag_coded_bits).  See rgb_kernels.cuh for the arithmetic.
+// b200dct_inverse_rgb, and with 4:2:0 chroma b200dct_forward_rgb420, b200dct_inverse_rgb420) and of the coded-size /
+// compression-factor kernel (b200dct_zigzag_coded_bits).  See rgb_kernels.cuh and rgb420_kernels.cuh for the arithmetic.
 #include <cuda_runtime.h>
 #include <string.h>
 
 #include "plan_internal.h"
+#include "rgb420_kernels.cuh"
 
 using namespace b200dct;
 
@@ -50,14 +52,16 @@ static int rgb_qk(const b200dct_plan *plan)
 }
 // One launch of a colour kernel.  Early path across launch boundaries (b200dct.cu, "early loads"): a pass whose
 // input `rd` is not written by the library's previous machine-filling launch on this stream reads and computes
-// before it waits (rd.ptr NULL: never); w0 / w1 are what the launch writes.
-static int run_rgb(RgbLauncher launch, RgbParams &P, dim3 grid, cudaStream_t s, Span rd, Span w0, Span w1)
+// before it waits (rd.ptr NULL: never); w0 .. w2 are what the launch writes.
+template <class Params> // RgbParams, Rgb420Params
+static int run_rgb(cudaError_t (*launch)(const Params &, dim3, dim3, size_t, cudaStream_t, bool, int *), Params &P, dim3 grid,
+                   cudaStream_t s, Span rd, Span w0, Span w1, Span w2 = Span{})
 {
     const bool capturing = stream_capturing(s), pdl = pdl_enabled(capturing), usable = pdl && !capturing;
     const dim3 block(32, 4);
     int per_sm = 0;
     if (usable) launch(P, grid, block, 0, s, pdl, &per_sm);
-    LaunchScope scope(s, LaunchScope::DIRECT, usable, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1);
+    LaunchScope scope(s, LaunchScope::DIRECT, usable, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1, w2);
     scope.apply(P);
     const cudaError_t e = launch(P, grid, block, 0, s, pdl, nullptr);
     if (e != cudaSuccess) return (int)e;
@@ -116,6 +120,76 @@ extern "C" int b200dct_inverse_rgb(const b200dct_plan *plan, const void *zz3, si
     static const RgbLauncher launchers[2] = {launch_kernel<k_rgb_inverse<false>>, launch_kernel<k_rgb_inverse<true>>};
     return run_rgb(launchers[use_factored_inverse_u8(plan)], P, grid, (cudaStream_t)stream, zz_span(zz3, zz_plane_bytes, H, W),
                    rgb_span(out, out_pitch, H, W), Span{nullptr, 0, 0, 0});
+}
+
+// ------------------------------------------------------------------ 4:2:0 chroma (rgb420_kernels.cuh)
+using Rgb420Launcher = cudaError_t (*)(const Rgb420Params &, dim3, dim3, size_t, cudaStream_t, bool, int *);
+
+// The argument rules of the 4:2:0 entry points: those of the 4:4:4 calls, H and W multiples of 16, and three
+// tightly packed streams, each 16-byte aligned.
+static int rgb420_params(const b200dct_plan *plan, const void *rgb_in, size_t in_pitch, void *rgb_out, size_t out_pitch,
+                         const void *zy, const void *zcb, const void *zcr, int H, int W, Rgb420Params &P)
+{
+    if (H <= 0 || W <= 0 || (H % 16) || (W % 16)) return B200DCT_ERR_SHAPE;
+    if ((rgb_in && in_pitch < (size_t)W * 3) || (rgb_out && out_pitch < (size_t)W * 3)) return B200DCT_ERR_SHAPE;
+    if (((uintptr_t)rgb_in & 7) || ((uintptr_t)rgb_out & 7) || (in_pitch & 7) || (out_pitch & 7)) return B200DCT_ERR_ALIGN;
+    if (((uintptr_t)zy & 15) || ((uintptr_t)zcb & 15) || ((uintptr_t)zcr & 15)) return B200DCT_ERR_ALIGN;
+    if (!plan->sparse) return B200DCT_ERR_ARG; // Haweel's T only, as the 4:4:4 calls
+    if ((W / 8 + 31) / 32 > 65535) return B200DCT_ERR_SHAPE;
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess) return B200DCT_ERR_NODEVICE;
+
+    memset(&P, 0, sizeof(P));
+    P.in = rgb_in; P.in_pitch = in_pitch;
+    P.out = rgb_out; P.out_pitch = out_pitch;
+    P.zz[0] = const_cast<void *>(zy); P.zz[1] = const_cast<void *>(zcb); P.zz[2] = const_cast<void *>(zcr);
+    P.zz_pitch[0] = (size_t)(W / 8) * 128; P.zz_pitch[1] = (size_t)(W / 16) * 128;
+    P.mx = W / 16; P.my = H / 16;
+    for (int k = 0; k < 64; k++) {
+        P.t[0].rd[k] = make_float2(plan->cp.q.rcp[k], plan->cp.q.d[k]);
+        P.t[0].keep[k] = plan->cp.q.keep[k];
+        P.t[1].rd[k] = make_float2(plan->qc.rcp[k], plan->qc.d[k]);
+        P.t[1].keep[k] = plan->qc.keep[k];
+    }
+    return B200DCT_OK;
+}
+static Span y_span(const void *zz, int H, int W) { return Span{zz, (size_t)(W / 8) * 128, (size_t)(W / 8) * 128, H / 8}; }
+static Span c_span(const void *zz, int H, int W) { return Span{zz, (size_t)(W / 16) * 128, (size_t)(W / 16) * 128, H / 16}; }
+extern "C" int b200dct_forward_rgb420(const b200dct_plan *plan, const void *rgb, size_t in_pitch, void *zz_y, void *zz_cb,
+                                      void *zz_cr, int H, int W, void *stream)
+{
+    note_launch(0, "none");
+    if (!plan || !rgb || !zz_y || !zz_cb || !zz_cr) return B200DCT_ERR_ARG;
+    Rgb420Params P;
+    const int rc = rgb420_params(plan, rgb, in_pitch, nullptr, 0, zz_y, zz_cb, zz_cr, H, W, P);
+    if (rc != B200DCT_OK) return rc;
+    static const Rgb420Launcher launchers[3] = {launch_kernel<k_rgb420_forward<0>>, launch_kernel<k_rgb420_forward<1>>,
+                                                launch_kernel<k_rgb420_forward<2>>};
+    const dim3 grid((unsigned)((H / 8 + 3) / 4), (unsigned)((W / 8 + 31) / 32)); // 16 x 2 MCUs per CTA
+    return run_rgb(launchers[rgb_qk(plan)], P, grid, (cudaStream_t)stream, rgb_span(rgb, in_pitch, H, W), y_span(zz_y, H, W),
+                      c_span(zz_cb, H, W), c_span(zz_cr, H, W));
+}
+
+extern "C" int b200dct_inverse_rgb420(const b200dct_plan *plan, const void *zz_y, const void *zz_cb, const void *zz_cr,
+                                      void *out, size_t out_pitch, int H, int W, void *stream)
+{
+    note_launch(0, "none");
+    if (!plan || !zz_y || !zz_cb || !zz_cr || !out) return B200DCT_ERR_ARG;
+    Rgb420Params P;
+    const int rc = rgb420_params(plan, nullptr, 0, out, out_pitch, zz_y, zz_cb, zz_cr, H, W, P);
+    if (rc != B200DCT_OK) return rc;
+    static const Rgb420Launcher launchers[2] = {launch_kernel<k_rgb420_inverse<false>>, launch_kernel<k_rgb420_inverse<true>>};
+    const dim3 grid((unsigned)((P.my + R420_MY - 1) / R420_MY), (unsigned)((P.mx + R420_MX - 1) / R420_MX));
+    // the early path's read span: the range that bounds the three streams (conservative when they lie apart)
+    const Span sp[3] = {y_span(zz_y, H, W), c_span(zz_cb, H, W), c_span(zz_cr, H, W)};
+    uintptr_t lo = ~(uintptr_t)0, hi = 0;
+    for (const Span &x : sp) {
+        lo = (uintptr_t)x.ptr < lo ? (uintptr_t)x.ptr : lo;
+        const uintptr_t end = (uintptr_t)x.ptr + (size_t)(x.rows - 1) * x.pitch + x.row_bytes;
+        hi = end > hi ? end : hi;
+    }
+    return run_rgb(launchers[use_factored_inverse_u8(plan)], P, grid, (cudaStream_t)stream,
+                      Span{(const void *)lo, hi - lo, hi - lo, 1}, rgb_span(out, out_pitch, H, W), Span{}, Span{});
 }
 
 // ------------------------------------------------------------------ coded size of a coefficient stream

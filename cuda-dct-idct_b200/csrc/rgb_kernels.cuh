@@ -129,7 +129,8 @@ using RgbPark = uint2[3][8][128];
 // early loads, b200dct.cu): the leading P.early CTAs of the grid may read and compute before
 // griddepcontrol.wait while the library's predecessor on the stream is provably still running; then every
 // global write of such a CTA must come after its wait.
-__device__ __forceinline__ bool rgb_early(const RgbParams &P, int tid)
+template <class Params> // RgbParams, Rgb420Params
+__device__ __forceinline__ bool rgb_early(const Params &P, int tid)
 {
     if (P.early != 0 && blockIdx.y * gridDim.x + blockIdx.x < (unsigned)P.early) { // CTA-uniform
         __shared__ int s_early;
@@ -161,31 +162,35 @@ __device__ __forceinline__ void rgb_load_ycc(const RgbParams &P, long long by, i
         park[2][r][tid] = pack_byte2(crv);
     }
 }
-// YCbCr -> RGB (jdcolor.c ycc_rgb_convert) of the parked planes + store, one row per iteration
+// YCbCr -> RGB (jdcolor.c ycc_rgb_convert) of eight pixels, each plane's samples as eight packed bytes, stored
+// as 24 bytes at `dst` (8-byte aligned)
+__device__ __forceinline__ void ycc_row_to_rgb(uint2 yw, uint2 bw, uint2 rw, char *dst)
+{
+    float o[24];
+    sfor<8>([&](auto k) {
+        const uint32_t ys = IC(k) < 4 ? yw.x : yw.y, bs = IC(k) < 4 ? bw.x : bw.y, rs = IC(k) < 4 ? rw.x : rw.y;
+        const float ym = u8_to_float(ys, IC(k) & 3) - RGB_MAGIC;
+        const float cb = u8_shifted(bs, IC(k) & 3), cr = u8_shifted(rs, IC(k) & 3);
+        o[3 * IC(k)] = floor_magic(__fmaf_rn(cr, B200_FIX(1.40200), 0.5f)) + ym;
+        o[3 * IC(k) + 1] = floor_magic(__fmaf_rn(cr, -B200_FIX(0.71414), __fmaf_rn(cb, -B200_FIX(0.34414), 0.5f))) + ym;
+        o[3 * IC(k) + 2] = floor_magic(__fmaf_rn(cb, B200_FIX(1.77200), 0.5f)) + ym;
+    });
+    uint2 *row = reinterpret_cast<uint2 *>(dst);
+    row[0] = make_uint2(pack4_u8(o[0], o[1], o[2], o[3]), pack4_u8(o[4], o[5], o[6], o[7]));       // range_limit = saturation
+    row[1] = make_uint2(pack4_u8(o[8], o[9], o[10], o[11]), pack4_u8(o[12], o[13], o[14], o[15]));
+    row[2] = make_uint2(pack4_u8(o[16], o[17], o[18], o[19]), pack4_u8(o[20], o[21], o[22], o[23]));
+}
+// YCbCr -> RGB of the parked planes + store, one row per iteration
 __device__ __forceinline__ void rgb_store_ycc(const RgbParams &P, long long by, int bxi, int tid, const RgbPark &park)
 {
     char *dst = (char *)P.out + (size_t)by * 8 * P.out_pitch + (size_t)bxi * 24;
 #pragma unroll 1
-    for (int r = 0; r < 8; r++) {
-        const uint2 yw = park[0][r][tid], bw = park[1][r][tid], rw = park[2][r][tid];
-        float o[24];
-        sfor<8>([&](auto k) {
-            const uint32_t ys = IC(k) < 4 ? yw.x : yw.y, bs = IC(k) < 4 ? bw.x : bw.y, rs = IC(k) < 4 ? rw.x : rw.y;
-            const float ym = u8_to_float(ys, IC(k) & 3) - RGB_MAGIC;
-            const float cb = u8_shifted(bs, IC(k) & 3), cr = u8_shifted(rs, IC(k) & 3);
-            o[3 * IC(k)] = floor_magic(__fmaf_rn(cr, B200_FIX(1.40200), 0.5f)) + ym;
-            o[3 * IC(k) + 1] = floor_magic(__fmaf_rn(cr, -B200_FIX(0.71414), __fmaf_rn(cb, -B200_FIX(0.34414), 0.5f))) + ym;
-            o[3 * IC(k) + 2] = floor_magic(__fmaf_rn(cb, B200_FIX(1.77200), 0.5f)) + ym;
-        });
-        uint2 *row = reinterpret_cast<uint2 *>(dst + (size_t)r * P.out_pitch);
-        row[0] = make_uint2(pack4_u8(o[0], o[1], o[2], o[3]), pack4_u8(o[4], o[5], o[6], o[7]));       // range_limit = saturation
-        row[1] = make_uint2(pack4_u8(o[8], o[9], o[10], o[11]), pack4_u8(o[12], o[13], o[14], o[15]));
-        row[2] = make_uint2(pack4_u8(o[16], o[17], o[18], o[19]), pack4_u8(o[20], o[21], o[22], o[23]));
-    }
+    for (int r = 0; r < 8; r++) ycc_row_to_rgb(park[0][r][tid], park[1][r][tid], park[2][r][tid], dst + (size_t)r * P.out_pitch);
 }
 // Every machine-filling launch must feed the stream's completion counter (P.chain_feed set by the host): a counter
 // left short would make every later call on the stream believe its predecessor is still running.
-__device__ __forceinline__ void rgb_feed_chain(const RgbParams &P, int tid)
+template <class Params>
+__device__ __forceinline__ void rgb_feed_chain(const Params &P, int tid)
 {
     if (P.chain_feed && tid == 0 && blockIdx.y * gridDim.x + blockIdx.x + (unsigned)P.chain_feed >= gridDim.x * gridDim.y)
         atomicAdd(P.chain, 1ull); // one of the last CTAs of the grid is (as good as) done

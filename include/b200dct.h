@@ -29,6 +29,7 @@
  *     dct_all_blocks_cuda per Y/Cb/Cr plane                b200dct_forward_rgb  (RGB -> 3 zig-zag streams)
  *     idct_all_blocks_cuda per Y/Cb/Cr plane               b200dct_inverse_rgb  (3 zig-zag streams -> RGB)
  *     both, one fused pass                                 b200dct_roundtrip_rgb
+ *     with 4:2:0 chroma (Cb, Cr at half resolution)        b200dct_forward_rgb420 / b200dct_inverse_rgb420
  *
  * Conventions: images are single-channel, row-major; H and W are multiples of 8 (the
  * reference silently computes garbage otherwise, main_newAppr.cu:261-262; here it is an
@@ -52,8 +53,9 @@
 extern "C" {
 #endif
 
-#define B200DCT_VERSION 102 /* 101: b200dct_forward_rgb / b200dct_inverse_rgb; 102: b200dct_zigzag_coded_bits flags
-                               * out-of-range symbols (B200DCT_CODED_OUT_OF_RANGE), f32 metrics in 128-bit fixed point */
+#define B200DCT_VERSION 103 /* 101: b200dct_forward_rgb / b200dct_inverse_rgb; 102: b200dct_zigzag_coded_bits flags
+                               * out-of-range symbols (B200DCT_CODED_OUT_OF_RANGE), f32 metrics in 128-bit fixed point;
+                               * 103: b200dct_forward_rgb420 / b200dct_inverse_rgb420 */
 
 typedef enum b200dct_dtype {
     B200DCT_F32 = 0, /* float pixels / integer-valued float coefficients (the reference's type) */
@@ -283,6 +285,31 @@ int b200dct_forward_rgb(const b200dct_plan *plan, const void *rgb, size_t in_pit
  * -> YCbCr -> RGB (libjpeg jdcolor.c). */
 int b200dct_inverse_rgb(const b200dct_plan *plan, const void *zz3, size_t zz_plane_bytes,
                         void *out, size_t out_pitch, int H, int W, void *stream);
+/* 4:2:0 chroma subsampling, what libjpeg and every JPEG encoder do by default: Cb and Cr at half the
+ * resolution in both directions, so a 16x16 macroblock (MCU) carries four Y blocks and one Cb and one Cr
+ * block -- half the coefficients of 4:4:4.  The resampling is libjpeg's, bit for bit: the encoder's
+ * h2v2_downsample (jcsample.c: a half-resolution sample is (a + b + c + d + bias) >> 2 over its 2x2 group of
+ * 8-bit samples, bias 1 at even and 2 at odd output columns) and the decoder's default h2v2_fancy_upsample
+ * (jdsample.c: triangle filter 3/4, 1/4 in both directions, edges replicated).
+ * rgb/out: as b200dct_roundtrip_rgb (interleaved RGB u8, 8-byte aligned rows, pitch in bytes).  H and W
+ * are positive multiples of 16 (B200DCT_ERR_SHAPE otherwise, and for a pitch below W*3).  Three separate
+ * block-major zig-zag int16 streams (B200DCT_I16_ZIGZAG layout), tightly packed, 16-byte aligned
+ * (B200DCT_ERR_ALIGN otherwise, as for misaligned pixel pointers or pitches): zz_y holds H/8 x W/8 blocks
+ * with a block-row pitch of (W/8)*128 bytes, zz_cb and zz_cr H/16 x W/16 blocks with a pitch of
+ * (W/16)*128 bytes.  NULL pointers and a dense T give B200DCT_ERR_ARG (Haweel's T only).  One launch
+ * each (b200dct_last_path() "rgb"), legal under stream capture.
+ * Forward: RGB -> YCbCr (jccolor.c) -> 2x2 downsampling of Cb and Cr -> per plane convertToFloat, dct,
+ * quantise (luminance Q for Y, chrominance Q for Cb and Cr, the plan's keep mask on all three).
+ * Inverse: per plane dequantise, idct (the plan's inverse mode), convertToUnsignedChar -> upsampling of Cb
+ * and Cr -> YCbCr -> RGB (jdcolor.c).
+ * Coded size: b200dct_zigzag_coded_bits of zz_y with table 0 (H, W), plus zz_cb and zz_cr with table 1 at
+ * (H/2, W/2), is exactly the entropy-coded size of a baseline JPEG with three non-interleaved scans, one per
+ * component (sampling factors 2x2, 1x1, 1x1): in such a scan a component's blocks come in raster order
+ * (ITU-T T.81 A.2.2), as that function counts them. */
+int b200dct_forward_rgb420(const b200dct_plan *plan, const void *rgb, size_t in_pitch,
+                           void *zz_y, void *zz_cb, void *zz_cr, int H, int W, void *stream);
+int b200dct_inverse_rgb420(const b200dct_plan *plan, const void *zz_y, const void *zz_cb, const void *zz_cr,
+                           void *out, size_t out_pitch, int H, int W, void *stream);
 
 /* Size in BITS of the baseline-JPEG entropy-coded scan (ITU-T T.81 sequential Huffman with the
  * Annex K.3 tables, i.e. what libjpeg writes with optimize off; no headers, stuffing or padding)
