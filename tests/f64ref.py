@@ -158,10 +158,11 @@ def check_quant(coef: np.ndarray, Y: np.ndarray, B: np.ndarray, Q, keep: int = A
 
 
 def check_close(got: np.ndarray, exact: np.ndarray, mag: np.ndarray, c: float = C_I) -> Check:
-    """f32 values (pixels from inverse64, or unquantised Y from forward64) within c u mag of exact."""
+    """f32 values (pixels from inverse64, or unquantised Y from forward64) within c u mag of exact.  A NaN or
+    infinity is outside every bound (an output the kernel never wrote keeps a NaN sentinel)."""
     err = np.abs(got.astype(np.float64) - exact)
     ratio = err / (U * np.maximum(mag, np.finfo(np.float64).tiny))
-    return Check(int((err > c * U * mag).sum()), 0.0, float(ratio.max()) if ratio.size else 0.0, got.size)
+    return Check(int((~(err <= c * U * mag)).sum()), 0.0, float(ratio.max()) if ratio.size else 0.0, got.size)
 
 
 def expected_u8(P: np.ndarray, Bi: np.ndarray, c: float = C_I):

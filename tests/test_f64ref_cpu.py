@@ -278,6 +278,11 @@ def test_check_helpers(oracle):
     P = np.array([[99.9999999, 99.5, 256.0, -3.0]])
     want, amb, other = R.expected_u8(P, np.full_like(P, 1000.0))
     assert want.tolist() == [[99, 99, 255, 0]] and amb.tolist() == [[True, False, False, False]] and other[0, 0] == 100
+    # f32: a NaN (an output left at its sentinel) or an infinity is outside every bound, however wide
+    exact = np.array([1.0, 2.0, 3.0, 4.0])
+    got = np.array([1.0, np.nan, np.inf, 4.0], np.float32)
+    assert R.check_close(got, exact, np.full(4, 1e30)).bad == 2
+    assert R.check_close(exact.astype(np.float32), exact, np.ones(4)).bad == 0
 
 
 # ---------------------------------------------------------------- 3. mutants fail
