@@ -292,12 +292,7 @@ static bool make_map(CUtensorMap *map, const void *ptr, int dt, size_t pitch, in
     encode_tiled_fn enc = get_encode();
     if (!enc) return false;
     CUresult r;
-    // developer knob: B200DCT_TMA_L2PROMO = 0 none, 1 64B, 2 128B, 3 256B (read once; magic statics are thread-safe)
-    static const int promo_env = [] {
-        const char *e = getenv("B200DCT_TMA_L2PROMO");
-        return (e && atoi(e) >= 0 && atoi(e) <= 3) ? atoi(e) : 3;
-    }();
-    const CUtensorMapL2promotion promo = (CUtensorMapL2promotion)promo_env;
+    const CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
     if (dt == DT_F32) {
         // {32 floats, W/32 segments, H rows}; box = 8 rows x 8 segments x 128 B, 128B swizzle
         cuuint64_t dims[3] = {32, (cuuint64_t)(W / 32), (cuuint64_t)H};
@@ -345,7 +340,7 @@ static int check_plane(const Plane &pl, int W, bool pixels)
 // walk the ring, so it gets a pair of its own for good from a second pool (CAPTURE_SLOTS per
 // device, never recycled): replays of one graph exec are stream-ordered by CUDA and every run
 // leaves the pair zeroed.  (Two execs instantiated from the SAME captured graph and replayed
-// concurrently would share a pair -- not supported; B200DCT_TMA_STATIC=1 avoids the counters.)
+// concurrently would share a pair -- not supported; B200DCT_PATH_DIRECT avoids the counters.)
 // Nothing can be allocated during capture, so both pools are created by the first ordinary call.
 namespace {
 constexpr int SCHED_SLOTS = 4096;
@@ -389,7 +384,7 @@ unsigned long long *sched_macc(const uint32_t *slot)
     return g_sched.macc[dev] + MACC_WORDS * ((slot - g_sched.base[dev]) / 2);
 }
 // The counters of a fused-metrics launch: those of its scheduler slot, or without one (capture pool used up,
-// B200DCT_TMA_STATIC=1, failed ring allocation) the caller's workspace, laid out as
+// failed ring allocation) the caller's workspace, laid out as
 // {u64 macc[MACC_WORDS]; u32 pair[2]}.  The kernel leaves either zeroed; the workspace starts unknown, so a launch on it
 // is preceded by a memset on its stream and takes no part in the early path.
 constexpr size_t METRICS_WORKSPACE_BYTES = MACC_WORDS * sizeof(unsigned long long) + 2 * sizeof(uint32_t);
@@ -566,9 +561,6 @@ void LaunchScope::done(bool launched)
 }
 }
 
-static bool tma_dynamic = true; // env B200DCT_TMA_STATIC=1 forces the static tile split
-static int tma_warps = 0; // env B200DCT_TMA_WARPS: warps per CTA of the persistent kernel (0 = per-flavour default; clamped to the kernel's CTA size and to shared memory)
-static int tma_max_run = 2;                       // env B200DCT_TMA_RUN: longest run of tiles per claim
 // Programmatic dependent launch (default on; env B200DCT_PDL=0 turns it off): consecutive kernels
 // of this library in one stream overlap the next kernel's CTA launch and set-up with the previous
 // kernel's tail.  Every kernel executes griddepcontrol.wait before its first global-memory access,
@@ -589,34 +581,10 @@ bool stream_capturing(cudaStream_t s)
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     return cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
 }
-// Under stream capture the attribute becomes a programmatic edge of the graph (CUDA >= 12.3);
-// off unless B200DCT_PDL_CAPTURE=1 (experiment).
-bool pdl_enabled(bool capturing)
-{
-    static const bool cap = [] {
-        const char *p = getenv("B200DCT_PDL_CAPTURE");
-        return p && atoi(p) == 1;
-    }();
-    return use_pdl() && (!capturing || cap);
-}
+// Under stream capture the attribute would become a programmatic edge of the graph (CUDA >= 12.3):
+// no gain on graph replay (82.4 vs 82.2 us at 8192^2 f32, profiles/r01_graph_replay.txt), so captured launches go without.
+bool pdl_enabled(bool capturing) { return use_pdl() && !capturing; }
 } // namespace b200dct
-static int tma_grid = 0;                          // env B200DCT_TMA_GRID: CTAs (default: one per SM)
-static bool direct_v8() // env B200DCT_DIRECT_V8=0: no 256-bit global accesses in the direct family (A/B)
-{
-    static const bool v = [] {
-        const char *p = getenv("B200DCT_DIRECT_V8");
-        return !(p && atoi(p) == 0);
-    }();
-    return v;
-}
-static bool compiled_masks() // env B200DCT_COMPILED_MASKS=0: retained-coefficient masks as runtime data only (A/B)
-{
-    static const bool v = [] {
-        const char *p = getenv("B200DCT_COMPILED_MASKS");
-        return !(p && atoi(p) == 0);
-    }();
-    return v;
-}
 
 // AUTO's family choice for a call that moves bytes_per_px (explained where run() makes it)
 constexpr unsigned long long TMA_BIG_PIXELS = 28ull << 20, TMA_HUGE_PIXELS = 64ull << 20;
@@ -643,7 +611,7 @@ static Variant variant_of(const b200dct_plan *pl, int mode, int pix, bool runtim
     // retained-coefficient round trips (first k = 6..10 zig-zag coefficients of the default
     // tables): kernels with the mask as a compile-time constant
     v.kmask = 0;
-    if (mode == MODE_RT && !runtime_mask && pl->sparse && pl->q_default && pl->q_fastdiv && compiled_masks())
+    if (mode == MODE_RT && !runtime_mask && pl->sparse && pl->q_default && pl->q_fastdiv)
         for (int k = 6; k <= 10; k++)
             if (pl->mask == b200dct_zigzag_mask(k)) v.kmask = k;
     v.finv = !v.kmask && use_factored_inverse(pl, mode, pix); // compile-time-mask kernels keep the chains
@@ -711,17 +679,6 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     // direct family (86.9 us at 8192^2), which beats the TMA family's static split (99.8 us).
     const bool capturing = stream_capturing(stream);
     const bool pdl = pdl_enabled(capturing);
-    static std::once_flag env_once;
-    std::call_once(env_once, [] {
-        const char *e = getenv("B200DCT_TMA_WARPS");
-        if (e && atoi(e) >= 1 && atoi(e) <= 32) tma_warps = atoi(e);
-        const char *r = getenv("B200DCT_TMA_RUN");
-        if (r && atoi(r) >= 1 && atoi(r) <= 4096) tma_max_run = atoi(r);
-        const char *g = getenv("B200DCT_TMA_GRID");
-        if (g && atoi(g) >= 1) tma_grid = atoi(g);
-        const char *d = getenv("B200DCT_TMA_STATIC");
-        if (d && atoi(d) == 1) tma_dynamic = false;
-    });
     // fused metrics on the TMA family: f32 round trips of Haweel's T (the input tile is compared where it
     // already is, in shared memory); everything else takes the direct family's metrics kernels
     const bool metrics_tma_ok = !workspace || (mode == MODE_RT && in.dt == DT_F32 && pl->tk == TK_HAWEEL && in.ptr != out.ptr);
@@ -729,7 +686,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
                               tma_plane_ok(in.ptr, in.dt, in.pitch, W) && tma_plane_ok(out.ptr, out.dt, out.pitch, W) &&
                               (!coef.ptr || tma_plane_ok(coef.ptr, coef.dt, coef.pitch, W));
     uint32_t *capture_sched = nullptr;
-    if (capturing && tma_dynamic && tma_possible) capture_sched = sched_slot(true);
+    if (capturing && tma_possible) capture_sched = sched_slot(true);
     const bool use_tma = tma_possible && !(capturing && !capture_sched && pl->path == B200DCT_PATH_AUTO);
     if (pl->path == B200DCT_PATH_TMA && !use_tma) return B200DCT_ERR_ALIGN;
     const Span rd = plane_span(in, H, W), w0 = plane_span(out, H, W), w1 = plane_span(coef, H, W);
@@ -767,27 +724,24 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
         P.coef_dt = coef_dt;
         P.has_coef = coef.ptr ? 1 : 0;
 
-        // dynamic tickets; a captured launch owns its pair (NULL = static split)
-        if (tma_dynamic) P.sched = capturing ? capture_sched : sched_slot(false);
+        // dynamic tickets; a captured launch owns its pair (NULL: no pair left, static split)
+        P.sched = capturing ? capture_sched : sched_slot(false);
         P.cp = pl->cp;
         // tile buffers as large as the largest tile image among the planes of this call
         uint32_t buf = tile_bytes_of(in.dt) > tile_bytes_of(out.dt) ? tile_bytes_of(in.dt) : tile_bytes_of(out.dt);
         if (coef.ptr && tile_bytes_of(coef.dt) > buf) buf = tile_bytes_of(coef.dt);
         P.buf_bytes = buf;
-        // warps per CTA: the flavour's CTA size (8 for sparse-T f32; all the CTA holds for the
-        // FP32-bound u8 and dense-T flavours), limited by 227 KiB of shared memory
-        const int max_w = (workspace ? B200DCT_TMA_CTA_THREADS_METRICS : tma_cta_threads(pix, pl->tk)) / 32;
-        int nw = tma_warps > 0 ? tma_warps : (pix == DT_U8 || !pl->sparse || workspace ? max_w : B200DCT_TMA_DEFAULT_WARPS);
-        if (nw > max_w) nw = max_w;
+        // warps per CTA: the flavour's CTA size, limited by 227 KiB of shared memory
+        int nw = (workspace ? TMA_METRICS_THREADS : tma_cta_threads(pix, pl->tk)) / 32;
         const unsigned nbuf = workspace ? 3u : 2u; // metrics: two input buffers per warp
         const int smem_w = (int)((227u * 1024u - 1024u) / (nbuf * buf + 16u));
         if (nw > smem_w) nw = smem_w;
         const size_t smem = (size_t)nw * nbuf * buf + (size_t)nw * 16 + 1024;
-        unsigned long long want = (nt + nw - 1) / nw;
-        const unsigned long long gcap = (unsigned long long)(tma_grid > 0 ? tma_grid : di.sms);
-        const int grid = (int)(want < gcap ? want : gcap);
-        // runs of tma_max_run tiles while more than two rounds of single tiles remain
-        P.run = (uint32_t)tma_max_run;
+        // at most one CTA per SM
+        const unsigned long long want = (nt + nw - 1) / nw, sms = (unsigned long long)di.sms;
+        const int grid = (int)(want < sms ? want : sms);
+        // runs of 2 tiles per ticket while more than two rounds of single tiles remain
+        P.run = 2;
         const unsigned long long tail = 2ull * (unsigned long long)grid * nw;
         P.run_tickets = nt > tail ? (uint32_t)((nt - tail) / P.run) : 0u;
         // Metrics: the dynamic scheduler always, on the counters of the slot or of the workspace; the last warp out
@@ -802,7 +756,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
         // the argument above needs the predecessor to occupy every SM (grid == SM count) and neither
         // launch to fit beside the other on one SM: both take more than half of its shared memory
         const bool heavy = smem > (size_t)(di.smem_optin / 2) + 1024;
-        LaunchScope scope(stream, mc.in_workspace ? LaunchScope::NONE : LaunchScope::TMA, pdl && !capturing && heavy && P.sched != nullptr,
+        LaunchScope scope(stream, mc.in_workspace ? LaunchScope::NONE : LaunchScope::TMA, pdl && heavy && P.sched != nullptr,
                           (unsigned long long)grid, 1, rd, w0, w1);
         scope.apply(P);
         const cudaError_t em = mc.zero(stream);
@@ -824,10 +778,9 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     P.bx = W / 8; P.by = H / 8;
     P.coef_dt = coef_dt;
     P.zz_smem = (coef_dt == DT_I16ZZ && !workspace) ? 1 : 0; // the metrics kernels are launched without dynamic smem
-    if (direct_v8()) { // f32 planes aligned to 32 bytes move with 256-bit accesses
-        auto aligned32 = [](const Plane &pl) { return pl.ptr && pl.dt == DT_F32 && !((uintptr_t)pl.ptr & 31) && !(pl.pitch & 31); };
-        P.v8 = (aligned32(in) ? 1 : 0) | (aligned32(out) ? 2 : 0) | (aligned32(coef) ? 4 : 0);
-    }
+    // f32 planes aligned to 32 bytes move with 256-bit accesses
+    auto aligned32 = [](const Plane &pl) { return pl.ptr && pl.dt == DT_F32 && !((uintptr_t)pl.ptr & 31) && !(pl.pitch & 31); };
+    P.v8 = (aligned32(in) ? 1 : 0) | (aligned32(out) ? 2 : 0) | (aligned32(coef) ? 4 : 0);
     P.cp = pl->cp;
     dim3 block(32, 4);
     dim3 grid((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32));
@@ -843,7 +796,7 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
         P.mdone = mc.pair;
         P.acc = acc;
     }
-    const bool usable = pdl && !capturing && !mc.in_workspace;
+    const bool usable = pdl && !mc.in_workspace;
     int per_sm = 0;
     if (usable) launch_direct(pl->tk, v, mode, pix, metrics, P, grid, block, stream, pdl, &per_sm);
     // the early path: fused round trips without a coefficient plane, forward calls without the X-128 write-back,
@@ -933,7 +886,7 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
     P.bx = W / 8; P.by = H / 8;
     P.coef_dt = DT_F32;
     P.cp = plan->cp;
-    bool v8 = dt == B200DCT_F32 && direct_v8() && !(in_pitch & 31) && !(out_pitch & 31);
+    bool v8 = dt == B200DCT_F32 && !(in_pitch & 31) && !(out_pitch & 31);
     for (int i = 0; v8 && i < n_images; i++) v8 = !((uintptr_t)imgs[i] & 31) && !((uintptr_t)outs[i] & 31);
     P.v8 = v8 ? 3 : 0;
     dim3 block(32, 4);

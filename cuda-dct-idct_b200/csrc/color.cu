@@ -57,11 +57,11 @@ template <class Params> // RgbParams, Rgb420Params
 static int run_rgb(cudaError_t (*launch)(const Params &, dim3, dim3, size_t, cudaStream_t, bool, int *), Params &P, dim3 grid,
                    cudaStream_t s, Span rd, Span w0, Span w1, Span w2 = Span{})
 {
-    const bool capturing = stream_capturing(s), pdl = pdl_enabled(capturing), usable = pdl && !capturing;
+    const bool pdl = pdl_enabled(stream_capturing(s));
     const dim3 block(32, 4);
     int per_sm = 0;
-    if (usable) launch(P, grid, block, 0, s, pdl, &per_sm);
-    LaunchScope scope(s, LaunchScope::DIRECT, usable, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1, w2);
+    if (pdl) launch(P, grid, block, 0, s, pdl, &per_sm);
+    LaunchScope scope(s, LaunchScope::DIRECT, pdl, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1, w2);
     scope.apply(P);
     const cudaError_t e = launch(P, grid, block, 0, s, pdl, nullptr);
     if (e != cudaSuccess) return (int)e;

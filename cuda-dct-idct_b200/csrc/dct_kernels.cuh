@@ -341,15 +341,10 @@ __device__ __forceinline__ void shift_row(float2 (&r)[4], float s)
 // Occupancy of the direct family: 5 CTAs of 128 threads per SM (<= 96 registers, 24-40 bytes of
 // spill) instead of the 4 that the unconstrained 128 registers allow.  Same box, 8192^2
 // (profiles/r01_direct_occupancy.txt): dense-T round trip 108.2 -> 92.4 us, f32 87.7 -> 85.9,
-// u8 65.3 -> 65.3; 6 CTAs (80 registers, up to 400 bytes of spill) loses everywhere.
-#ifndef B200DCT_DIRECT_MIN_BLOCKS
-#define B200DCT_DIRECT_MIN_BLOCKS 5
-#endif
-#ifndef B200DCT_METRICS_MIN_BLOCKS
-#define B200DCT_METRICS_MIN_BLOCKS 4
-#endif
+// u8 65.3 -> 65.3; 6 CTAs (80 registers, up to 400 bytes of spill) loses everywhere.  The metrics kernels: 4.
+constexpr int DIRECT_CTAS_PER_SM = 5, METRICS_CTAS_PER_SM = 4;
 template <int MODE, int TK, int QMODE, int PIX, bool METRICS = false, bool FINV = false>
-__global__ void __launch_bounds__(128, METRICS ? B200DCT_METRICS_MIN_BLOCKS : B200DCT_DIRECT_MIN_BLOCKS) k_direct(const __grid_constant__ DirectParams P)
+__global__ void __launch_bounds__(128, METRICS ? METRICS_CTAS_PER_SM : DIRECT_CTAS_PER_SM) k_direct(const __grid_constant__ DirectParams P)
 {
     constexpr bool BIASED = inverse_is_biased(TK, FINV);
     // CTA = 32 block-columns x 4 block-rows; grid.x walks block-rows (no 65535 limit),
@@ -704,38 +699,19 @@ __device__ __forceinline__ uint32_t tile_bytes()
 //    consecutive tiles per ticket removed that -- profiles/r01_tma_run_scheduler.txt.)
 //  * u8 pixels and dense T (FP32-pipe bound): more, smaller warps -- 512 threads / 128 registers
 //    for u8 (tile buffers are only 2 KiB), 384 threads / 168 registers for dense T.
-#ifndef B200DCT_TMA_CTA_THREADS
-#define B200DCT_TMA_CTA_THREADS 256
-#endif
-#ifndef B200DCT_TMA_CTA_THREADS_U8
-#define B200DCT_TMA_CTA_THREADS_U8 512
-#endif
-#ifndef B200DCT_TMA_CTA_THREADS_DENSE
-#define B200DCT_TMA_CTA_THREADS_DENSE 384
-#endif
-#ifndef B200DCT_TMA_CTA_THREADS_SYM
-#define B200DCT_TMA_CTA_THREADS_SYM 384
-#endif
-#ifndef B200DCT_TMA_DEFAULT_WARPS
-#define B200DCT_TMA_DEFAULT_WARPS 8
-#endif
 __host__ __device__ constexpr int tma_cta_threads(int pix, int tk)
 {
-    return pix == DT_U8 ? B200DCT_TMA_CTA_THREADS_U8
-                        : (tk == TK_HAWEEL ? B200DCT_TMA_CTA_THREADS : (tk == TK_DENSE_SYM ? B200DCT_TMA_CTA_THREADS_SYM : B200DCT_TMA_CTA_THREADS_DENSE));
+    return pix == DT_U8 ? 512 : (tk == TK_HAWEEL ? 256 : 384);
 }
 // the metrics flavour carries three tile buffers per warp (24 KiB): nine warps fill the 227 KiB
-#ifndef B200DCT_TMA_CTA_THREADS_METRICS
-#define B200DCT_TMA_CTA_THREADS_METRICS 288
-#endif
-#define B200DCT_TMA_BOUNDS __launch_bounds__(METRICS ? B200DCT_TMA_CTA_THREADS_METRICS : tma_cta_threads(PIX, TK), 1)
+constexpr int TMA_METRICS_THREADS = 288;
 
 // METRICS (f32 round trips): the warp keeps TWO input buffers (the tile being transformed stays in
 // shared memory until its output exists, while the next tile is already arriving in the other one),
 // so the squared error and the signal energy are taken from the input tile where it already is
 // instead of re-reading it from global memory as the direct family's metrics kernel does.
 template <int MODE, int TK, int QMODE, int PIX, bool FINV = false, bool METRICS = false>
-__global__ void B200DCT_TMA_BOUNDS k_tma(const __grid_constant__ TmaParams P)
+__global__ void __launch_bounds__(METRICS ? TMA_METRICS_THREADS : tma_cta_threads(PIX, TK), 1) k_tma(const __grid_constant__ TmaParams P)
 {
     static_assert(!METRICS || (MODE == MODE_RT && PIX == DT_F32), "fused metrics on the TMA family: f32 round trips");
     constexpr bool BIASED = inverse_is_biased(TK, FINV);
@@ -802,16 +778,14 @@ __global__ void B200DCT_TMA_BOUNDS k_tma(const __grid_constant__ TmaParams P)
         mbar_init(bar0, 1);
         if constexpr (METRICS) mbar_init(bar0 + 8, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-#ifndef B200DCT_NO_TMAP_PREFETCH
         // the descriptors are kernel parameters, not data of the previous kernel: fetch them into
-        // the TMA unit's cache while this CTA still waits for its predecessor (A/B on B200:
-        // 82.6 us either way at 8192^2 -- kept because it is free)
+        // the TMA unit's cache while this CTA still waits for its predecessor (measured on B200:
+        // 82.6 us with or without at 8192^2 -- kept because it is free)
         if (warp == 0) {
             asm volatile("prefetch.tensormap [%0];" ::"l"(&P.in_map) : "memory");
             asm volatile("prefetch.tensormap [%0];" ::"l"(&P.out_map) : "memory");
             if (P.has_coef) asm volatile("prefetch.tensormap [%0];" ::"l"(&P.coef_map) : "memory");
         }
-#endif
     }
     // Only lane 0 ever touches global memory (TMA loads / stores, scheduler and metrics atomics).
     bool early = false;

@@ -22,13 +22,6 @@ cudaError_t B200_CAT(launch_direct_, INST_TAG)(int mode, int pix, bool finv, boo
 #if INST_SPARSE == 1
     B200_DIRECT_CASE(MODE_RT, DT_U8, true, false)
 #endif
-#ifdef B200DCT_FAST_BUILD /* experiment builds: round trip only (+ f32 split for the default quantiser) */
-#if INST_Q == 0
-    B200_DIRECT_CASE(MODE_FWD, DT_F32, false, false)
-    B200_DIRECT_CASE(MODE_INV, DT_F32, false, false)
-#endif
-    return cudaErrorInvalidValue;
-#else
     B200_DIRECT_CASE(MODE_FWD, DT_F32, false, false)
     B200_DIRECT_CASE(MODE_FWD, DT_U8, false, false)
     B200_DIRECT_CASE(MODE_INV, DT_F32, false, false)
@@ -40,7 +33,6 @@ cudaError_t B200_CAT(launch_direct_, INST_TAG)(int mode, int pix, bool finv, boo
     B200_DIRECT_CASE(MODE_RT, DT_F32, false, true)
     B200_DIRECT_CASE(MODE_RT, DT_U8, false, true)
     return cudaErrorInvalidValue;
-#endif
 }
 
 } // namespace b200dct

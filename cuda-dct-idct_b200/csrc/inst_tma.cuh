@@ -23,13 +23,6 @@ cudaError_t B200_CAT(launch_tma_, INST_TAG)(int mode, int pix, bool finv, const 
     B200_TMA_CASE(MODE_RT, DT_U8, true)
     B200_TMA_CASE_M(MODE_RT, DT_F32, false, true) // fused MSE / PEEN / non-zero count (P.macc != NULL)
 #endif
-#ifdef B200DCT_FAST_BUILD
-#if INST_Q == 0
-    B200_TMA_CASE(MODE_FWD, DT_F32, false)
-    B200_TMA_CASE(MODE_INV, DT_F32, false)
-#endif
-    return cudaErrorInvalidValue;
-#else
     B200_TMA_CASE(MODE_FWD, DT_F32, false)
     B200_TMA_CASE(MODE_FWD, DT_U8, false)
     B200_TMA_CASE(MODE_INV, DT_F32, false)
@@ -38,7 +31,6 @@ cudaError_t B200_CAT(launch_tma_, INST_TAG)(int mode, int pix, bool finv, const 
     B200_TMA_CASE(MODE_INV, DT_U8, true)
 #endif
     return cudaErrorInvalidValue;
-#endif
 }
 
 } // namespace b200dct

@@ -73,5 +73,5 @@ private:
 void note_launch(int launches, const char *path); // b200dct_last_launch_count / b200dct_last_path of this thread
 bool use_factored_inverse_u8(const b200dct_plan *pl);
 bool stream_capturing(cudaStream_t s);
-bool pdl_enabled(bool capturing); // programmatic dependent launch for a launch on a (non-)capturing stream
+bool pdl_enabled(bool capturing); // programmatic dependent launch for a launch (never on a capturing stream)
 }

@@ -38,7 +38,7 @@ struct Rgb420Params {
 // 12 KiB of shared memory.  Early path: loads, colour conversion and downsampling before the wait; each thread
 // waits before its first stream store.
 template <int QK>
-__global__ void __launch_bounds__(128, B200DCT_RGB_MIN_BLOCKS) k_rgb420_forward(const __grid_constant__ Rgb420Params P)
+__global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb420_forward(const __grid_constant__ Rgb420Params P)
 {
     __shared__ uint2 ypark[8][128];  // [row][thread]
     __shared__ uint2 cpark[2][8][32]; // [Cb / Cr][row][MCU of the CTA]: a warp's access is contiguous
@@ -152,7 +152,7 @@ __device__ __forceinline__ uint2 upsample_h2v2(const unsigned char *up, const un
 }
 
 template <bool FINV>
-__global__ void __launch_bounds__(128, B200DCT_RGB_MIN_BLOCKS) k_rgb420_inverse(const __grid_constant__ Rgb420Params P)
+__global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb420_inverse(const __grid_constant__ Rgb420Params P)
 {
     __shared__ __align__(16) unsigned char cs[2][R420_CH][R420_CW];
     __shared__ uint2 ypark[8][128];

@@ -119,9 +119,7 @@ __device__ __forceinline__ uint2 pack_byte2(const uint32_t (&v)[8])
 // Now the three planes run through ONE copy of the transform in a loop, and the two conversions are
 // one row of code each, looped over the rows through shared memory.
 // QK: 0 all coefficients kept, exact fast division; 1 mask + exact fast division; 2 mask + __fdiv_rn
-#ifndef B200DCT_RGB_MIN_BLOCKS
-#define B200DCT_RGB_MIN_BLOCKS 5
-#endif
+constexpr int RGB_CTAS_PER_SM = 5;
 // [plane][row][thread] 8-byte slots: a warp's access is 256 contiguous bytes (conflict-free)
 using RgbPark = uint2[3][8][128];
 
@@ -199,7 +197,7 @@ __device__ __forceinline__ void rgb_feed_chain(const Params &P, int tid)
 // ZZ: also emit the three zig-zag coefficient streams (its own instantiation: 150 instructions the
 // default kernel does not have to carry through the instruction cache)
 template <int QK, bool FINV, bool ZZ>
-__global__ void __launch_bounds__(128, B200DCT_RGB_MIN_BLOCKS) k_rgb(const __grid_constant__ RgbParams P)
+__global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb(const __grid_constant__ RgbParams P)
 {
     __shared__ RgbPark park;
     const int tid = threadIdx.y * 32 + threadIdx.x;
@@ -240,7 +238,7 @@ __global__ void __launch_bounds__(128, B200DCT_RGB_MIN_BLOCKS) k_rgb(const __gri
 // Forward: RGB -> YCbCr -> per plane dct + quantise -> zig-zag streams (reads P.in, writes P.zz).  Early
 // path: load, colour conversion and the Y transform run before the wait, which precedes the first stream store.
 template <int QK>
-__global__ void __launch_bounds__(128, B200DCT_RGB_MIN_BLOCKS) k_rgb_forward(const __grid_constant__ RgbParams P)
+__global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb_forward(const __grid_constant__ RgbParams P)
 {
     __shared__ RgbPark park;
     const int tid = threadIdx.y * 32 + threadIdx.x;
@@ -266,7 +264,7 @@ __global__ void __launch_bounds__(128, B200DCT_RGB_MIN_BLOCKS) k_rgb_forward(con
 // writes P.out).  Both inverse routines read only Q (qp.d), never the mask or 1/Q, so there is no quantiser variant.
 // Early path: the streams are loaded and transformed before the wait, which precedes the RGB stores.
 template <bool FINV>
-__global__ void __launch_bounds__(128, B200DCT_RGB_MIN_BLOCKS) k_rgb_inverse(const __grid_constant__ RgbParams P)
+__global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb_inverse(const __grid_constant__ RgbParams P)
 {
     __shared__ RgbPark park;
     const int tid = threadIdx.y * 32 + threadIdx.x;

@@ -229,7 +229,8 @@ int b200dct_roundtrip_any(const b200dct_plan *plan, const void *img, b200dct_dty
  * README.md:67-68 of the reference) and the coefficient density need no second pass over the
  * images.  `workspace`: device, >= b200dct_metrics_workspace_bytes, caller-owned, 8-byte aligned.  It holds
  * the call's counters when no scheduler slot is free (under stream capture with the capture pool used up,
- * or B200DCT_TMA_STATIC=1), so one workspace must not serve two calls that are in flight at once.
+ * or when the slot pool could not be allocated), so one workspace must not serve two calls that are in
+ * flight at once.
  * `out` must not alias `img`.  Large f32 images of Haweel's T run the TMA family's metrics kernel (the
  * error is taken from the input tile in shared memory); everything else the direct family's.  Every call
  * is one launch, and its result is the same bit for bit on every path, including capture with an empty pool.

@@ -1,10 +1,10 @@
-"""Fused metrics where no scheduler slot is free: under stream capture once the capture pool is used up, and with
-B200DCT_TMA_STATIC=1.  The launch then keeps its counters in the caller's workspace and still runs ONE kernel whose
-pixels, coefficients and sums equal those of the ordinary path bit for bit.
+"""Launches that find no scheduler slot free: under stream capture once the capture pool is used up.  A fused-metrics
+call then keeps its counters in the caller's workspace and still runs ONE kernel whose pixels, coefficients and sums
+equal those of the ordinary path bit for bit; a round trip forced onto the TMA family takes the static tile split.
 
-The capture pool and the environment knobs belong to the process, so these cases run in a child process: this file run
-as a script.  The child inherits the test's environment (the arithmetic modes of the autouse fixture), prints its
-metrics and launch records as JSON and leaves its pixels and coefficients in an .npz file."""
+The capture pool belongs to the process, so these cases run in a child process: this file run as a script.  The child
+inherits the test's environment (the arithmetic modes of the autouse fixture), prints its metrics and launch records
+as JSON and leaves its pixels and coefficients in an .npz file."""
 import json
 import os
 import subprocess
@@ -102,29 +102,30 @@ def child_pool(dct, arrays):
         g.replay()
         res[name] = {"rc": rc, "launches": launches, "path": family, "once": once, "twice": c.sums(),
                      "slots_left": int(lib.b200dct_capture_slots_left())}
+    # a round trip without metrics, forced onto the TMA family: without a ticket-counter pair, the static tile split
+    x = torch.from_numpy(case_table()["f32_tma"][0]).cuda()
+    out, coef = torch.empty_like(x), torch.empty_like(x)
+    plan = dct.Plan(path=PATH_TMA)
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g, stream=s):
+        dct.roundtrip(x, out=out, coef=coef, plan=plan, stream=s)
+        launches, family = dct.api.last_launch_count(), dct.api.last_path()
+    for replay in (1, 2):
+        out.fill_(float("nan"))
+        coef.fill_(float("nan"))
+        g.replay()
+        torch.cuda.synchronize()
+        arrays[f"plain{replay}_out"] = out.cpu().numpy()
+        arrays[f"plain{replay}_coef"] = coef.cpu().numpy()
+    res["plain"] = {"launches": launches, "path": family, "slots_left": int(lib.b200dct_capture_slots_left())}
     return res
 
 
-def child_static(dct, arrays):
-    """B200DCT_TMA_STATIC=1: an f32 metrics call on the TMA family, and a round trip without metrics."""
-    c = Call(dct, *case_table()["f32_tma"][:4])
-    rc = c(torch.cuda.current_stream())
-    res = {"rc": rc, "launches": dct.api.last_launch_count(), "path": dct.api.last_path(), "sums": c.sums()}
-    arrays["metrics_out"] = c.out.cpu().numpy()
-    arrays["metrics_coef"] = c.coef.cpu().numpy()
-    x = torch.from_numpy(inputs.float_noise(1024, 2048, seed=3)).cuda()
-    coef = torch.empty_like(x)
-    out = dct.roundtrip(x, coef=coef, plan=dct.Plan(path=PATH_TMA))
-    res["plain_path"] = dct.api.last_path()
-    arrays["plain_out"] = out.cpu().numpy()
-    arrays["plain_coef"] = coef.cpu().numpy()
-    return res
-
-
-def run_child(mode, tmp_path, **env):
-    npz = tmp_path / f"{mode}.npz"
-    r = subprocess.run([sys.executable, os.path.abspath(__file__), mode, str(npz)], capture_output=True, text=True,
-                       timeout=600, cwd=ROOT, env={**os.environ, **env})
+def run_child(tmp_path):
+    npz = tmp_path / "pool.npz"
+    r = subprocess.run([sys.executable, os.path.abspath(__file__), str(npz)], capture_output=True, text=True,
+                       timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
     return json.loads(r.stdout.strip().splitlines()[-1]), np.load(npz)
 
@@ -141,7 +142,7 @@ def same_bits(a, b):
 
 
 def test_metrics_with_the_capture_pool_used_up(dct, oracle, tmp_path):
-    res, arrays = run_child("pool", tmp_path)
+    res, arrays = run_child(tmp_path)
     assert res["slots_left_after_fill"] == 0
     for name in case_table():
         r = res[name]
@@ -154,17 +155,13 @@ def test_metrics_with_the_capture_pool_used_up(dct, oracle, tmp_path):
             assert same_bits(arrays[name + "_coef"], coef), name
         assert r["once"] == ordinary(dct, name), name           # the same bits as on a scheduler slot
         assert r["twice"] == [2 * v for v in r["once"]], name   # every replay adds the same sums
-
-
-def test_metrics_with_static_tma_split(dct, oracle, tmp_path):
-    res, arrays = run_child("static", tmp_path, B200DCT_TMA_STATIC="1")
-    assert res["rc"] == 0 and res["launches"] == 1 and res["path"] == "tma", res
-    assert res["sums"] == ordinary(dct, "f32_tma")
+    # the static tile split: one launch on the TMA family, exact, and every replay the same
+    r = res["plain"]
+    assert r["launches"] == 1 and r["path"] == "tma" and r["slots_left"] == 0, r
     out, coef = want(oracle, "f32_tma")
-    assert same_bits(arrays["metrics_out"], out) and same_bits(arrays["metrics_coef"], coef)
-    # a launch without metrics still takes the static split, and stays exact
-    assert res["plain_path"] == "tma"
-    assert same_bits(arrays["plain_out"], out) and same_bits(arrays["plain_coef"], coef)
+    for replay in (1, 2):
+        assert same_bits(arrays[f"plain{replay}_out"], out), replay
+        assert same_bits(arrays[f"plain{replay}_coef"], coef), replay
 
 
 def test_metrics_workspace_size(dct):
@@ -181,6 +178,6 @@ if __name__ == "__main__":
 
     cuda_dct_idct_b200.lib()
     arrays = {}
-    result = {"pool": child_pool, "static": child_static}[sys.argv[1]](cuda_dct_idct_b200, arrays)
-    np.savez(sys.argv[2], **arrays)
+    result = child_pool(cuda_dct_idct_b200, arrays)
+    np.savez(sys.argv[1], **arrays)
     print(json.dumps(result))
