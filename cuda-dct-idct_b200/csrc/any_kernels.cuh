@@ -28,8 +28,8 @@ struct AnyParams {
 template <int TK, int QMODE, int PIX, bool FINV = false>
 __global__ void __launch_bounds__(128, 5) k_any(const __grid_constant__ AnyParams P)
 {
+    static_assert(PIX == DT_F32, "8-bit images take k_any_u8");
     constexpr bool BIASED = inverse_is_biased(TK, FINV);
-    using elem_t = typename std::conditional<PIX == DT_F32, float, uint8_t>::type;
     __shared__ __align__(16) uint32_t stage[4][8 * 256];
     const int lane = threadIdx.x;
     const long long y0 = ((long long)blockIdx.x * 4 + threadIdx.y) * 8;
@@ -55,7 +55,7 @@ __global__ void __launch_bounds__(128, 5) k_any(const __grid_constant__ AnyParam
     sfor<8>([&](auto s) { xs[IC(s)] = xw + 32 * IC(s) < P.W ? xw + 32 * IC(s) : P.W - 1; });
     sfor<8>([&](auto r) {
         const long long y = y0 + IC(r) < P.H ? y0 + IC(r) : P.H - 1;
-        const elem_t *row = reinterpret_cast<const elem_t *>((const char *)P.in + (size_t)y * P.in_pitch);
+        const float *row = reinterpret_cast<const float *>((const char *)P.in + (size_t)y * P.in_pitch);
         sfor<8>([&](auto s) { st[IC(r) * 256 + 32 * IC(s) + ((IC(s) & 1) ? lane_odd : lane)] = __float_as_uint((float)row[xs[IC(s)]] - 128.0f); });
     });
     __syncwarp();
@@ -70,17 +70,8 @@ __global__ void __launch_bounds__(128, 5) k_any(const __grid_constant__ AnyParam
 
     run_block<MODE_RT, TK, QMODE, true, FINV>(p, P.cp, [](float2 (&)[8][4]) {});
 
-    // blocks -> stage: the final element value (f32 bits, or the u8 value) per pixel
-    auto fin = [](float v) -> uint32_t {
-        const float o = BIASED ? v : v + 128.0f; // add_matrix_scalar, utils_kernels.cu:29
-        if constexpr (PIX == DT_F32) {
-            return __float_as_uint(o);
-        } else {
-            uint32_t b;
-            asm("cvt.rzi.sat.u8.f32 %0, %1;" : "=r"(b) : "f"(o)); // convertToUnsignedChar, utils.cu:21
-            return b;
-        }
-    };
+    // blocks -> stage: the final pixel value per pixel
+    auto fin = [](float v) -> uint32_t { return __float_as_uint(BIASED ? v : v + 128.0f); }; // add_matrix_scalar, utils_kernels.cu:29
     sfor<8>([&](auto r) {
         *reinterpret_cast<uint4 *>(st + IC(r) * 256 + blk_a) =
             make_uint4(fin(p[IC(r)][0].x), fin(p[IC(r)][0].y), fin(p[IC(r)][1].x), fin(p[IC(r)][1].y));
@@ -90,13 +81,9 @@ __global__ void __launch_bounds__(128, 5) k_any(const __grid_constant__ AnyParam
     __syncwarp();
     sfor<8>([&](auto r) {
         if (y0 + IC(r) < P.H) {
-            elem_t *row = reinterpret_cast<elem_t *>((char *)P.out + (size_t)(y0 + IC(r)) * P.out_pitch);
+            float *row = reinterpret_cast<float *>((char *)P.out + (size_t)(y0 + IC(r)) * P.out_pitch);
             sfor<8>([&](auto s) {
-                if (xw + 32 * IC(s) < P.W) {
-                    const uint32_t v = st[IC(r) * 256 + 32 * IC(s) + ((IC(s) & 1) ? lane_odd : lane)];
-                    if constexpr (PIX == DT_F32) row[xw + 32 * IC(s)] = __uint_as_float(v);
-                    else row[xw + 32 * IC(s)] = (uint8_t)v;
-                }
+                if (xw + 32 * IC(s) < P.W) row[xw + 32 * IC(s)] = __uint_as_float(st[IC(r) * 256 + 32 * IC(s) + ((IC(s) & 1) ? lane_odd : lane)]);
             });
         }
     });

@@ -56,7 +56,7 @@ namespace b200dct {
 void note_launch(int launches, const char *path)
 {
     tl_launches = launches;
-    tl_path = path;
+    if (path) tl_path = path;
 }
 } // namespace b200dct
 
@@ -65,7 +65,6 @@ static void plan_refresh(b200dct_plan *pl)
     pl->sparse = true;
     pl->q_default = true;
     pl->q_fastdiv = true;
-    pl->qc_default = true;
     pl->qc_fastdiv = true;
     for (int k = 0; k < 64; k++) {
         const float h = haweel(k / 8, k % 8);
@@ -78,12 +77,10 @@ static void plan_refresh(b200dct_plan *pl)
         pl->cp.q.rcp[k] = 1.0f / d; // IEEE RN on the host
         pl->cp.q.keep[k] = ((pl->mask >> k) & 1) ? 0xffffffffu : 0u;
         const float dc = pl->Qc[k];
-        if (dc != jpeg_q_chroma(k)) pl->qc_default = false;
         if (!(dc >= 1.0f && dc <= 255.0f && dc == floorf(dc))) pl->qc_fastdiv = false;
-        pl->qc.d[k] = dc;
-        pl->qc.neg_d[k] = -dc;
-        pl->qc.rcp[k] = 1.0f / dc;
-        pl->qc.keep[k] = pl->cp.q.keep[k];
+        pl->rgb_t[0].rd[k] = make_float2(pl->cp.q.rcp[k], d);
+        pl->rgb_t[1].rd[k] = make_float2(1.0f / dc, dc);
+        pl->rgb_t[0].keep[k] = pl->rgb_t[1].keep[k] = pl->cp.q.keep[k];
         pl->cp.t.t[k] = pl->T[k];
         pl->cp.t.tt[(k % 8) * 8 + k / 8] = pl->T[k];
     }
@@ -384,10 +381,8 @@ unsigned long long *sched_macc(const uint32_t *slot)
     return g_sched.macc[dev] + MACC_WORDS * ((slot - g_sched.base[dev]) / 2);
 }
 // The counters of a fused-metrics launch: those of its scheduler slot, or without one (capture pool used up,
-// failed ring allocation) the caller's workspace, laid out as
-// {u64 macc[MACC_WORDS]; u32 pair[2]}.  The kernel leaves either zeroed; the workspace starts unknown, so a launch on it
-// is preceded by a memset on its stream and takes no part in the early path.
-constexpr size_t METRICS_WORKSPACE_BYTES = MACC_WORDS * sizeof(unsigned long long) + 2 * sizeof(uint32_t);
+// failed ring allocation) the caller's workspace (METRICS_WORKSPACE_BYTES).  The kernel leaves either zeroed; the
+// workspace starts unknown, so a launch on it is preceded by a memset on its stream and takes no part in the early path.
 struct MetricsCounters {
     uint32_t *pair; // {next ticket, finished CTAs / warps}
     unsigned long long *macc;
@@ -637,12 +632,145 @@ static Span plane_span(const Plane &p, int H, int W)
     return Span{p.ptr, p.pitch, (size_t)W * elem_size(p.dt), H};
 }
 
+// A call of run() whose arguments have passed the checks, and what the family functions share
+struct Call {
+    const b200dct_plan *pl;
+    int mode, pix, coef_dt, H, W;
+    Variant v;
+    Plane in, out, coef;
+    float *shifted;
+    cudaStream_t stream;
+    bool capturing;
+    void *workspace; // fused metrics: the caller's workspace and accumulator (NULL: none)
+    double *acc;
+    Span rd, w0, w1; // the plane the call reads, the planes it writes
+};
+
+// the tensor-core arm of the dense variant (opt-in): f32 fused round trips, optional f32 coefficient plane
+static int run_mma(const Call &c)
+{
+    MmaParams M;
+    memset(&M, 0, sizeof(M));
+    M.in = (const float *)c.in.ptr; M.in_pitch = c.in.pitch;
+    M.out = (float *)const_cast<void *>(c.out.ptr); M.out_pitch = c.out.pitch;
+    M.coef = (float *)const_cast<void *>(c.coef.ptr); M.coef_pitch = c.coef.pitch;
+    M.bx = c.W / 8; M.by = c.H / 8;
+    M.cp = c.pl->cp;
+    dim3 grid;
+    if (!block_grid(M.by, M.bx, grid)) return B200DCT_ERR_SHAPE;
+    return launch_blocks(c.stream, c.capturing, grid, M, false, Span{}, Span{}, Span{}, Span{}, "mma",
+                         [&](const MmaParams &P, bool pdl, int *) { return launch_mma(c.pl->q_fastdiv, P, grid, dim3(32, 4), c.stream, pdl); });
+}
+
+// the persistent TMA family; capture_sched: the ticket-counter pair of a captured launch (NULL: none left, or not capturing)
+static int run_tma(const Call &c, const DevInfo &di, uint32_t *capture_sched)
+{
+    const Plane &in = c.in, &out = c.out, &coef = c.coef;
+    const int H = c.H, W = c.W;
+    TmaParams P;
+    memset(&P, 0, sizeof(P));
+    if (!make_map(&P.in_map, in.ptr, in.dt, in.pitch, H, W) || !make_map(&P.out_map, out.ptr, out.dt, out.pitch, H, W))
+        return B200DCT_ERR_ARG;
+    if (coef.ptr && !make_map(&P.coef_map, coef.ptr, coef.dt, coef.pitch, H, W)) return B200DCT_ERR_ARG;
+    P.tiles_x = (uint32_t)((W + 255) / 256);
+    P.bx = (uint32_t)(W / 8);
+    const unsigned long long nt = (unsigned long long)P.tiles_x * (unsigned long long)(H / 8);
+    if (nt > 0x7fffffffull) return B200DCT_ERR_SHAPE;
+    P.ntiles = (uint32_t)nt;
+    P.coef_dt = c.coef_dt;
+    P.has_coef = coef.ptr ? 1 : 0;
+
+    // dynamic tickets; a captured launch owns its pair (NULL: no pair left, static split)
+    P.sched = c.capturing ? capture_sched : sched_slot(false);
+    P.cp = c.pl->cp;
+    // tile buffers as large as the largest tile image among the planes of this call
+    uint32_t buf = tile_bytes_of(in.dt) > tile_bytes_of(out.dt) ? tile_bytes_of(in.dt) : tile_bytes_of(out.dt);
+    if (coef.ptr && tile_bytes_of(coef.dt) > buf) buf = tile_bytes_of(coef.dt);
+    P.buf_bytes = buf;
+    // warps per CTA: the flavour's CTA size, limited by 227 KiB of shared memory
+    int nw = (c.workspace ? TMA_METRICS_THREADS : tma_cta_threads(c.pix, c.pl->tk)) / 32;
+    const unsigned nbuf = c.workspace ? 3u : 2u; // metrics: two input buffers per warp
+    const int smem_w = (int)((227u * 1024u - 1024u) / (nbuf * buf + 16u));
+    if (nw > smem_w) nw = smem_w;
+    const size_t smem = (size_t)nw * nbuf * buf + (size_t)nw * 16 + 1024;
+    // at most one CTA per SM
+    const unsigned long long want = (nt + nw - 1) / nw, sms = (unsigned long long)di.sms;
+    const int grid = (int)(want < sms ? want : sms);
+    // runs of 2 tiles per ticket while more than two rounds of single tiles remain
+    P.run = 2;
+    const unsigned long long tail = 2ull * (unsigned long long)grid * nw;
+    P.run_tickets = nt > tail ? (uint32_t)((nt - tail) / P.run) : 0u;
+    // Metrics: the dynamic scheduler always, on the counters of the slot or of the workspace; the last warp out
+    // folds the integer sums into acc -- one launch
+    MetricsCounters mc{};
+    if (c.workspace) {
+        mc = metrics_counters(P.sched, c.workspace);
+        P.sched = mc.pair;
+        P.macc = mc.macc;
+        P.acc = c.acc;
+    }
+    const bool pdl = pdl_enabled(c.capturing);
+    // the argument above needs the predecessor to occupy every SM (grid == SM count) and neither
+    // launch to fit beside the other on one SM: both take more than half of its shared memory
+    const bool heavy = smem > (size_t)(di.smem_optin / 2) + 1024;
+    LaunchScope scope(c.stream, mc.in_workspace ? LaunchScope::NONE : LaunchScope::TMA, pdl && heavy && P.sched != nullptr,
+                      (unsigned long long)grid, 1, c.rd, c.w0, c.w1);
+    scope.apply(P);
+    const cudaError_t em = mc.zero(c.stream);
+    if (em != cudaSuccess) return (int)em;
+    const cudaError_t e = launch_tma(c.pl->tk, c.v, c.mode, c.pix, P, grid, nw * 32, smem, c.stream, pdl && !mc.in_workspace);
+    if (e != cudaSuccess) return (int)e;
+    scope.done(true);
+    note_launch(1, "tma");
+    return B200DCT_OK;
+}
+
+// the direct family: hardware-scheduled CTAs, a lane per block
+static int run_direct(const Call &c)
+{
+    DirectParams P;
+    memset(&P, 0, sizeof(P));
+    P.in = c.in.ptr; P.in_pitch = c.in.pitch;
+    P.out = const_cast<void *>(c.out.ptr); P.out_pitch = c.out.pitch;
+    P.coef = const_cast<void *>(c.coef.ptr); P.coef_pitch = c.coef.pitch;
+    P.shifted = c.shifted; P.shifted_pitch = c.in.pitch;
+    P.bx = c.W / 8; P.by = c.H / 8;
+    P.coef_dt = c.coef_dt;
+    P.zz_smem = (c.coef_dt == DT_I16ZZ && !c.workspace) ? 1 : 0; // the metrics kernels are launched without dynamic smem
+    // f32 planes aligned to 32 bytes move with 256-bit accesses
+    auto aligned32 = [](const Plane &pl) { return pl.ptr && pl.dt == DT_F32 && !((uintptr_t)pl.ptr & 31) && !(pl.pitch & 31); };
+    P.v8 = (aligned32(c.in) ? 1 : 0) | (aligned32(c.out) ? 2 : 0) | (aligned32(c.coef) ? 4 : 0);
+    P.cp = c.pl->cp;
+    dim3 grid;
+    if (!block_grid(P.by, P.bx, grid)) return B200DCT_ERR_SHAPE;
+    const bool metrics = c.workspace != nullptr;
+    MetricsCounters mc{};
+    if (metrics) {
+        if (c.mode != MODE_RT || c.in.ptr == c.out.ptr) return B200DCT_ERR_ARG;
+        // One launch: integer sums through 64-bit atomics into the accumulator of a ticket-counter pair, the last
+        // CTA out folds them into acc (the TMA family's scheme).  Dependent launch and the early path apply on a slot.
+        mc = metrics_counters(sched_slot(c.capturing), c.workspace);
+        P.macc = mc.macc;
+        P.mdone = mc.pair;
+        P.acc = c.acc;
+    }
+    // the early path: fused round trips without a coefficient plane, forward calls without the X-128 write-back,
+    // inverse calls whose coefficients are a plane (not the zig-zag stream)
+    const bool may_load_early = !c.coef.ptr && !c.shifted && !(c.mode == MODE_INV && c.in.dt == DT_I16ZZ);
+    const Span w2 = metrics ? Span{c.acc, 0, 3 * sizeof(double), 1} : Span{c.shifted, c.in.pitch, (size_t)c.W * 4, c.H};
+    return launch_blocks(c.stream, c.capturing, grid, P, true, may_load_early ? c.rd : Span{}, c.w0, c.w1, w2, "direct",
+                         [&](const DirectParams &Q, bool pdl, int *per_sm) {
+                             return launch_direct(c.pl->tk, c.v, c.mode, c.pix, metrics, Q, grid, dim3(32, 4), c.stream, pdl, per_sm);
+                         },
+                         mc.in_workspace ? mc.macc : nullptr);
+}
+
 static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef, float *shifted, int H, int W,
                cudaStream_t stream, void *workspace = nullptr, double *acc = nullptr)
 {
-    tl_launches = 0;
+    note_launch(0);
     if (!pl) return B200DCT_ERR_ARG;
-    if (H <= 0 || W <= 0 || (H % 8) || (W % 8)) return B200DCT_ERR_SHAPE;
+    if (!whole_blocks(H, W)) return B200DCT_ERR_SHAPE;
     int rc;
     if ((rc = check_plane(in, W, mode != MODE_INV)) != 0) return rc;
     if ((rc = check_plane(out, W, mode != MODE_FWD)) != 0) return rc;
@@ -655,7 +783,9 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
 
     const int pix = (mode == MODE_INV) ? out.dt : in.dt;
     const int coef_dt = (mode == MODE_FWD) ? out.dt : (mode == MODE_INV ? in.dt : (coef.ptr ? coef.dt : DT_F32));
-    const Variant v = variant_of(pl, mode, pix, workspace != nullptr); // the metrics kernels take runtime masks
+    // the metrics kernels take runtime masks
+    const Call c{pl, mode, pix, coef_dt, H, W, variant_of(pl, mode, pix, workspace != nullptr), in, out, coef, shifted, stream,
+                 stream_capturing(stream), workspace, acc, plane_span(in, H, W), plane_span(out, H, W), plane_span(coef, H, W)};
 
     // AUTO: the TMA family wins where the call is HBM-bound (>= 4 bytes moved per pixel: any
     // f32/i16 plane); all-u8 round trips move 2 B/px, are instruction-issue bound, and run faster
@@ -674,146 +804,24 @@ static int run(const b200dct_plan *pl, int mode, Plane in, Plane out, Plane coef
     // dense kernels stay on the direct family.
     // (TMA_HUGE_PIXELS = 64 Mpixel)
     const bool prefer_tma = prefers_tma(pl, bytes_per_px, H, W);
-    // Under stream capture the launch takes a ticket-counter pair of its own (see SchedRing); when
-    // none is left (or the pools do not exist yet) AUTO falls back to the hardware-scheduled
-    // direct family (86.9 us at 8192^2), which beats the TMA family's static split (99.8 us).
-    const bool capturing = stream_capturing(stream);
-    const bool pdl = pdl_enabled(capturing);
     // fused metrics on the TMA family: f32 round trips of Haweel's T (the input tile is compared where it
     // already is, in shared memory); everything else takes the direct family's metrics kernels
     const bool metrics_tma_ok = !workspace || (mode == MODE_RT && in.dt == DT_F32 && pl->tk == TK_HAWEEL && in.ptr != out.ptr);
     const bool tma_possible = pl->path != B200DCT_PATH_DIRECT && prefer_tma && !shifted && metrics_tma_ok && get_encode() != nullptr &&
                               tma_plane_ok(in.ptr, in.dt, in.pitch, W) && tma_plane_ok(out.ptr, out.dt, out.pitch, W) &&
                               (!coef.ptr || tma_plane_ok(coef.ptr, coef.dt, coef.pitch, W));
+    // Under stream capture the launch takes a ticket-counter pair of its own (see SchedRing); when
+    // none is left (or the pools do not exist yet) AUTO falls back to the hardware-scheduled
+    // direct family (86.9 us at 8192^2), which beats the TMA family's static split (99.8 us).
     uint32_t *capture_sched = nullptr;
-    if (capturing && tma_possible) capture_sched = sched_slot(true);
-    const bool use_tma = tma_possible && !(capturing && !capture_sched && pl->path == B200DCT_PATH_AUTO);
+    if (c.capturing && tma_possible) capture_sched = sched_slot(true);
+    const bool use_tma = tma_possible && !(c.capturing && !capture_sched && pl->path == B200DCT_PATH_AUTO);
     if (pl->path == B200DCT_PATH_TMA && !use_tma) return B200DCT_ERR_ALIGN;
-    const Span rd = plane_span(in, H, W), w0 = plane_span(out, H, W), w1 = plane_span(coef, H, W);
-    // the tensor-core arm of the dense variant (opt-in): f32 fused round trips, optional f32 coefficient plane
     if (pl->dense == B200DCT_DENSE_MMA && !pl->sparse && mode == MODE_RT && in.dt == DT_F32 && !workspace && !shifted &&
-        (!coef.ptr || coef.dt == DT_F32)) {
-        MmaParams M;
-        memset(&M, 0, sizeof(M));
-        M.in = (const float *)in.ptr; M.in_pitch = in.pitch;
-        M.out = (float *)const_cast<void *>(out.ptr); M.out_pitch = out.pitch;
-        M.coef = (float *)const_cast<void *>(coef.ptr); M.coef_pitch = coef.pitch;
-        M.bx = W / 8; M.by = H / 8;
-        M.cp = pl->cp;
-        dim3 mblock(32, 4), mgrid((unsigned)((M.by + 3) / 4), (unsigned)((M.bx + 31) / 32));
-        if (mgrid.y > 65535u) return B200DCT_ERR_SHAPE;
-        LaunchScope order(stream);
-        const cudaError_t em = launch_mma(pl->q_fastdiv, M, mgrid, mblock, stream, pdl);
-        if (em != cudaSuccess) return (int)em;
-        tl_launches = 1;
-        tl_path = "mma";
-        return B200DCT_OK;
-    }
-
-    if (use_tma) {
-        TmaParams P;
-        memset(&P, 0, sizeof(P));
-        if (!make_map(&P.in_map, in.ptr, in.dt, in.pitch, H, W) || !make_map(&P.out_map, out.ptr, out.dt, out.pitch, H, W))
-            return B200DCT_ERR_ARG;
-        if (coef.ptr && !make_map(&P.coef_map, coef.ptr, coef.dt, coef.pitch, H, W)) return B200DCT_ERR_ARG;
-        P.tiles_x = (uint32_t)((W + 255) / 256);
-        P.bx = (uint32_t)(W / 8);
-        const unsigned long long nt = (unsigned long long)P.tiles_x * (unsigned long long)(H / 8);
-        if (nt > 0x7fffffffull) return B200DCT_ERR_SHAPE;
-        P.ntiles = (uint32_t)nt;
-        P.coef_dt = coef_dt;
-        P.has_coef = coef.ptr ? 1 : 0;
-
-        // dynamic tickets; a captured launch owns its pair (NULL: no pair left, static split)
-        P.sched = capturing ? capture_sched : sched_slot(false);
-        P.cp = pl->cp;
-        // tile buffers as large as the largest tile image among the planes of this call
-        uint32_t buf = tile_bytes_of(in.dt) > tile_bytes_of(out.dt) ? tile_bytes_of(in.dt) : tile_bytes_of(out.dt);
-        if (coef.ptr && tile_bytes_of(coef.dt) > buf) buf = tile_bytes_of(coef.dt);
-        P.buf_bytes = buf;
-        // warps per CTA: the flavour's CTA size, limited by 227 KiB of shared memory
-        int nw = (workspace ? TMA_METRICS_THREADS : tma_cta_threads(pix, pl->tk)) / 32;
-        const unsigned nbuf = workspace ? 3u : 2u; // metrics: two input buffers per warp
-        const int smem_w = (int)((227u * 1024u - 1024u) / (nbuf * buf + 16u));
-        if (nw > smem_w) nw = smem_w;
-        const size_t smem = (size_t)nw * nbuf * buf + (size_t)nw * 16 + 1024;
-        // at most one CTA per SM
-        const unsigned long long want = (nt + nw - 1) / nw, sms = (unsigned long long)di.sms;
-        const int grid = (int)(want < sms ? want : sms);
-        // runs of 2 tiles per ticket while more than two rounds of single tiles remain
-        P.run = 2;
-        const unsigned long long tail = 2ull * (unsigned long long)grid * nw;
-        P.run_tickets = nt > tail ? (uint32_t)((nt - tail) / P.run) : 0u;
-        // Metrics: the dynamic scheduler always, on the counters of the slot or of the workspace; the last warp out
-        // folds the integer sums into acc -- one launch
-        MetricsCounters mc{};
-        if (workspace) {
-            mc = metrics_counters(P.sched, workspace);
-            P.sched = mc.pair;
-            P.macc = mc.macc;
-            P.acc = acc;
-        }
-        // the argument above needs the predecessor to occupy every SM (grid == SM count) and neither
-        // launch to fit beside the other on one SM: both take more than half of its shared memory
-        const bool heavy = smem > (size_t)(di.smem_optin / 2) + 1024;
-        LaunchScope scope(stream, mc.in_workspace ? LaunchScope::NONE : LaunchScope::TMA, pdl && heavy && P.sched != nullptr,
-                          (unsigned long long)grid, 1, rd, w0, w1);
-        scope.apply(P);
-        const cudaError_t em = mc.zero(stream);
-        if (em != cudaSuccess) return (int)em;
-        const cudaError_t e = launch_tma(pl->tk, v, mode, pix, P, grid, nw * 32, smem, stream, pdl && !mc.in_workspace);
-        if (e != cudaSuccess) return (int)e;
-        scope.done(true);
-        tl_launches = 1;
-        tl_path = "tma";
-        return B200DCT_OK;
-    }
-
-    DirectParams P;
-    memset(&P, 0, sizeof(P));
-    P.in = in.ptr; P.in_pitch = in.pitch;
-    P.out = const_cast<void *>(out.ptr); P.out_pitch = out.pitch;
-    P.coef = const_cast<void *>(coef.ptr); P.coef_pitch = coef.pitch;
-    P.shifted = shifted; P.shifted_pitch = in.pitch;
-    P.bx = W / 8; P.by = H / 8;
-    P.coef_dt = coef_dt;
-    P.zz_smem = (coef_dt == DT_I16ZZ && !workspace) ? 1 : 0; // the metrics kernels are launched without dynamic smem
-    // f32 planes aligned to 32 bytes move with 256-bit accesses
-    auto aligned32 = [](const Plane &pl) { return pl.ptr && pl.dt == DT_F32 && !((uintptr_t)pl.ptr & 31) && !(pl.pitch & 31); };
-    P.v8 = (aligned32(in) ? 1 : 0) | (aligned32(out) ? 2 : 0) | (aligned32(coef) ? 4 : 0);
-    P.cp = pl->cp;
-    dim3 block(32, 4);
-    dim3 grid((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32));
-    if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
-    const bool metrics = workspace != nullptr;
-    MetricsCounters mc{};
-    if (metrics) {
-        if (mode != MODE_RT || in.ptr == out.ptr) return B200DCT_ERR_ARG;
-        // One launch: integer sums through 64-bit atomics into the accumulator of a ticket-counter pair, the last
-        // CTA out folds them into acc (the TMA family's scheme).  Dependent launch and the early path apply on a slot.
-        mc = metrics_counters(sched_slot(capturing), workspace);
-        P.macc = mc.macc;
-        P.mdone = mc.pair;
-        P.acc = acc;
-    }
-    const bool usable = pdl && !mc.in_workspace;
-    int per_sm = 0;
-    if (usable) launch_direct(pl->tk, v, mode, pix, metrics, P, grid, block, stream, pdl, &per_sm);
-    // the early path: fused round trips without a coefficient plane, forward calls without the X-128 write-back,
-    // inverse calls whose coefficients are a plane (not the zig-zag stream)
-    const bool may_load_early = !coef.ptr && !shifted && !(mode == MODE_INV && in.dt == DT_I16ZZ);
-    const Span w2 = metrics ? Span{acc, 0, 3 * sizeof(double), 1} : Span{shifted, in.pitch, (size_t)W * 4, H};
-    LaunchScope scope(stream, mc.in_workspace ? LaunchScope::NONE : LaunchScope::DIRECT, usable, (unsigned long long)grid.x * grid.y,
-                      per_sm, may_load_early ? rd : Span{}, w0, w1, w2);
-    scope.apply(P);
-    const cudaError_t em = mc.zero(stream);
-    if (em != cudaSuccess) return (int)em;
-    const cudaError_t e = launch_direct(pl->tk, v, mode, pix, metrics, P, grid, block, stream, pdl && !mc.in_workspace);
-    if (e != cudaSuccess) return (int)e;
-    scope.done(true);
-    tl_launches = 1;
-    tl_path = "direct";
-    return B200DCT_OK;
+        (!coef.ptr || coef.dt == DT_F32))
+        return run_mma(c);
+    if (use_tma) return run_tma(c, di, capture_sched);
+    return run_direct(c);
 }
 
 extern "C" int b200dct_forward(const b200dct_plan *plan, const void *img, b200dct_dtype img_dt, size_t img_pitch,
@@ -848,10 +856,10 @@ extern "C" int b200dct_roundtrip(const b200dct_plan *plan, const void *img, b200
 extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, const void *const *imgs, void *const *outs,
                                        b200dct_dtype dt, size_t in_pitch, size_t out_pitch, int H, int W, void *stream)
 {
-    tl_launches = 0;
+    note_launch(0);
     if (!plan || n_images < 0 || (n_images > 0 && (!imgs || !outs))) return B200DCT_ERR_ARG;
     if (dt != B200DCT_F32 && dt != B200DCT_U8) return B200DCT_ERR_ARG;
-    if (H <= 0 || W <= 0 || (H % 8) || (W % 8)) return B200DCT_ERR_SHAPE;
+    if (!whole_blocks(H, W)) return B200DCT_ERR_SHAPE;
     for (int i = 0; i < n_images; i++) {
         int rc;
         if ((rc = check_plane(Plane{imgs[i], (int)dt, in_pitch}, W, true)) != 0) return rc;
@@ -874,8 +882,7 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
             launches += tl_launches;
             path = tl_path;
         }
-        tl_launches = launches;
-        tl_path = path;
+        note_launch(launches, path);
         return B200DCT_OK;
     }
     const Variant v = variant_of(plan, MODE_RT, (int)dt, false);
@@ -889,9 +896,8 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
     bool v8 = dt == B200DCT_F32 && !(in_pitch & 31) && !(out_pitch & 31);
     for (int i = 0; v8 && i < n_images; i++) v8 = !((uintptr_t)imgs[i] & 31) && !((uintptr_t)outs[i] & 31);
     P.v8 = v8 ? 3 : 0;
-    dim3 block(32, 4);
-    dim3 grid((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32), 1);
-    if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
+    dim3 grid;
+    if (!block_grid(P.by, P.bx, grid)) return B200DCT_ERR_SHAPE;
     LaunchScope order(s);
     int launches = 0;
     for (int first = 0; first < n_images; first += DIRECT_BATCH_MAX) {
@@ -903,12 +909,11 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
         }
         P.in = P.img_in[0]; P.out = P.img_out[0];
         grid.z = (unsigned)n;
-        const cudaError_t e = launch_direct(plan->tk, v, MODE_RT, (int)dt, false, P, grid, block, s, pdl);
+        const cudaError_t e = launch_direct(plan->tk, v, MODE_RT, (int)dt, false, P, grid, dim3(32, 4), s, pdl);
         if (e != cudaSuccess) return (int)e;
         launches++;
     }
-    tl_launches = launches;
-    tl_path = "direct";
+    note_launch(launches, "direct");
     return B200DCT_OK;
 }
 
@@ -916,14 +921,14 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
 extern "C" int b200dct_roundtrip_any(const b200dct_plan *plan, const void *img, b200dct_dtype dt, size_t in_pitch,
                                      void *out, size_t out_pitch, int H, int W, void *stream)
 {
-    tl_launches = 0;
+    note_launch(0);
     if (!plan || !img || !out || H <= 0 || W <= 0) return B200DCT_ERR_ARG;
     if (dt != B200DCT_F32 && dt != B200DCT_U8) return B200DCT_ERR_ARG;
     const size_t es = elem_size((int)dt);
     if (in_pitch < (size_t)W * es || out_pitch < (size_t)W * es) return B200DCT_ERR_SHAPE;
     if (((uintptr_t)img % es) || ((uintptr_t)out % es) || (in_pitch % es) || (out_pitch % es)) return B200DCT_ERR_ALIGN;
     const size_t al = dt == B200DCT_U8 ? 8 : 16;
-    const bool fast = !(H % 8) && !(W % 8) && !((uintptr_t)img % al) && !((uintptr_t)out % al) && !(in_pitch % al) &&
+    const bool fast = whole_blocks(H, W) && !((uintptr_t)img % al) && !((uintptr_t)out % al) && !(in_pitch % al) &&
                       !(out_pitch % al);
     if (fast) return b200dct_roundtrip(plan, img, dt, in_pitch, out, dt, out_pitch, nullptr, B200DCT_F32, 0, H, W, stream);
     // everything else: one pass of the edge-replicating scalar-access kernel, no scratch image
@@ -937,16 +942,11 @@ extern "C" int b200dct_roundtrip_any(const b200dct_plan *plan, const void *img, 
     P.H = H; P.W = W;
     P.cp = plan->cp;
     const Variant v = variant_of(plan, MODE_RT, (int)dt, true); // finv only for 8-bit pixels
-    const unsigned nby = (unsigned)((H + 7) / 8), nbx = (unsigned)((W + 7) / 8);
-    dim3 block(32, 4), grid((nby + 3) / 4, (nbx + 31) / 32);
-    if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
-    const bool pdl = pdl_enabled(stream_capturing(s));
-    LaunchScope order(s);
-    const cudaError_t e = (dt == B200DCT_F32 ? launch_any_f32 : launch_any_u8)(plan->tk, v.qm, v.finv, P, grid, block, s, pdl);
-    if (e != cudaSuccess) return (int)e;
-    tl_launches = 1;
-    tl_path = "any";
-    return B200DCT_OK;
+    dim3 grid;
+    if (!block_grid((H + 7) / 8, (W + 7) / 8, grid)) return B200DCT_ERR_SHAPE;
+    const auto launch_any = dt == B200DCT_F32 ? launch_any_f32 : launch_any_u8;
+    return launch_blocks(s, stream_capturing(s), grid, P, false, Span{}, Span{}, Span{}, Span{}, "any",
+                         [&](const AnyParams &Q, bool pdl, int *) { return launch_any(plan->tk, v.qm, v.finv, Q, grid, dim3(32, 4), s, pdl); });
 }
 
 extern "C" size_t b200dct_metrics_workspace_bytes(int H, int W)
@@ -1005,7 +1005,7 @@ extern "C" int b200dct_time_calls(const b200dct_plan *plan, int which, const voi
     }
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
-    tl_launches = launches;
+    note_launch(launches);
     return rc;
 }
 
@@ -1044,7 +1044,7 @@ __global__ void k_metrics(const T *__restrict__ a, const T *__restrict__ b, size
 extern "C" int b200dct_metrics_accumulate(const void *ref_img, const void *test_img, b200dct_dtype dt, size_t pitch,
                                           int H, int W, double *d_acc, void *stream)
 {
-    tl_launches = 0;
+    note_launch(0);
     if (!ref_img || !test_img || !d_acc || H <= 0 || W <= 0) return B200DCT_ERR_ARG;
     const DevInfo di = dev_info();
     if (!di.ok) return B200DCT_ERR_NODEVICE;
@@ -1057,7 +1057,7 @@ extern "C" int b200dct_metrics_accumulate(const void *ref_img, const void *test_
         return B200DCT_ERR_ARG;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return (int)e;
-    tl_launches = 1;
+    note_launch(1);
     return B200DCT_OK;
 }
 

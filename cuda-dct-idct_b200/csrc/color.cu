@@ -18,7 +18,7 @@ using RgbLauncher = cudaError_t (*)(const RgbParams &, dim3, dim3, size_t, cudaS
 static int rgb_params(const b200dct_plan *plan, const void *rgb_in, size_t in_pitch, void *rgb_out, size_t out_pitch,
                       void *zz, size_t zz_plane_bytes, int H, int W, RgbParams &P, dim3 &grid)
 {
-    if (H <= 0 || W <= 0 || (H % 8) || (W % 8)) return B200DCT_ERR_SHAPE;
+    if (!whole_blocks(H, W)) return B200DCT_ERR_SHAPE;
     if ((rgb_in && in_pitch < (size_t)W * 3) || (rgb_out && out_pitch < (size_t)W * 3)) return B200DCT_ERR_SHAPE;
     if (((uintptr_t)rgb_in & 7) || ((uintptr_t)rgb_out & 7) || (in_pitch & 7) || (out_pitch & 7)) return B200DCT_ERR_ALIGN;
     if (!plan->sparse) return B200DCT_ERR_ARG; // the colour path is built for Haweel's T (the reference's HpApprDCT)
@@ -32,15 +32,8 @@ static int rgb_params(const b200dct_plan *plan, const void *rgb_in, size_t in_pi
     P.out = rgb_out; P.out_pitch = out_pitch;
     P.zz = zz; P.zz_plane = zz_plane_bytes; P.zz_pitch = (size_t)(W / 8) * 128;
     P.bx = W / 8; P.by = H / 8;
-    for (int k = 0; k < 64; k++) {
-        P.t[0].rd[k] = make_float2(plan->cp.q.rcp[k], plan->cp.q.d[k]);
-        P.t[0].keep[k] = plan->cp.q.keep[k];
-        P.t[1].rd[k] = make_float2(plan->qc.rcp[k], plan->qc.d[k]);
-        P.t[1].keep[k] = plan->qc.keep[k];
-    }
-    grid = dim3((unsigned)((P.by + 3) / 4), (unsigned)((P.bx + 31) / 32));
-    if (grid.y > 65535u) return B200DCT_ERR_SHAPE;
-    return B200DCT_OK;
+    memcpy(P.t, plan->rgb_t, sizeof(P.t));
+    return block_grid(P.by, P.bx, grid) ? B200DCT_OK : B200DCT_ERR_SHAPE;
 }
 static Span rgb_span(const void *p, size_t pitch, int H, int W) { return Span{p, pitch, (size_t)W * 3, H}; }
 static Span zz_span(const void *zz, size_t plane_bytes, int H, int W) { return Span{zz, plane_bytes, (size_t)(H / 8) * (size_t)(W / 8) * 128, 3}; }
@@ -50,24 +43,15 @@ static int rgb_qk(const b200dct_plan *plan)
 {
     return (!plan->q_fastdiv || !plan->qc_fastdiv) ? 2 : (plan->mask == ~(uint64_t)0 ? 0 : 1);
 }
-// One launch of a colour kernel.  Early path across launch boundaries (b200dct.cu, "early loads"): a pass whose
+// One launch of a colour kernel, in the early path across launch boundaries (b200dct.cu, "early loads"): a pass whose
 // input `rd` is not written by the library's previous machine-filling launch on this stream reads and computes
 // before it waits (rd.ptr NULL: never); w0 .. w2 are what the launch writes.
 template <class Params> // RgbParams, Rgb420Params
 static int run_rgb(cudaError_t (*launch)(const Params &, dim3, dim3, size_t, cudaStream_t, bool, int *), Params &P, dim3 grid,
                    cudaStream_t s, Span rd, Span w0, Span w1, Span w2 = Span{})
 {
-    const bool pdl = pdl_enabled(stream_capturing(s));
-    const dim3 block(32, 4);
-    int per_sm = 0;
-    if (pdl) launch(P, grid, block, 0, s, pdl, &per_sm);
-    LaunchScope scope(s, LaunchScope::DIRECT, pdl, (unsigned long long)grid.x * grid.y, per_sm, rd, w0, w1, w2);
-    scope.apply(P);
-    const cudaError_t e = launch(P, grid, block, 0, s, pdl, nullptr);
-    if (e != cudaSuccess) return (int)e;
-    scope.done(true);
-    note_launch(1, "rgb");
-    return B200DCT_OK;
+    return launch_blocks(s, stream_capturing(s), grid, P, true, rd, w0, w1, w2, "rgb",
+                         [&](const Params &Q, bool pdl, int *per_sm) { return launch(Q, grid, dim3(32, 4), 0, s, pdl, per_sm); });
 }
 
 extern "C" int b200dct_roundtrip_rgb(const b200dct_plan *plan, const void *rgb, size_t in_pitch, void *out,
@@ -127,15 +111,16 @@ using Rgb420Launcher = cudaError_t (*)(const Rgb420Params &, dim3, dim3, size_t,
 
 // The argument rules of the 4:2:0 entry points: those of the 4:4:4 calls, H and W multiples of 16, and three
 // tightly packed streams, each 16-byte aligned.
+// grid: the forward kernel's (16 x 2 MCUs per CTA)
 static int rgb420_params(const b200dct_plan *plan, const void *rgb_in, size_t in_pitch, void *rgb_out, size_t out_pitch,
-                         const void *zy, const void *zcb, const void *zcr, int H, int W, Rgb420Params &P)
+                         const void *zy, const void *zcb, const void *zcr, int H, int W, Rgb420Params &P, dim3 &grid)
 {
-    if (H <= 0 || W <= 0 || (H % 16) || (W % 16)) return B200DCT_ERR_SHAPE;
+    if (!whole_blocks(H, W, 16)) return B200DCT_ERR_SHAPE;
     if ((rgb_in && in_pitch < (size_t)W * 3) || (rgb_out && out_pitch < (size_t)W * 3)) return B200DCT_ERR_SHAPE;
     if (((uintptr_t)rgb_in & 7) || ((uintptr_t)rgb_out & 7) || (in_pitch & 7) || (out_pitch & 7)) return B200DCT_ERR_ALIGN;
     if (((uintptr_t)zy & 15) || ((uintptr_t)zcb & 15) || ((uintptr_t)zcr & 15)) return B200DCT_ERR_ALIGN;
     if (!plan->sparse) return B200DCT_ERR_ARG; // Haweel's T only, as the 4:4:4 calls
-    if ((W / 8 + 31) / 32 > 65535) return B200DCT_ERR_SHAPE;
+    if (!block_grid(H / 8, W / 8, grid)) return B200DCT_ERR_SHAPE;
     int dev = -1;
     if (cudaGetDevice(&dev) != cudaSuccess) return B200DCT_ERR_NODEVICE;
 
@@ -145,12 +130,7 @@ static int rgb420_params(const b200dct_plan *plan, const void *rgb_in, size_t in
     P.zz[0] = const_cast<void *>(zy); P.zz[1] = const_cast<void *>(zcb); P.zz[2] = const_cast<void *>(zcr);
     P.zz_pitch[0] = (size_t)(W / 8) * 128; P.zz_pitch[1] = (size_t)(W / 16) * 128;
     P.mx = W / 16; P.my = H / 16;
-    for (int k = 0; k < 64; k++) {
-        P.t[0].rd[k] = make_float2(plan->cp.q.rcp[k], plan->cp.q.d[k]);
-        P.t[0].keep[k] = plan->cp.q.keep[k];
-        P.t[1].rd[k] = make_float2(plan->qc.rcp[k], plan->qc.d[k]);
-        P.t[1].keep[k] = plan->qc.keep[k];
-    }
+    memcpy(P.t, plan->rgb_t, sizeof(P.t));
     return B200DCT_OK;
 }
 static Span y_span(const void *zz, int H, int W) { return Span{zz, (size_t)(W / 8) * 128, (size_t)(W / 8) * 128, H / 8}; }
@@ -161,11 +141,11 @@ extern "C" int b200dct_forward_rgb420(const b200dct_plan *plan, const void *rgb,
     note_launch(0, "none");
     if (!plan || !rgb || !zz_y || !zz_cb || !zz_cr) return B200DCT_ERR_ARG;
     Rgb420Params P;
-    const int rc = rgb420_params(plan, rgb, in_pitch, nullptr, 0, zz_y, zz_cb, zz_cr, H, W, P);
+    dim3 grid;
+    const int rc = rgb420_params(plan, rgb, in_pitch, nullptr, 0, zz_y, zz_cb, zz_cr, H, W, P, grid);
     if (rc != B200DCT_OK) return rc;
     static const Rgb420Launcher launchers[3] = {launch_kernel<k_rgb420_forward<0>>, launch_kernel<k_rgb420_forward<1>>,
                                                 launch_kernel<k_rgb420_forward<2>>};
-    const dim3 grid((unsigned)((H / 8 + 3) / 4), (unsigned)((W / 8 + 31) / 32)); // 16 x 2 MCUs per CTA
     return run_rgb(launchers[rgb_qk(plan)], P, grid, (cudaStream_t)stream, rgb_span(rgb, in_pitch, H, W), y_span(zz_y, H, W),
                       c_span(zz_cb, H, W), c_span(zz_cr, H, W));
 }
@@ -176,10 +156,11 @@ extern "C" int b200dct_inverse_rgb420(const b200dct_plan *plan, const void *zz_y
     note_launch(0, "none");
     if (!plan || !zz_y || !zz_cb || !zz_cr || !out) return B200DCT_ERR_ARG;
     Rgb420Params P;
-    const int rc = rgb420_params(plan, nullptr, 0, out, out_pitch, zz_y, zz_cb, zz_cr, H, W, P);
+    dim3 grid;
+    const int rc = rgb420_params(plan, nullptr, 0, out, out_pitch, zz_y, zz_cb, zz_cr, H, W, P, grid);
     if (rc != B200DCT_OK) return rc;
     static const Rgb420Launcher launchers[2] = {launch_kernel<k_rgb420_inverse<false>>, launch_kernel<k_rgb420_inverse<true>>};
-    const dim3 grid((unsigned)((P.my + R420_MY - 1) / R420_MY), (unsigned)((P.mx + R420_MX - 1) / R420_MX));
+    grid = dim3((unsigned)((P.my + R420_MY - 1) / R420_MY), (unsigned)((P.mx + R420_MX - 1) / R420_MX));
     // the early path's read span: the range that bounds the three streams (conservative when they lie apart)
     const Span sp[3] = {y_span(zz_y, H, W), c_span(zz_cb, H, W), c_span(zz_cr, H, W)};
     uintptr_t lo = ~(uintptr_t)0, hi = 0;
@@ -321,7 +302,7 @@ extern "C" int b200dct_zigzag_coded_bits(const void *zz, size_t pitch, int H, in
 {
     note_launch(0, "none");
     if (!zz || !d_bits || (table != 0 && table != 1)) return B200DCT_ERR_ARG;
-    if (H <= 0 || W <= 0 || (H % 8) || (W % 8) || pitch < (size_t)(W / 8) * 128) return B200DCT_ERR_SHAPE;
+    if (!whole_blocks(H, W) || pitch < (size_t)(W / 8) * 128) return B200DCT_ERR_SHAPE;
     if (((uintptr_t)zz & 15) || (pitch & 15) || ((uintptr_t)d_bits & 7)) return B200DCT_ERR_ALIGN;
     int dev = -1, sms = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)

@@ -8,12 +8,12 @@
 // across slots (both copy engines and the SMs busy at once).  The slot ring simply carries on
 // from one image to the next, so consecutive submissions overlap as well: image i+1 is uploading
 // while image i is still on its way back -- no fill/drain bubble per image.
-#include "b200dct.h"
-
 #include <cuda_runtime.h>
 #include <stdlib.h>
 
 #include <new>
+
+#include "plan_internal.h"
 
 namespace {
 constexpr int MAX_SLOTS = 8;
@@ -115,7 +115,7 @@ extern "C" int b200dct_host_pipeline_submit(b200dct_host_pipeline *p, const b200
                                             unsigned long long *ticket_or_null)
 {
     if (!p || !plan || !h_in || !h_out) return B200DCT_ERR_ARG;
-    if (H <= 0 || W <= 0 || (H % 8) || (W % 8)) return B200DCT_ERR_SHAPE;
+    if (!b200dct::whole_blocks(H, W)) return B200DCT_ERR_SHAPE;
     if (in_dt != out_dt || (in_dt != B200DCT_F32 && in_dt != B200DCT_U8)) return B200DCT_ERR_ARG;
     int dev = -1;
     if (cudaGetDevice(&dev) != cudaSuccess) return B200DCT_ERR_NODEVICE;
@@ -209,7 +209,7 @@ extern "C" int b200dct_roundtrip_host(const b200dct_plan *plan, const void *h_in
 {
     tl_host_launches = 0;
     if (!plan || !h_in || !h_out) return B200DCT_ERR_ARG;
-    if (H <= 0 || W <= 0 || (H % 8) || (W % 8)) return B200DCT_ERR_SHAPE;
+    if (!b200dct::whole_blocks(H, W)) return B200DCT_ERR_SHAPE;
     if (in_dt != out_dt || (in_dt != B200DCT_F32 && in_dt != B200DCT_U8)) return B200DCT_ERR_ARG;
     int dev = -1;
     if (cudaGetDevice(&dev) != cudaSuccess) return B200DCT_ERR_NODEVICE;

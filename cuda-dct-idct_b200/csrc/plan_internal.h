@@ -18,12 +18,13 @@ struct b200dct_plan {
     bool symmetric;  // dense T whose even rows are symmetric and odd rows antisymmetric
     int tk;          // TK_HAWEEL / TK_DENSE_SYM / TK_DENSE: the kernels this plan runs
     b200dct::CommonParams cp; // device-ready tables
-    b200dct::QuantTables qc; // device-ready chrominance tables (same mask)
-    bool qc_default, qc_fastdiv;
+    b200dct::PlaneTables rgb_t[2]; // the colour kernels' tables: [0] luminance (Q), [1] chrominance (Qc), same mask
+    bool qc_fastdiv; // as q_fastdiv, for Qc
 };
 
 
 namespace b200dct {
+struct MmaParams;
 struct Span { const void *ptr; size_t pitch, row_bytes; int rows; }; // rows of row_bytes, pitch bytes apart
 // Every launch of a library kernel happens inside one of these (see "early loads" in b200dct.cu).  The scope
 // holds the launch-order lock from its decision until done() or its end, so that the per-(device, stream)
@@ -58,6 +59,9 @@ public:
         P.chain = chain_;
         P.chain_target = chain_target_;
     }
+    // kernels without the early path (any size, tensor-core arm): nothing to pass
+    void apply(AnyParams &) const {}
+    void apply(MmaParams &) const {}
     // launched: the scope's kernels are in the stream and the record describes them from now on; releases the lock
     void done(bool launched);
 private:
@@ -70,8 +74,53 @@ private:
     Span w_[3];
     bool finished_ = false;
 };
-void note_launch(int launches, const char *path); // b200dct_last_launch_count / b200dct_last_path of this thread
+// b200dct_last_launch_count / b200dct_last_path of this thread (path NULL: left as it is)
+void note_launch(int launches, const char *path = nullptr);
 bool use_factored_inverse_u8(const b200dct_plan *pl);
 bool stream_capturing(cudaStream_t s);
 bool pdl_enabled(bool capturing); // programmatic dependent launch for a launch (never on a capturing stream)
+
+// The caller's metrics workspace: {u64 macc[MACC_WORDS]; u32 pair[2]} (see MetricsCounters in b200dct.cu)
+constexpr size_t METRICS_WORKSPACE_BYTES = MACC_WORDS * sizeof(unsigned long long) + 2 * sizeof(uint32_t);
+
+// H and W positive multiples of m: whole 8 x 8 blocks, or (m = 16) whole 4:2:0 MCUs
+inline bool whole_blocks(int H, int W, int m = 8) { return H > 0 && W > 0 && !(H % m) && !(W % m); }
+
+// Grid of a kernel of 32 x 4-thread CTAs over by x bx blocks: a lane per block, a warp per 32 blocks of a block-row,
+// a CTA per 4 block-rows.  false: more than 65535 CTAs across a row (B200DCT_ERR_SHAPE).
+inline bool block_grid(int by, int bx, dim3 &grid)
+{
+    grid = dim3((unsigned)((by + 3) / 4), (unsigned)((bx + 31) / 32));
+    return grid.y <= 65535u;
+}
+
+// One launch of a kernel of hardware-scheduled 32 x 4-thread CTAs (direct family, any size, tensor-core arm, colour) in
+// the library's launch order: dependent launch unless the stream is capturing; with `early`, a part in the early path
+// (LaunchScope::DIRECT at the occupancy of the very kernel) reading rd (ptr NULL: never early) and writing w0 .. w2.  The
+// decision goes into P, and this thread's last launch is `path`.  launch(P, pdl, ctas_per_sm) launches, or with
+// ctas_per_sm != NULL only reports the kernel's resident CTAs per SM.
+// workspace: the metrics workspace the kernel counts in (NULL: none), zeroed on the stream inside the scope ahead of the
+// kernel; its contents are unknown before that, so such a launch takes no part in the early path and has no dependent launch.
+template <class Params, class Launch>
+int launch_blocks(cudaStream_t s, bool capturing, dim3 grid, Params &P, bool early, Span rd, Span w0, Span w1, Span w2,
+                  const char *path, Launch &&launch, void *workspace = nullptr)
+{
+    const bool pdl = pdl_enabled(capturing) && !workspace;
+    const bool part = early && !workspace;
+    const bool usable = part && pdl;
+    int per_sm = 0;
+    if (usable) launch(P, pdl, &per_sm);
+    LaunchScope scope(s, part ? LaunchScope::DIRECT : LaunchScope::NONE, usable, (unsigned long long)grid.x * grid.y, per_sm, rd,
+                      w0, w1, w2);
+    scope.apply(P);
+    if (workspace) {
+        const cudaError_t e = cudaMemsetAsync(workspace, 0, METRICS_WORKSPACE_BYTES, s);
+        if (e != cudaSuccess) return (int)e;
+    }
+    const cudaError_t e = launch(P, pdl, nullptr);
+    if (e != cudaSuccess) return (int)e;
+    scope.done(true);
+    note_launch(1, path);
+    return B200DCT_OK;
+}
 }

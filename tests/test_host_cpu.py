@@ -93,7 +93,112 @@ def test_argument_errors_and_no_cpu_fallback(m):
     assert L.b200dct_forward(p._h, baddr, 0, 64, baddr, 3, 128, None, 8, 16, None) == -2        # 2 blocks need 256 B
     assert L.b200dct_forward(p._h, baddr, 0, 64, baddr, 3, 264, None, 8, 16, None) == -3        # pitch not 16 B aligned
     assert L.b200dct_error_string(-4).decode().startswith("no usable CUDA device")
+    ARG, SHAPE, ALIGN, NODEV = -1, -2, -3, -4
+    a16 = baddr                       # 16-byte aligned, never dereferenced: every call below fails before device work
+    dense = m.Plan(T=np.eye(8, dtype=np.float32))
+    assert not dense.is_sparse
+    # forward / inverse / roundtrip: NULL plan before shape, H and W positive multiples of 8, pitch >= row
+    assert L.b200dct_roundtrip(None, a16, 0, 32, a16, 0, 32, None, 0, 0, 8, 12, None) == ARG
+    for H, W in ((0, 8), (8, 0), (-8, 8), (12, 8)):
+        assert L.b200dct_roundtrip(p._h, a16, 0, 32, a16, 0, 32, None, 0, 0, H, W, None) == SHAPE
+    assert L.b200dct_forward(None, a16, 0, 32, a16, 0, 32, None, 8, 4, None) == ARG
+    assert L.b200dct_forward(p._h, a16, 0, 32, a16, 0, 32, None, 4, 8, None) == SHAPE
+    assert L.b200dct_inverse(None, a16, 0, 32, a16, 0, 32, 8, 12, None) == ARG
+    assert L.b200dct_inverse(p._h, a16, 0, 32, a16, 0, 32, 8, 12, None) == SHAPE
+    assert L.b200dct_inverse(p._h, a16, 0, 16, a16, 0, 32, 8, 8, None) == SHAPE                    # pitch < row
+    # fused metrics: workspace and accumulator first, then the rules of roundtrip
+    ws = L.b200dct_metrics_workspace_bytes(8, 8)
+    assert L.b200dct_roundtrip_metrics(p._h, a16, 0, 32, a16, 0, 32, None, 0, 0, 8, 8, None, a16, ws, None) == ARG
+    assert L.b200dct_roundtrip_metrics(p._h, a16, 0, 32, a16, 0, 32, None, 0, 0, 8, 8, a16, a16, ws - 1, None) == ARG
+    assert L.b200dct_roundtrip_metrics(None, a16, 0, 32, a16, 0, 32, None, 0, 0, 8, 12, a16, a16, ws, None) == ARG
+    assert L.b200dct_roundtrip_metrics(p._h, a16, 0, 32, a16, 0, 32, None, 0, 0, 8, 12, a16, a16, ws, None) == SHAPE
+    # any size: non-positive sides are ARG, pitch < row SHAPE, element misalignment ALIGN
+    assert L.b200dct_roundtrip_any(p._h, a16, 0, 28, a16, 28, 0, 7, None) == ARG
+    assert L.b200dct_roundtrip_any(p._h, a16, 0, 24, a16, 28, 5, 7, None) == SHAPE
+    assert L.b200dct_roundtrip_any(p._h, a16 + 2, 0, 28, a16, 28, 5, 7, None) == ALIGN
+    assert L.b200dct_roundtrip_any(p._h, a16 + 2, 0, 24, a16, 28, 5, 7, None) == SHAPE           # pitch before alignment
+    assert L.b200dct_roundtrip_any(p._h, a16, 2, 28, a16, 28, 5, 7, None) == ARG                 # i16 pixels
+    # batch: arguments, then shape, then every image's planes; no images and valid arguments: nothing to do
+    imgs = (C.c_void_p * 2)(a16, a16)
+    assert L.b200dct_roundtrip_batch(None, 2, imgs, imgs, 0, 32, 32, 8, 12, None) == ARG
+    assert L.b200dct_roundtrip_batch(p._h, 2, imgs, imgs, 2, 32, 32, 8, 12, None) == ARG          # i16 pixels
+    assert L.b200dct_roundtrip_batch(p._h, 2, imgs, imgs, 0, 32, 32, 8, 12, None) == SHAPE
+    assert L.b200dct_roundtrip_batch(p._h, 0, None, None, 0, 32, 32, 12, 8, None) == SHAPE
+    assert L.b200dct_roundtrip_batch(p._h, 2, imgs, imgs, 0, 16, 32, 8, 8, None) == SHAPE          # pitch < row
+    assert L.b200dct_roundtrip_batch(p._h, 2, imgs, imgs, 0, 40, 32, 8, 8, None) == ALIGN
+    assert L.b200dct_roundtrip_batch(p._h, 0, None, None, 0, 32, 32, 8, 8, None) == 0
+    # colour 4:4:4: NULL, shape, pitch, 8-byte RGB alignment, Haweel's T, stream alignment -- in this order
+    zzb = 128
+    for rc, args in ((ARG, (p._h, None, 24, a16, 24, None, 0, 8, 8)), (SHAPE, (p._h, a16, 24, a16, 24, None, 0, 8, 12)),
+                     (SHAPE, (p._h, a16, 16, a16, 24, None, 0, 8, 8)), (ALIGN, (p._h, a16 + 4, 24, a16, 24, None, 0, 8, 8)),
+                     (ALIGN, (p._h, a16, 28, a16, 24, None, 0, 8, 8)), (ARG, (dense._h, a16, 24, a16, 24, None, 0, 8, 8)),
+                     (ALIGN, (p._h, a16, 24, a16, 24, a16 + 8, zzb, 8, 8)), (ALIGN, (p._h, a16, 24, a16, 24, a16, zzb - 16, 8, 8)),
+                     (SHAPE, (dense._h, a16, 24, a16, 24, None, 0, 8, 12)), (ALIGN, (dense._h, a16 + 4, 24, a16, 24, None, 0, 8, 8)),
+                     (ARG, (dense._h, a16, 24, a16, 24, a16 + 8, zzb, 8, 8))):
+        assert L.b200dct_roundtrip_rgb(*args, None) == rc, (rc, args)
+    assert L.b200dct_forward_rgb(p._h, a16, 24, None, zzb, 8, 8, None) == ARG
+    assert L.b200dct_forward_rgb(p._h, a16, 24, a16, zzb, 12, 8, None) == SHAPE
+    assert L.b200dct_forward_rgb(p._h, a16 + 4, 24, a16, zzb, 8, 8, None) == ALIGN
+    assert L.b200dct_forward_rgb(dense._h, a16, 24, a16, zzb, 8, 8, None) == ARG
+    assert L.b200dct_forward_rgb(p._h, a16, 24, a16 + 8, zzb, 8, 8, None) == ALIGN
+    assert L.b200dct_forward_rgb(dense._h, a16, 24, a16 + 8, zzb, 8, 12, None) == SHAPE
+    assert L.b200dct_inverse_rgb(p._h, None, zzb, a16, 24, 8, 8, None) == ARG
+    assert L.b200dct_inverse_rgb(p._h, a16, zzb, a16, 16, 8, 8, None) == SHAPE
+    assert L.b200dct_inverse_rgb(p._h, a16, zzb, a16, 28, 8, 8, None) == ALIGN
+    assert L.b200dct_inverse_rgb(dense._h, a16, zzb, a16, 24, 8, 8, None) == ARG
+    assert L.b200dct_inverse_rgb(p._h, a16, zzb + 8, a16, 24, 8, 8, None) == ALIGN
+    # colour 4:2:0: sides multiples of 16, pitch, RGB and stream alignment, Haweel's T, then the grid (before the device)
+    wide = (1 << 24) + 16                                                                         # 65537 CTAs across
+    assert L.b200dct_forward_rgb420(p._h, a16, 48, a16, None, a16, 16, 16, None) == ARG
+    assert L.b200dct_forward_rgb420(p._h, a16, 48, a16, a16, a16, 24, 16, None) == SHAPE
+    assert L.b200dct_forward_rgb420(p._h, a16, 40, a16, a16, a16, 16, 16, None) == SHAPE
+    assert L.b200dct_forward_rgb420(p._h, a16, 52, a16, a16, a16, 16, 16, None) == ALIGN
+    assert L.b200dct_forward_rgb420(p._h, a16, 48, a16, a16 + 8, a16, 16, 16, None) == ALIGN
+    assert L.b200dct_forward_rgb420(dense._h, a16, 48, a16, a16, a16, 16, 16, None) == ARG
+    assert L.b200dct_forward_rgb420(p._h, a16, 3 * wide, a16, a16, a16, 16, wide, None) == SHAPE
+    assert L.b200dct_forward_rgb420(dense._h, a16, 3 * wide, a16, a16, a16, 16, wide, None) == ARG
+    assert L.b200dct_forward_rgb420(dense._h, a16, 48, a16, a16, a16 + 8, 16, 24, None) == SHAPE
+    assert L.b200dct_inverse_rgb420(p._h, a16, a16, a16, None, 48, 16, 16, None) == ARG
+    assert L.b200dct_inverse_rgb420(p._h, a16, a16, a16, a16, 48, 16, 8, None) == SHAPE
+    assert L.b200dct_inverse_rgb420(p._h, a16, a16, a16 + 8, a16, 48, 16, 16, None) == ALIGN
+    assert L.b200dct_inverse_rgb420(dense._h, a16, a16, a16, a16, 48, 16, 16, None) == ARG
+    assert L.b200dct_inverse_rgb420(p._h, a16, a16, a16, a16, 3 * wide, 16, wide, None) == SHAPE
+    # coded size: arguments, shape and pitch, alignment
+    assert L.b200dct_zigzag_coded_bits(a16, 128, 8, 8, 2, a16, None) == ARG
+    assert L.b200dct_zigzag_coded_bits(None, 128, 8, 12, 0, a16, None) == ARG
+    assert L.b200dct_zigzag_coded_bits(a16, 128, 8, 12, 0, a16, None) == SHAPE
+    assert L.b200dct_zigzag_coded_bits(a16, 128, 0, 8, 0, a16, None) == SHAPE
+    assert L.b200dct_zigzag_coded_bits(a16, 112, 8, 8, 0, a16, None) == SHAPE
+    assert L.b200dct_zigzag_coded_bits(a16, 136, 8, 8, 0, a16, None) == ALIGN
+    assert L.b200dct_zigzag_coded_bits(a16 + 8, 128, 8, 12, 0, a16, None) == SHAPE
+    # host pipeline: arguments, shape, pixel dtypes
+    assert L.b200dct_roundtrip_host(None, a16, 0, a16, 0, 8, 12) == ARG
+    assert L.b200dct_roundtrip_host(p._h, a16, 0, a16, 0, 8, 12) == SHAPE
+    assert L.b200dct_roundtrip_host(p._h, a16, 0, a16, 0, -8, 8) == SHAPE
+    assert L.b200dct_roundtrip_host(p._h, a16, 0, a16, 1, 8, 8) == ARG
+    assert L.b200dct_roundtrip_host(p._h, a16, 0, a16, 1, 8, 12) == SHAPE
+    assert L.b200dct_host_pipeline_submit(None, p._h, a16, 0, a16, 0, 8, 12, None) == ARG
     if not torch.cuda.is_available():
+        # valid calls reach the device check on every entry point
+        assert L.b200dct_forward(p._h, a16, 0, 32, a16, 0, 32, None, 8, 8, None) == NODEV
+        assert L.b200dct_inverse(p._h, a16, 0, 32, a16, 0, 32, 8, 8, None) == NODEV
+        assert L.b200dct_roundtrip(p._h, a16, 0, 32, a16, 0, 32, None, 0, 0, 8, 8, None) == NODEV
+        assert L.b200dct_roundtrip_metrics(p._h, a16, 0, 32, a16, 0, 32, None, 0, 0, 8, 8, a16, a16, ws, None) == NODEV
+        assert L.b200dct_roundtrip_any(p._h, a16, 0, 28, a16, 28, 5, 7, None) == NODEV
+        assert L.b200dct_roundtrip_any(p._h, a16, 0, 32, a16, 32, 8, 8, None) == NODEV
+        assert L.b200dct_roundtrip_batch(p._h, 2, imgs, imgs, 0, 32, 32, 8, 8, None) == NODEV
+        assert L.b200dct_roundtrip_rgb(p._h, a16, 24, a16, 24, None, 0, 8, 8, None) == NODEV
+        assert L.b200dct_roundtrip_rgb(p._h, a16, 24, a16, 24, a16, zzb, 8, 8, None) == NODEV
+        assert L.b200dct_forward_rgb(p._h, a16, 24, a16, zzb, 8, 8, None) == NODEV
+        assert L.b200dct_inverse_rgb(p._h, a16, zzb, a16, 24, 8, 8, None) == NODEV
+        assert L.b200dct_forward_rgb420(p._h, a16, 48, a16, a16, a16, 16, 16, None) == NODEV
+        assert L.b200dct_inverse_rgb420(p._h, a16, a16, a16, a16, 48, 16, 16, None) == NODEV
+        assert L.b200dct_zigzag_coded_bits(a16, 128, 8, 8, 0, a16, None) == NODEV
+        assert L.b200dct_roundtrip_host(p._h, a16, 0, a16, 0, 8, 8) == NODEV
+        # the grid rule comes after the device check everywhere but 4:2:0
+        assert L.b200dct_roundtrip(p._h, a16, 0, 4 * wide, a16, 0, 4 * wide, None, 0, 0, 8, wide, None) == NODEV
+        assert L.b200dct_roundtrip_rgb(p._h, a16, 3 * wide, a16, 3 * wide, None, 0, 8, wide, None) == NODEV
+
         # valid arguments, no device: the product path refuses -- it never computes on the CPU
         a = np.zeros((8, 8), np.float32)
         b = np.zeros((8, 8), np.float32)
