@@ -18,18 +18,17 @@
 #include "mma_kernels.cuh"
 
 namespace b200dct {
-// one launcher per family and translation unit of kernel instantiations (inst_<family>_<s|d|y><quantiser>.cu);
-// ctas_per_sm != NULL: no launch, only the resident-CTA count of the kernel the arguments select
+// one launcher per family and translation unit of kernel instantiations (inst_<family>_<s|d|y><quantiser>.cu, and
+// inst_<family>_k.cu for the compile-time masks Q_IMM_K6..K10); ctas_per_sm != NULL: no launch, only the resident-CTA
+// count of the kernel the arguments select
 #define B200_DECL(tag)                                                                                                  \
-    cudaError_t launch_direct_##tag(int mode, int pix, bool finv, bool metrics, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm); \
-    cudaError_t launch_tma_##tag(int mode, int pix, bool finv, const TmaParams &P, int grid, int block, size_t smem, cudaStream_t s, bool pdl);
-B200_DECL(s0) B200_DECL(s1) B200_DECL(s2) B200_DECL(d1) B200_DECL(d2) B200_DECL(y1) B200_DECL(y2)
+    cudaError_t launch_direct_##tag(int qm, int mode, int pix, bool finv, bool metrics, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm); \
+    cudaError_t launch_tma_##tag(int qm, int mode, int pix, bool finv, bool metrics, const TmaParams &P, int grid, int block, size_t smem, cudaStream_t s, bool pdl);
+B200_DECL(s0) B200_DECL(s1) B200_DECL(s2) B200_DECL(d1) B200_DECL(d2) B200_DECL(y1) B200_DECL(y2) B200_DECL(k)
 #undef B200_DECL
-cudaError_t launch_direct_kmask(int k, int pix, const DirectParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm); // inst_direct_k.cu
 cudaError_t launch_any_f32(int tk, int qm, bool finv, const AnyParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl); // inst_any_f32.cu
 cudaError_t launch_any_u8(int tk, int qm, bool finv, const AnyParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl);  // inst_any_u8.cu
 cudaError_t launch_mma(bool fastdiv, const MmaParams &P, dim3 grid, dim3 block, cudaStream_t s, bool pdl);                           // inst_mma.cu
-cudaError_t launch_tma_kmask(int k, int pix, const TmaParams &P, int grid, int block, size_t smem, cudaStream_t s, bool pdl);          // inst_tma_k.cu
 
 struct Unit {
     decltype(&launch_direct_s0) direct;
@@ -39,6 +38,7 @@ struct Unit {
 static Unit unit_of(int tk, int q)
 {
 #define B200_UNIT(tag) Unit{launch_direct_##tag, launch_tma_##tag}
+    if (is_kmask(q)) return B200_UNIT(k);
     if (tk == TK_DENSE_SYM) return q == 1 ? B200_UNIT(y1) : B200_UNIT(y2);
     if (tk == TK_HAWEEL) return q == 0 ? B200_UNIT(s0) : q == 1 ? B200_UNIT(s1) : B200_UNIT(s2);
     return q == 1 ? B200_UNIT(d1) : B200_UNIT(d2);
@@ -590,11 +590,10 @@ static bool prefers_tma(const b200dct_plan *pl, size_t bytes_per_px, int H, int 
            (bytes_per_px >= 4 && pl->tk == TK_DENSE_SYM && px >= TMA_HUGE_PIXELS);
 }
 
-// The kernel variant a plan runs for (mode, pixel dtype): quantiser, compile-time retained-coefficient mask (kmask
-// = k of the first k zig-zag coefficients, 0: none) and the factored inverse.  runtime_mask: the kernels take the
-// mask as data only (metrics, any size).
+// The kernel variant a plan runs for (mode, pixel dtype): quantiser and the factored inverse.  runtime_mask: the
+// kernels take the mask as data only (metrics, any size).
 struct Variant {
-    int qm, kmask;
+    int qm;
     bool finv;
 };
 static Variant variant_of(const b200dct_plan *pl, int mode, int pix, bool runtime_mask)
@@ -605,25 +604,11 @@ static Variant variant_of(const b200dct_plan *pl, int mode, int pix, bool runtim
     else v.qm = Q_PARAM;
     // retained-coefficient round trips (first k = 6..10 zig-zag coefficients of the default
     // tables): kernels with the mask as a compile-time constant
-    v.kmask = 0;
     if (mode == MODE_RT && !runtime_mask && pl->sparse && pl->q_default && pl->q_fastdiv)
         for (int k = 6; k <= 10; k++)
-            if (pl->mask == b200dct_zigzag_mask(k)) v.kmask = k;
-    v.finv = !v.kmask && use_factored_inverse(pl, mode, pix); // compile-time-mask kernels keep the chains
+            if (pl->mask == b200dct_zigzag_mask(k)) v.qm = Q_IMM_K6 + (k - 6);
+    v.finv = !is_kmask(v.qm) && use_factored_inverse(pl, mode, pix); // compile-time-mask kernels keep the chains
     return v;
-}
-// ctas_per_sm != NULL: no launch, only the resident-CTA count of the kernel the arguments select
-static cudaError_t launch_direct(int tk, const Variant &v, int mode, int pix, bool metrics, const DirectParams &P, dim3 grid,
-                                 dim3 block, cudaStream_t s, bool pdl, int *ctas_per_sm = nullptr)
-{
-    if (v.kmask) return launch_direct_kmask(v.kmask, pix, P, grid, block, s, pdl, ctas_per_sm);
-    return unit_of(tk, v.qm).direct(mode, pix, v.finv, metrics, P, grid, block, s, pdl, ctas_per_sm);
-}
-static cudaError_t launch_tma(int tk, const Variant &v, int mode, int pix, const TmaParams &P, int grid, int block, size_t smem,
-                              cudaStream_t s, bool pdl)
-{
-    if (v.kmask) return launch_tma_kmask(v.kmask, pix, P, grid, block, smem, s, pdl);
-    return unit_of(tk, v.qm).tma(mode, pix, v.finv, P, grid, block, smem, s, pdl);
 }
 // the bytes of one plane of a call (the zig-zag stream: H/8 rows of W/8 blocks of 128 bytes)
 static Span plane_span(const Plane &p, int H, int W)
@@ -718,7 +703,8 @@ static int run_tma(const Call &c, const DevInfo &di, uint32_t *capture_sched)
     scope.apply(P);
     const cudaError_t em = mc.zero(c.stream);
     if (em != cudaSuccess) return (int)em;
-    const cudaError_t e = launch_tma(c.pl->tk, c.v, c.mode, c.pix, P, grid, nw * 32, smem, c.stream, pdl && !mc.in_workspace);
+    const cudaError_t e = unit_of(c.pl->tk, c.v.qm).tma(c.v.qm, c.mode, c.pix, c.v.finv, c.workspace != nullptr, P, grid, nw * 32, smem,
+                                                        c.stream, pdl && !mc.in_workspace);
     if (e != cudaSuccess) return (int)e;
     scope.done(true);
     note_launch(1, "tma");
@@ -760,7 +746,7 @@ static int run_direct(const Call &c)
     const Span w2 = metrics ? Span{c.acc, 0, 3 * sizeof(double), 1} : Span{c.shifted, c.in.pitch, (size_t)c.W * 4, c.H};
     return launch_blocks(c.stream, c.capturing, grid, P, true, may_load_early ? c.rd : Span{}, c.w0, c.w1, w2, "direct",
                          [&](const DirectParams &Q, bool pdl, int *per_sm) {
-                             return launch_direct(c.pl->tk, c.v, c.mode, c.pix, metrics, Q, grid, dim3(32, 4), c.stream, pdl, per_sm);
+                             return unit_of(c.pl->tk, c.v.qm).direct(c.v.qm, c.mode, c.pix, c.v.finv, metrics, Q, grid, dim3(32, 4), c.stream, pdl, per_sm);
                          },
                          mc.in_workspace ? mc.macc : nullptr);
 }
@@ -909,7 +895,7 @@ extern "C" int b200dct_roundtrip_batch(const b200dct_plan *plan, int n_images, c
         }
         P.in = P.img_in[0]; P.out = P.img_out[0];
         grid.z = (unsigned)n;
-        const cudaError_t e = launch_direct(plan->tk, v, MODE_RT, (int)dt, false, P, grid, dim3(32, 4), s, pdl);
+        const cudaError_t e = unit_of(plan->tk, v.qm).direct(v.qm, MODE_RT, (int)dt, v.finv, false, P, grid, dim3(32, 4), s, pdl, nullptr);
         if (e != cudaSuccess) return (int)e;
         launches++;
     }

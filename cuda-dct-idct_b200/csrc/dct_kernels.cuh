@@ -33,6 +33,54 @@ enum { DT_F32 = 0, DT_U8 = 1, DT_I16 = 2, DT_I16ZZ = 3, DT_NONE = -1 };
 // 3..7 = JPEG immediates with the first 6..10 zig-zag coefficients retained, the mask a
 // compile-time constant (README.md:63 of the reference): fused round trips only
 enum { Q_IMM = 0, Q_PARAM = 1, Q_PARAM_DIV = 2, Q_IMM_K6 = 3, Q_IMM_K7 = 4, Q_IMM_K8 = 5, Q_IMM_K9 = 6, Q_IMM_K10 = 7 };
+__host__ __device__ constexpr bool is_kmask(int qm) { return qm >= Q_IMM_K6 && qm <= Q_IMM_K10; }
+
+// Which kernels exist: the instantiation units (inst_*.cuh) compile exactly the (T family, quantiser, mode, pixel
+// type, factored inverse, fused metrics) their family's rule allows, and return cudaErrorInvalidValue for the rest.
+//   - JPEG immediates (Q_IMM, the compile-time masks) come with Haweel's T only;
+//   - the factored inverse: Haweel's T, 8-bit pixels, a mode that is not forward-only;
+//   - fused metrics: round trips; on the TMA family only f32 round trips of Haweel's T;
+//   - compile-time masks: fused round trips of Haweel's T, with no factored inverse and no metrics;
+//   - the any-size kernels: fused round trips without metrics, runtime masks only.
+constexpr bool direct_compiled(int tk, int qm, int mode, int pix, bool finv, bool metrics)
+{
+    return (tk == TK_HAWEEL || (qm != Q_IMM && !is_kmask(qm))) && (!finv || (tk == TK_HAWEEL && pix == DT_U8 && mode != MODE_FWD)) &&
+           (!metrics || mode == MODE_RT) && (!is_kmask(qm) || (mode == MODE_RT && !finv && !metrics));
+}
+constexpr bool tma_compiled(int tk, int qm, int mode, int pix, bool finv, bool metrics)
+{
+    return direct_compiled(tk, qm, mode, pix, finv, metrics) && (!metrics || (tk == TK_HAWEEL && pix == DT_F32));
+}
+constexpr bool any_compiled(int tk, int qm, int mode, int pix, bool finv, bool metrics)
+{
+    return direct_compiled(tk, qm, mode, pix, finv, metrics) && mode == MODE_RT && !metrics && !is_kmask(qm);
+}
+
+// Calls f(std::integral_constant<..., V>{}) for the V of the list that equals v: a runtime value becomes a template
+// argument.  No match: cudaErrorInvalidValue.
+template <auto... V, class F>
+cudaError_t pick(int v, F &&f)
+{
+    cudaError_t e = cudaErrorInvalidValue;
+    (void)((v == (int)V && (e = f(std::integral_constant<decltype(V), V>{}), true)) || ...);
+    return e;
+}
+// f(Q, MODE, PIX, FINV, METRICS) for one launch request of a unit with the quantisers QS (inst_direct.cuh, inst_tma.cuh)
+template <int... QS, class F>
+cudaError_t pick_kernel(int qm, int mode, int pix, bool finv, bool metrics, F &&f)
+{
+    return pick<QS...>(qm, [&](auto q) {
+        return pick<MODE_FWD, MODE_INV, MODE_RT>(mode, [&](auto m) {
+            return pick<DT_F32, DT_U8>(pix, [&](auto x) {
+                return pick<false, true>(finv, [&](auto fi) {
+                    return pick<false, true>(metrics, [&](auto me) { return f(q, m, x, fi, me); });
+                });
+            });
+        });
+    });
+}
+#define B200_CAT_(a, b) a##b
+#define B200_CAT(a, b) B200_CAT_(a, b)
 
 struct CommonParams {
     QuantTables q;
@@ -46,7 +94,7 @@ struct QSel { // Q_IMM and Q_IMM_K6..K10
 };
 template <int QMODE>
 struct KeepOf {
-    using type = KeepMask<(QMODE >= Q_IMM_K6 && QMODE <= Q_IMM_K10) ? zigzag_prefix_mask(QMODE - Q_IMM_K6 + 6) : ~0ull>;
+    using type = KeepMask<is_kmask(QMODE) ? zigzag_prefix_mask(QMODE - Q_IMM_K6 + 6) : ~0ull>;
 };
 template <>
 struct QSel<Q_PARAM> {

@@ -1,4 +1,4 @@
-#define INST_SPARSE 0
-#define INST_Q 1
+#define INST_TK TK_DENSE
+#define INST_Q Q_PARAM
 #define INST_TAG d1
 #include "inst_direct.cuh"

@@ -1,4 +1,4 @@
-#define INST_SPARSE 0
-#define INST_Q 2
+#define INST_TK TK_DENSE
+#define INST_Q Q_PARAM_DIV
 #define INST_TAG d2
 #include "inst_direct.cuh"

@@ -1,4 +1,4 @@
-#define INST_SPARSE 1
-#define INST_Q 0
+#define INST_TK TK_HAWEEL
+#define INST_Q Q_IMM
 #define INST_TAG s0
 #include "inst_tma.cuh"
