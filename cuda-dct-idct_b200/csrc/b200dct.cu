@@ -414,36 +414,50 @@ MetricsCounters metrics_counters(uint32_t *slot, void *workspace)
 //     having passed its own wait: everything older than the predecessor is complete by the time a
 //     successor CTA runs, and only the predecessor's writes matter;
 //   * so: predecessor on this stream = such a launch, and [input plane] disjoint from its output /
-//     coefficient planes  =>  early_loads.  Launches that do not qualify as predecessors clear the record.
+//     coefficient planes  =>  early tile loads.  Launches that do not qualify as predecessors clear the record.
 // Every launch of the library, taking part or not, happens inside a LaunchScope (plan_internal.h), which holds
 // g_last_mu across the decision, the launch and the update of the record.
 // Not under stream capture.  env B200DCT_EARLY_LOADS=0 disables (A/B).
-namespace {
+//
+// The direct family (hardware-scheduled 128-thread CTAs, several per SM) has its own version of the argument:
+// a dependent launch starts once every CTA of its predecessor has STARTED (executed launch_dependents).
+// If the predecessor has more CTAs than the machine can hold at once (grid > resident CTAs per SM x SMs,
+// the occupancy of that very kernel), "all started" implies "some exited", and a CTA only exits after its
+// griddepcontrol.wait -- so again everything older than the predecessor is complete when a successor CTA
+// runs, and only the predecessor's own writes matter.  A direct-family round trip whose input is disjoint
+// from them loads AND transforms its blocks before its wait (L2-coherent loads) and only holds back its
+// stores: its CTAs work in the slots the predecessor's last wave leaves idle instead of sitting at the wait
+// (8192^2 u8: 11 waves of ~5 us, on average half a wave idle per launch boundary).  CTAs beyond one
+// machine-full start after the predecessor anyway.
+//
+// Both arguments are about the library's own kernels; what the CALLER enqueues between two calls is
+// invisible to the host side.  A kernel of the caller that writes the next call's input is covered on
+// the device: every machine-filling launch feeds a per-(device, stream) completion counter, the host knows
+// the value the counter has once the predecessor is complete, and a successor only takes the early path
+// when it READS a smaller value -- the predecessor is then provably still running, so nothing enqueued
+// after it (which, launched the ordinary way, starts only when the predecessor has completed) can stand
+// between the two; otherwise the successor waits first like any dependent launch.  (Not covered: foreign
+// kernels themselves launched with programmatic stream serialization between two calls of the library.)
+// The device side of the protocol is EarlyPath (dct_kernels.cuh).
+namespace b200dct {
 struct Range {
     uintptr_t lo = 0, hi = 0; // [lo, hi)
 };
 struct LastLaunch {
     int dev = -1;
     cudaStream_t stream = nullptr;
-    bool tma = false;     // persistent TMA-family launch that fills the machine (see above)
-    bool direct = false;  // direct-family launch with more CTAs than the machine holds at once (see below)
+    LaunchScope::Family family = LaunchScope::NONE; // of a machine-filling launch that fed the counter, else NONE
     Range w[3];
     bool chain_ok = true; // false once the record has been taken over by another stream (its counter may still be fed)
     unsigned long long expected = 0; // value of the record's completion counter once every recorded launch has completed
 };
+} // namespace b200dct
+namespace {
 constexpr int LAST_SLOTS = 16;
 LastLaunch g_last[LAST_SLOTS];
 unsigned long long *g_chain[64] = {}; // per device: one completion counter per record
 std::mutex g_last_mu;
-Range plane_range(const Span &sp)
-{
-    Range r;
-    if (sp.ptr) {
-        r.lo = (uintptr_t)sp.ptr;
-        r.hi = r.lo + (size_t)(sp.rows - 1) * sp.pitch + sp.row_bytes;
-    }
-    return r;
-}
+Range plane_range(const Span &sp) { return sp.ptr ? Range{(uintptr_t)sp.ptr, sp.end()} : Range{}; }
 bool disjoint(const Range &a, const Range &b) { return a.hi <= b.lo || b.hi <= a.lo || a.lo == a.hi || b.lo == b.hi; }
 bool early_loads_enabled()
 {
@@ -453,74 +467,10 @@ bool early_loads_enabled()
     }();
     return v;
 }
-// The direct family (hardware-scheduled 128-thread CTAs, several per SM) has its own version of the argument:
-// a dependent launch starts once every CTA of its predecessor has STARTED (executed launch_dependents).
-// If the predecessor has more CTAs than the machine can hold at once (grid > resident CTAs per SM x SMs,
-// the occupancy of that very kernel), "all started" implies "some exited", and a CTA only exits after its
-// griddepcontrol.wait -- so again everything older than the predecessor is complete when a successor CTA
-// runs, and only the predecessor's own writes matter.  A direct-family round trip whose input is disjoint
-// from them loads AND transforms its blocks before its wait (L2-coherent loads) and only holds back its
-// stores: its CTAs work in the slots the predecessor's last wave leaves idle instead of sitting at the wait
-// (8192^2 u8: 11 waves of ~5 us, on average half a wave idle per launch boundary).
-//
-// Both arguments are about the library's own kernels; what the CALLER enqueues between two calls is
-// invisible to the host side.  A kernel of the caller that writes the next call's input is covered on
-// the device: every machine-filling launch feeds a per-(device, stream) completion counter (direct
-// family: one increment per CTA at its end; TMA family: one by the last warp out), the host knows the
-// value the counter has once the predecessor is complete, and a successor only takes the early path
-// when it READS a smaller value -- the predecessor is then provably still running, so nothing enqueued
-// after it (which, launched the ordinary way, starts only when the predecessor has completed) can stand
-// between the two; otherwise the successor waits first like any dependent launch.  (Not covered: foreign
-// kernels themselves launched with programmatic stream serialization between two calls of the library.)
-struct LaunchTicket {
-    LastLaunch *rec = nullptr;
-    bool early = false;                  // this launch may take the early path (subject to the device-side check)
-    unsigned long long *chain = nullptr; // the record's completion counter (NULL: none, no early path around this launch)
-    unsigned long long target = 0;       // its value once the predecessor is complete
-};
-// Before the launch: may a launch of family `tma` / direct reading `rd` on `stream` load early?  (fills: it
-// satisfies its family's machine-filling condition.)  Leaves the record cleared; LaunchScope::done fills it in
-// once the kernel is in the stream.  The caller holds g_last_mu from here until then.
-LaunchTicket begin_launch_locked(cudaStream_t stream, bool tma, bool fills, bool may_allocate, const Range &rd)
-{
-    LaunchTicket t;
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return t;
-    LastLaunch *e = nullptr, *freeslot = nullptr;
-    for (auto &x : g_last) {
-        if (x.dev == dev && x.stream == stream) e = &x;
-        if (x.dev < 0 && !freeslot) freeslot = &x;
-    }
-    const bool known = e != nullptr;
-    if (!e) {
-        if (freeslot) e = freeslot;
-        else { // evicting a record is always safe: no early path on it any more
-            e = &g_last[((uintptr_t)stream >> 4) % LAST_SLOTS];
-            e->chain_ok = false;
-        }
-        e->expected = 0; // a fresh record's counter has never been fed; an evicted one has no counter any more
-        e->dev = dev;
-        e->stream = stream;
-        e->tma = e->direct = false;
-    }
-    if (e->chain_ok && !g_chain[dev] && may_allocate) {
-        unsigned long long *p = nullptr;
-        if (cudaMalloc(&p, LAST_SLOTS * sizeof(unsigned long long)) == cudaSuccess) {
-            if (cudaMemset(p, 0, LAST_SLOTS * sizeof(unsigned long long)) == cudaSuccess) g_chain[dev] = p;
-            else cudaFree(p);
-        }
-    }
-    t.rec = e;
-    t.chain = (e->chain_ok && g_chain[dev]) ? g_chain[dev] + (e - g_last) : nullptr;
-    t.target = e->expected;
-    // (TMA family: the successor must not fit beside the predecessor either, i.e. satisfy the condition itself)
-    t.early = known && t.chain && (tma ? (fills && e->tma) : e->direct) && rd.lo != rd.hi && disjoint(rd, e->w[0]) &&
-              disjoint(rd, e->w[1]) && disjoint(rd, e->w[2]) && early_loads_enabled();
-    e->tma = e->direct = false; // until committed
-    return t;
-}
 } // namespace
 namespace b200dct {
+// Before the launch: may a launch of `family` reading `rd` on `s` take the early path, and does it feed the counter?
+// Leaves the record cleared; done() fills it in once the kernel is in the stream.
 LaunchScope::LaunchScope(cudaStream_t s, Family family, bool usable, unsigned long long ctas, int ctas_per_sm, Span rd, Span w0,
                          Span w1, Span w2)
     : family_(family), w_{w0, w1, w2}
@@ -531,26 +481,54 @@ LaunchScope::LaunchScope(cudaStream_t s, Family family, bool usable, unsigned lo
     const unsigned long long machine = (unsigned long long)(ctas_per_sm > 0 ? ctas_per_sm : 0) * (unsigned long long)di.sms;
     // direct style: more CTAs than the machine holds at once; TMA: a CTA on every SM
     const bool fills = usable && machine > 0 && (family == TMA ? ctas >= machine : ctas > machine);
-    const LaunchTicket t = begin_launch_locked(s, family == TMA, fills, usable, usable ? plane_range(rd) : Range{});
-    const bool feeds = fills && t.chain != nullptr;
-    rec_ = t.rec;
-    // direct style: CTAs beyond one machine-full start after the predecessor anyway, and the last CTAs of the grid
-    // feed the counter
-    early_ = t.early ? (family == TMA ? 1 : (int)(ctas < machine ? ctas : machine)) : 0;
-    chain_feed_ = feeds ? (family == TMA ? 1 : (int)(ctas < 1024 ? ctas : 1024)) : 0;
-    chain_ = (feeds || t.early) ? t.chain : nullptr;
-    chain_target_ = t.target;
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return;
+    LastLaunch *e = nullptr, *freeslot = nullptr;
+    for (auto &x : g_last) {
+        if (x.dev == dev && x.stream == s) e = &x;
+        if (x.dev < 0 && !freeslot) freeslot = &x;
+    }
+    const bool known = e != nullptr;
+    if (!e) {
+        if (freeslot) e = freeslot;
+        else { // evicting a record is always safe: no early path on it any more
+            e = &g_last[((uintptr_t)s >> 4) % LAST_SLOTS];
+            e->chain_ok = false;
+        }
+        e->expected = 0; // a fresh record's counter has never been fed; an evicted one has no counter any more
+        e->dev = dev;
+        e->stream = s;
+        e->family = NONE;
+    }
+    if (e->chain_ok && !g_chain[dev] && usable) {
+        unsigned long long *p = nullptr;
+        if (cudaMalloc(&p, LAST_SLOTS * sizeof(unsigned long long)) == cudaSuccess) {
+            if (cudaMemset(p, 0, LAST_SLOTS * sizeof(unsigned long long)) == cudaSuccess) g_chain[dev] = p;
+            else cudaFree(p);
+        }
+    }
+    rec_ = e;
+    unsigned long long *const chain = (e->chain_ok && g_chain[dev]) ? g_chain[dev] + (e - g_last) : nullptr;
+    const Range r = usable ? plane_range(rd) : Range{};
+    // (TMA family: the successor must not fit beside the predecessor either, i.e. satisfy the condition itself)
+    const bool early = known && chain && family != NONE && e->family == family && (family == DIRECT || fills) && r.lo != r.hi &&
+                       disjoint(r, e->w[0]) && disjoint(r, e->w[1]) && disjoint(r, e->w[2]) && early_loads_enabled();
+    const bool feeds = fills && chain != nullptr;
+    e->family = NONE; // until committed
+    // the first machine-full of the grid (TMA: the whole grid); the last CTAs of the grid feed (TMA: its last warp out)
+    ep_.early = early ? (int)(ctas < machine ? ctas : machine) : 0;
+    ep_.chain_feed = feeds ? (family == TMA ? 1 : (int)(ctas < 1024 ? ctas : 1024)) : 0;
+    ep_.chain = (feeds || early) ? chain : nullptr;
+    ep_.chain_target = e->expected;
 }
 void LaunchScope::done(bool launched)
 {
     if (finished_) return;
     finished_ = true;
-    LastLaunch *r = static_cast<LastLaunch *>(rec_);
-    if (launched && r) { // this launch as the next one's predecessor
-        r->tma = family_ == TMA && chain_feed_ > 0;
-        r->direct = family_ == DIRECT && chain_feed_ > 0;
-        for (int i = 0; i < 3; i++) r->w[i] = plane_range(w_[i]);
-        r->expected += (unsigned long long)chain_feed_;
+    if (launched && rec_) { // this launch as the next one's predecessor
+        rec_->family = ep_.chain_feed > 0 ? family_ : NONE;
+        for (int i = 0; i < 3; i++) rec_->w[i] = plane_range(w_[i]);
+        rec_->expected += (unsigned long long)ep_.chain_feed;
     }
     g_last_mu.unlock();
 }
@@ -643,8 +621,8 @@ static int run_mma(const Call &c)
     M.cp = c.pl->cp;
     dim3 grid;
     if (!block_grid(M.by, M.bx, grid)) return B200DCT_ERR_SHAPE;
-    return launch_blocks(c.stream, c.capturing, grid, M, false, Span{}, Span{}, Span{}, Span{}, "mma",
-                         [&](const MmaParams &P, bool pdl, int *) { return launch_mma(c.pl->q_fastdiv, P, grid, dim3(32, 4), c.stream, pdl); });
+    return launch_blocks(c.stream, c.capturing, grid, false, Span{}, Span{}, Span{}, Span{}, "mma",
+                         [&](const EarlyPath &, bool pdl, int *) { return launch_mma(c.pl->q_fastdiv, M, grid, dim3(32, 4), c.stream, pdl); });
 }
 
 // the persistent TMA family; capture_sched: the ticket-counter pair of a captured launch (NULL: none left, or not capturing)
@@ -700,7 +678,7 @@ static int run_tma(const Call &c, const DevInfo &di, uint32_t *capture_sched)
     const bool heavy = smem > (size_t)(di.smem_optin / 2) + 1024;
     LaunchScope scope(c.stream, mc.in_workspace ? LaunchScope::NONE : LaunchScope::TMA, pdl && heavy && P.sched != nullptr,
                       (unsigned long long)grid, 1, c.rd, c.w0, c.w1);
-    scope.apply(P);
+    P.ep = scope.early_path();
     const cudaError_t em = mc.zero(c.stream);
     if (em != cudaSuccess) return (int)em;
     const cudaError_t e = unit_of(c.pl->tk, c.v.qm).tma(c.v.qm, c.mode, c.pix, c.v.finv, c.workspace != nullptr, P, grid, nw * 32, smem,
@@ -744,9 +722,10 @@ static int run_direct(const Call &c)
     // inverse calls whose coefficients are a plane (not the zig-zag stream)
     const bool may_load_early = !c.coef.ptr && !c.shifted && !(c.mode == MODE_INV && c.in.dt == DT_I16ZZ);
     const Span w2 = metrics ? Span{c.acc, 0, 3 * sizeof(double), 1} : Span{c.shifted, c.in.pitch, (size_t)c.W * 4, c.H};
-    return launch_blocks(c.stream, c.capturing, grid, P, true, may_load_early ? c.rd : Span{}, c.w0, c.w1, w2, "direct",
-                         [&](const DirectParams &Q, bool pdl, int *per_sm) {
-                             return unit_of(c.pl->tk, c.v.qm).direct(c.v.qm, c.mode, c.pix, c.v.finv, metrics, Q, grid, dim3(32, 4), c.stream, pdl, per_sm);
+    return launch_blocks(c.stream, c.capturing, grid, true, may_load_early ? c.rd : Span{}, c.w0, c.w1, w2, "direct",
+                         [&](const EarlyPath &ep, bool pdl, int *per_sm) {
+                             P.ep = ep;
+                             return unit_of(c.pl->tk, c.v.qm).direct(c.v.qm, c.mode, c.pix, c.v.finv, metrics, P, grid, dim3(32, 4), c.stream, pdl, per_sm);
                          },
                          mc.in_workspace ? mc.macc : nullptr);
 }
@@ -931,8 +910,8 @@ extern "C" int b200dct_roundtrip_any(const b200dct_plan *plan, const void *img, 
     dim3 grid;
     if (!block_grid((H + 7) / 8, (W + 7) / 8, grid)) return B200DCT_ERR_SHAPE;
     const auto launch_any = dt == B200DCT_F32 ? launch_any_f32 : launch_any_u8;
-    return launch_blocks(s, stream_capturing(s), grid, P, false, Span{}, Span{}, Span{}, Span{}, "any",
-                         [&](const AnyParams &Q, bool pdl, int *) { return launch_any(plan->tk, v.qm, v.finv, Q, grid, dim3(32, 4), s, pdl); });
+    return launch_blocks(s, stream_capturing(s), grid, false, Span{}, Span{}, Span{}, Span{}, "any",
+                         [&](const EarlyPath &, bool pdl, int *) { return launch_any(plan->tk, v.qm, v.finv, P, grid, dim3(32, 4), s, pdl); });
 }
 
 extern "C" size_t b200dct_metrics_workspace_bytes(int H, int W)

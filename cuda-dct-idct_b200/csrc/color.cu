@@ -50,8 +50,10 @@ template <class Params> // RgbParams, Rgb420Params
 static int run_rgb(cudaError_t (*launch)(const Params &, dim3, dim3, size_t, cudaStream_t, bool, int *), Params &P, dim3 grid,
                    cudaStream_t s, Span rd, Span w0, Span w1, Span w2 = Span{})
 {
-    return launch_blocks(s, stream_capturing(s), grid, P, true, rd, w0, w1, w2, "rgb",
-                         [&](const Params &Q, bool pdl, int *per_sm) { return launch(Q, grid, dim3(32, 4), 0, s, pdl, per_sm); });
+    return launch_blocks(s, stream_capturing(s), grid, true, rd, w0, w1, w2, "rgb", [&](const EarlyPath &ep, bool pdl, int *per_sm) {
+        P.ep = ep;
+        return launch(P, grid, dim3(32, 4), 0, s, pdl, per_sm);
+    });
 }
 
 extern "C" int b200dct_roundtrip_rgb(const b200dct_plan *plan, const void *rgb, size_t in_pitch, void *out,
@@ -161,16 +163,9 @@ extern "C" int b200dct_inverse_rgb420(const b200dct_plan *plan, const void *zz_y
     if (rc != B200DCT_OK) return rc;
     static const Rgb420Launcher launchers[2] = {launch_kernel<k_rgb420_inverse<false>>, launch_kernel<k_rgb420_inverse<true>>};
     grid = dim3((unsigned)((P.my + R420_MY - 1) / R420_MY), (unsigned)((P.mx + R420_MX - 1) / R420_MX));
-    // the early path's read span: the range that bounds the three streams (conservative when they lie apart)
-    const Span sp[3] = {y_span(zz_y, H, W), c_span(zz_cb, H, W), c_span(zz_cr, H, W)};
-    uintptr_t lo = ~(uintptr_t)0, hi = 0;
-    for (const Span &x : sp) {
-        lo = (uintptr_t)x.ptr < lo ? (uintptr_t)x.ptr : lo;
-        const uintptr_t end = (uintptr_t)x.ptr + (size_t)(x.rows - 1) * x.pitch + x.row_bytes;
-        hi = end > hi ? end : hi;
-    }
+    // the early path's read span: one range over the three streams
     return run_rgb(launchers[use_factored_inverse_u8(plan)], P, grid, (cudaStream_t)stream,
-                      Span{(const void *)lo, hi - lo, hi - lo, 1}, rgb_span(out, out_pitch, H, W), Span{}, Span{});
+                   span_hull({y_span(zz_y, H, W), c_span(zz_cb, H, W), c_span(zz_cr, H, W)}), rgb_span(out, out_pitch, H, W), Span{}, Span{});
 }
 
 // ------------------------------------------------------------------ coded size of a coefficient stream

@@ -146,6 +146,48 @@ __device__ __forceinline__ unsigned long long ld_counter(const unsigned long lon
     asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
     return v;
 }
+// The early path across a launch boundary, as the host decided it for one launch (see "early loads" in b200dct.cu for
+// why it is safe).  The first `early` CTAs of the grid (at most one machine-full: later CTAs only start once these
+// have left, i.e. after the predecessor completed) may read and compute before griddepcontrol.wait, with L2-coherent
+// loads, if the completion counter `chain` still reads below `chain_target`: the predecessor is then provably still
+// running.  Every global write of such a CTA comes after its wait.  chain_feed = F > 0: the last F CTAs of the grid
+// add 1 each to the counter at their end (the TMA family: F = 1, its last warp out).  A launch the host sets up to
+// feed must feed: a counter left short would make every later launch on the stream believe its predecessor still
+// runs.  One reader per CTA and at most 1024 feeders: 32768 warps polling one L2 line per launch cost the HBM-bound
+// kernels 2-15 us.  All zero: the launch takes no part.
+struct EarlyPath {
+    int early;
+    int chain_feed;
+    unsigned long long *chain;
+    unsigned long long chain_target;
+};
+// the CTA's index in its grid, counted along x, then y, then z (the image of a batch)
+__device__ __forceinline__ unsigned cta_index() { return (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x; }
+// The check in two halves, so that a kernel can hide the read's latency behind other set-up: the CTA's leader thread
+// reads the counter (early_read), then every thread of the CTA takes the CTA-uniform decision on what the leader read,
+// seen() (early_decide, a CTA barrier; non-zero: early).
+__device__ __forceinline__ unsigned long long early_read(const EarlyPath &ep) { return ld_counter(ep.chain); }
+template <class Seen>
+__device__ __forceinline__ int early_decide(const EarlyPath &ep, bool leader, Seen &&seen)
+{
+    __shared__ int s_early;
+    if (leader) s_early = seen() < ep.chain_target;
+    __syncthreads();
+    return s_early;
+}
+// the CTA is one of the grid's first `early` CTAs
+__device__ __forceinline__ bool early_leading(const EarlyPath &ep) { return ep.early != 0 && cta_index() < (unsigned)ep.early; }
+// The whole check: true when this CTA takes the early path.  leader: one thread of the CTA that has not returned.
+__device__ __forceinline__ bool early_check(const EarlyPath &ep, bool leader)
+{
+    if (early_leading(ep)) return early_decide(ep, leader, [&] { return early_read(ep); }) != 0;
+    return false;
+}
+// The feed, by the same leader once the CTA's work is (as good as) done.
+__device__ __forceinline__ void early_feed(const EarlyPath &ep, bool leader)
+{
+    if (ep.chain_feed && leader && cta_index() + (unsigned)ep.chain_feed >= gridDim.x * gridDim.y * gridDim.z) atomicAdd(ep.chain, 1ull);
+}
 // f32 metrics: every block's float sums are converted EXACTLY to unsigned 128-bit fixed point in units of 2^-50 and
 // accumulated as integers (order-independent => deterministic).  The floor: a block sum rounds to a multiple of
 // 2^-50; the ceiling: totals below 2^78 (2^22 blocks of 64 pixels of magnitude 2^20 sum to 2^68).
@@ -228,20 +270,9 @@ struct DirectParams {
     // f32 planes that are 32-byte aligned in address and pitch move with 256-bit accesses: bit 0 = the input plane
     // (all inputs of a batch), bit 1 = the output plane, bit 2 = the optional coefficient plane of a round trip
     int v8;
-    // early = E > 0 (never with a coefficient plane beside a round trip, the X-128 write-back or a zig-zag input
-    // stream: every global write must be in the store section): the host has established that nothing
-    // this launch READS is written by the launch it may overlap with (see early loads, b200dct.cu).  The first
-    // E CTAs of the grid (one machine-full: later CTAs only start once these have left, i.e. after the
-    // predecessor completed) load their block (L2-coherent loads) and transform it before griddepcontrol.wait,
-    // only their stores wait for the predecessor to complete: they work in the slots its last wave leaves idle.
-    int early;
-    // completion counter of the (device, stream) record (b200dct.cu): chain_feed = F > 0: the last F CTAs of
-    // the grid add 1 each at their end; a CTA takes the early path only if the counter still reads below
-    // chain_target, i.e. the predecessor is provably still running.  (One reader per CTA, F <= 1024 feeders:
-    // 32768 warps polling one L2 line per launch cost the HBM-bound kernels 2-15 us.)
-    int chain_feed;
-    unsigned long long *chain;
-    unsigned long long chain_target;
+    // never early with a coefficient plane beside a round trip, the X-128 write-back or a zig-zag input stream:
+    // every global write must be in the store section
+    EarlyPath ep;
     const void *img_in[DIRECT_BATCH_MAX];
     void *img_out[DIRECT_BATCH_MAX];
     CommonParams cp;
@@ -412,14 +443,12 @@ __global__ void __launch_bounds__(128, METRICS ? METRICS_CTAS_PER_SM : DIRECT_CT
     unsigned i_xx = 0, i_xy = 0, i_yy = 0; // u8 metrics
     // programmatic dependent launch (no-ops unless the host asked for it): see k_tma
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    // thread (0,0) is always valid; every global write of a launch without coef and shifted is in its store section.
+    // The check's parts rather than early_check behind these tests: the nested form schedules the metrics kernels
+    // differently (and spills differently in one of them).
     bool early = false;
-    if (P.early != 0 && P.coef == nullptr && P.shifted == nullptr && // every global write of such a launch is in its store section
-        (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x < (unsigned)P.early) { // CTA-uniform
-        __shared__ int s_early;
-        if (threadIdx.x == 0 && threadIdx.y == 0) s_early = ld_counter(P.chain) < P.chain_target; // thread (0,0) is always valid
-        __syncthreads();
-        early = s_early != 0;
-    }
+    if (P.coef == nullptr && P.shifted == nullptr && early_leading(P.ep))
+        early = early_decide(P.ep, threadIdx.x == 0 && threadIdx.y == 0, [&] { return early_read(P.ep); }) != 0;
     if (!early) asm volatile("griddepcontrol.wait;" ::: "memory");
 
     // zig-zag stream: full warps transpose their 4 KiB span through shared memory (warp-uniform)
@@ -539,9 +568,7 @@ __global__ void __launch_bounds__(128, METRICS ? METRICS_CTAS_PER_SM : DIRECT_CT
         });
     }
 
-    if (P.chain_feed && threadIdx.x == 0 && threadIdx.y == 0 &&
-        (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x + (unsigned)P.chain_feed >= gridDim.x * gridDim.y * gridDim.z)
-        atomicAdd(P.chain, 1ull); // one of the last CTAs of the grid is (as good as) done
+    early_feed(P.ep, threadIdx.x == 0 && threadIdx.y == 0);
     if constexpr (METRICS) {
         using Acc = std::conditional_t<PIX == DT_U8, unsigned long long, U128>;
         Acc v[2] = {Acc{}, Acc{}};
@@ -612,15 +639,7 @@ struct TmaParams {
     // => deterministic)
     unsigned long long *macc;
     double *acc;          // METRICS (always with the dynamic scheduler): the last warp out adds macc into acc[0..2] and re-zeroes macc
-    // 1: the host has established that nothing this launch READS is written by the launch it may
-    // overlap with (see LaunchScope in b200dct.cu): tile loads start before griddepcontrol.wait,
-    // every global write (TMA stores, metrics atomics) still waits for the predecessor to complete
-    int early_loads;
-    // completion counter of the (device, stream) record: chain_feed = 1: the last warp out adds 1; early_loads = 1:
-    // a warp only loads early if the counter still reads below chain_target (predecessor provably still running)
-    int chain_feed;
-    unsigned long long *chain;
-    unsigned long long chain_target;
+    EarlyPath ep;         // early: tile loads; every global write (TMA stores, metrics atomics) waits
     uint32_t bx;          // blocks per image row (lanes of a right-edge tile beyond it hold TMA zero fill, not pixels)
     CommonParams cp;
 };
@@ -819,9 +838,9 @@ __global__ void __launch_bounds__(METRICS ? TMA_METRICS_THREADS : tma_cta_thread
     // touch global memory before every earlier kernel has completed and flushed.
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     // early loads: ONE thread of the CTA reads the completion counter (1184 warps polling one L2 line cost
-    // 0.5 us per launch); issued here, consumed after the barrier set-up below
+    // 0.5 us per launch); issued here, consumed after the barrier set-up below.  Every CTA is a leading CTA.
     unsigned long long chain_seen = 0;
-    if (P.early_loads && threadIdx.x == 0) chain_seen = ld_counter(P.chain);
+    if (P.ep.early && threadIdx.x == 0) chain_seen = early_read(P.ep);
     if (lane == 0) {
         mbar_init(bar0, 1);
         if constexpr (METRICS) mbar_init(bar0 + 8, 1);
@@ -836,13 +855,8 @@ __global__ void __launch_bounds__(METRICS ? TMA_METRICS_THREADS : tma_cta_thread
         }
     }
     // Only lane 0 ever touches global memory (TMA loads / stores, scheduler and metrics atomics).
-    bool early = false;
-    if (P.early_loads) { // CTA-uniform; the only CTA-wide barrier of the kernel, before any work exists
-        __shared__ int s_early;
-        if (threadIdx.x == 0) s_early = chain_seen < P.chain_target;
-        __syncthreads();
-        early = s_early != 0;
-    }
+    bool early = false; // the only CTA-wide barrier of the kernel, before any work exists
+    if (P.ep.early) early = early_decide(P.ep, threadIdx.x == 0, [&] { return chain_seen; }) != 0;
     bool dep_done = !early;
     auto ensure_dep = [&]() { // lane 0, before its first global write
         if (!dep_done) {
@@ -991,7 +1005,7 @@ __global__ void __launch_bounds__(METRICS ? TMA_METRICS_THREADS : tma_cta_thread
                 if constexpr (METRICS) metrics_fold(P.macc, P.acc, METRICS_FIXED_POINT);
                 sched[0] = 0;
                 sched[1] = 0;
-                if (P.chain_feed) atomicAdd(P.chain, 1ull); // this launch is (as good as) complete
+                if (P.ep.chain_feed) atomicAdd(P.ep.chain, 1ull); // this launch is (as good as) complete
                 __threadfence();
             }
         }

@@ -1,5 +1,7 @@
 // plan_internal.h -- the plan object behind the opaque b200dct_plan handle (host TUs only).
 #pragma once
+#include <initializer_list>
+
 #include "b200dct.h"
 #include "any_kernels.cuh"
 #include "rgb_kernels.cuh"
@@ -24,8 +26,21 @@ struct b200dct_plan {
 
 
 namespace b200dct {
-struct MmaParams;
-struct Span { const void *ptr; size_t pitch, row_bytes; int rows; }; // rows of row_bytes, pitch bytes apart
+struct Span {
+    const void *ptr; size_t pitch, row_bytes; int rows; // rows of row_bytes, pitch bytes apart
+    uintptr_t end() const { return (uintptr_t)ptr + (size_t)(rows - 1) * pitch + row_bytes; } // past the last byte
+};
+// one span from the lowest start to the highest end of `spans` (conservative where they lie apart)
+inline Span span_hull(std::initializer_list<Span> spans)
+{
+    uintptr_t lo = ~(uintptr_t)0, hi = 0;
+    for (const Span &x : spans) {
+        lo = (uintptr_t)x.ptr < lo ? (uintptr_t)x.ptr : lo;
+        hi = x.end() > hi ? x.end() : hi;
+    }
+    return Span{(const void *)lo, hi - lo, hi - lo, 1};
+}
+struct LastLaunch; // the (device, stream) record of b200dct.cu
 // Every launch of a library kernel happens inside one of these (see "early loads" in b200dct.cu).  The scope
 // holds the launch-order lock from its decision until done() or its end, so that the per-(device, stream)
 // record of the last launch follows stream order even when several host threads launch on one stream.
@@ -43,34 +58,14 @@ public:
     ~LaunchScope() { done(false); }
     LaunchScope(const LaunchScope &) = delete;
     LaunchScope &operator=(const LaunchScope &) = delete;
-    // the decision in the kernel's parameters
-    template <class DirectStyleParams> // DirectParams, RgbParams
-    void apply(DirectStyleParams &P) const
-    {
-        P.early = early_;
-        P.chain_feed = chain_feed_;
-        P.chain = chain_;
-        P.chain_target = chain_target_;
-    }
-    void apply(TmaParams &P) const
-    {
-        P.early_loads = early_;
-        P.chain_feed = chain_feed_;
-        P.chain = chain_;
-        P.chain_target = chain_target_;
-    }
-    // kernels without the early path (any size, tensor-core arm): nothing to pass
-    void apply(AnyParams &) const {}
-    void apply(MmaParams &) const {}
+    // the decision, for the kernel's parameters
+    const EarlyPath &early_path() const { return ep_; }
     // launched: the scope's kernels are in the stream and the record describes them from now on; releases the lock
     void done(bool launched);
 private:
     Family family_;
-    int early_ = 0;                       // leading CTAs that may load before griddepcontrol.wait (TMA: 1 = early tile loads)
-    int chain_feed_ = 0;                  // what the kernel adds to the completion counter in total
-    unsigned long long *chain_ = nullptr; // completion counter of the (device, stream) record
-    unsigned long long chain_target_ = 0; // its value once the predecessor is complete
-    void *rec_ = nullptr;                 // the (device, stream) record of b200dct.cu
+    EarlyPath ep_{};
+    LastLaunch *rec_ = nullptr;
     Span w_[3];
     bool finished_ = false;
 };
@@ -96,28 +91,27 @@ inline bool block_grid(int by, int bx, dim3 &grid)
 
 // One launch of a kernel of hardware-scheduled 32 x 4-thread CTAs (direct family, any size, tensor-core arm, colour) in
 // the library's launch order: dependent launch unless the stream is capturing; with `early`, a part in the early path
-// (LaunchScope::DIRECT at the occupancy of the very kernel) reading rd (ptr NULL: never early) and writing w0 .. w2.  The
-// decision goes into P, and this thread's last launch is `path`.  launch(P, pdl, ctas_per_sm) launches, or with
-// ctas_per_sm != NULL only reports the kernel's resident CTAs per SM.
+// (LaunchScope::DIRECT at the occupancy of the very kernel) reading rd (ptr NULL: never early) and writing w0 .. w2.  This
+// thread's last launch is `path`.  launch(ep, pdl, ctas_per_sm) launches with the decision ep (the kernels without an
+// early path ignore it), or with ctas_per_sm != NULL only reports the kernel's resident CTAs per SM.
 // workspace: the metrics workspace the kernel counts in (NULL: none), zeroed on the stream inside the scope ahead of the
 // kernel; its contents are unknown before that, so such a launch takes no part in the early path and has no dependent launch.
-template <class Params, class Launch>
-int launch_blocks(cudaStream_t s, bool capturing, dim3 grid, Params &P, bool early, Span rd, Span w0, Span w1, Span w2,
-                  const char *path, Launch &&launch, void *workspace = nullptr)
+template <class Launch>
+int launch_blocks(cudaStream_t s, bool capturing, dim3 grid, bool early, Span rd, Span w0, Span w1, Span w2, const char *path,
+                  Launch &&launch, void *workspace = nullptr)
 {
     const bool pdl = pdl_enabled(capturing) && !workspace;
     const bool part = early && !workspace;
     const bool usable = part && pdl;
     int per_sm = 0;
-    if (usable) launch(P, pdl, &per_sm);
+    if (usable) launch(EarlyPath{}, pdl, &per_sm);
     LaunchScope scope(s, part ? LaunchScope::DIRECT : LaunchScope::NONE, usable, (unsigned long long)grid.x * grid.y, per_sm, rd,
                       w0, w1, w2);
-    scope.apply(P);
     if (workspace) {
         const cudaError_t e = cudaMemsetAsync(workspace, 0, METRICS_WORKSPACE_BYTES, s);
         if (e != cudaSuccess) return (int)e;
     }
-    const cudaError_t e = launch(P, pdl, nullptr);
+    const cudaError_t e = launch(scope.early_path(), pdl, nullptr);
     if (e != cudaSuccess) return (int)e;
     scope.done(true);
     note_launch(1, path);

@@ -26,9 +26,7 @@ struct Rgb420Params {
     size_t in_pitch, out_pitch;
     size_t zz_pitch[2];       // bytes per block-row: [0] Y, [1] Cb and Cr
     int mx, my;               // MCUs (16 x 16 pixels) per row / column
-    int early, chain_feed;    // early path across a launch boundary, as RgbParams
-    unsigned long long *chain;
-    unsigned long long chain_target;
+    EarlyPath ep;
     PlaneTables t[2];         // [0] luminance, [1] chrominance
 };
 
@@ -46,7 +44,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb420_forward(const _
     const int bxi = blockIdx.y * 32 + threadIdx.x;
     const long long by = (long long)blockIdx.x * 4 + threadIdx.y;
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    const bool early = rgb_early(P, tid);
+    const bool early = early_check(P.ep, tid == 0);
     if (!early) asm volatile("griddepcontrol.wait;" ::: "memory");
 
     if (bxi < 2 * P.mx && by < 2 * P.my) {
@@ -102,7 +100,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb420_forward(const _
         }
         st_block_zigzag((char *)P.zz[pl] + (size_t)row * P.zz_pitch[!luma] + (size_t)col * 128, p);
     }
-    rgb_feed_chain(P, tid);
+    early_feed(P.ep, tid == 0);
 }
 
 // ---- inverse.  A 128-thread CTA owns a tile of R420_MX x R420_MY MCUs.  Upsampling reads one chroma sample beyond
@@ -159,7 +157,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb420_inverse(const _
     const int tid = threadIdx.y * 32 + threadIdx.x;
     const int cy0 = blockIdx.x * R420_MY, cx0 = blockIdx.y * R420_MX; // tile origin, in MCUs = chroma blocks
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    const bool early = rgb_early(P, tid);
+    const bool early = early_check(P.ep, tid == 0);
     if (!early) asm volatile("griddepcontrol.wait;" ::: "memory");
 
     // own chroma blocks and the ring around them: local block (lr, lc), -1 and R420_MY / R420_MX = ring
@@ -208,7 +206,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb420_inverse(const _
             ycc_row_to_rgb(ypark[r][tid], bw, rw, dst + (size_t)r * P.out_pitch);
         }
     }
-    rgb_feed_chain(P, tid);
+    early_feed(P.ep, tid == 0);
 }
 
 } // namespace b200dct

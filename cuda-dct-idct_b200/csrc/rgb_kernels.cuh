@@ -59,11 +59,7 @@ struct RgbParams {
                      // the fused kernel, output of the forward kernel, input of the inverse kernel
     size_t in_pitch, out_pitch, zz_plane, zz_pitch; // bytes; zz_pitch = bytes per block-row of one stream
     int bx, by;
-    // early path across a launch boundary (not for the fused kernel with streams), as DirectParams: early = leading
-    // CTAs that may load and transform before griddepcontrol.wait, chain_feed = trailing CTAs that feed the counter
-    int early, chain_feed;
-    unsigned long long *chain;
-    unsigned long long chain_target;
+    EarlyPath ep;    // not for the fused kernel with streams
     PlaneTables t[2]; // [0] luminance, [1] chrominance
 };
 template <bool MASKED, bool FASTDIV>
@@ -123,21 +119,8 @@ constexpr int RGB_CTAS_PER_SM = 5;
 // [plane][row][thread] 8-byte slots: a warp's access is 256 contiguous bytes (conflict-free)
 using RgbPark = uint2[3][8][128];
 
-// The pieces below are shared by the fused kernel and the two halves of the split API.  The early path (see
-// early loads, b200dct.cu): the leading P.early CTAs of the grid may read and compute before
-// griddepcontrol.wait while the library's predecessor on the stream is provably still running; then every
-// global write of such a CTA must come after its wait.
-template <class Params> // RgbParams, Rgb420Params
-__device__ __forceinline__ bool rgb_early(const Params &P, int tid)
-{
-    if (P.early != 0 && blockIdx.y * gridDim.x + blockIdx.x < (unsigned)P.early) { // CTA-uniform
-        __shared__ int s_early;
-        if (tid == 0) s_early = ld_counter(P.chain) < P.chain_target; // thread 0 of a CTA is always inside the image
-        __syncthreads();
-        return s_early != 0;
-    }
-    return false;
-}
+// The pieces below are shared by the fused kernel and the two halves of the split API.  Thread 0 of a CTA is always
+// inside the image: it is the CTA's leader in the early path (EarlyPath).
 // load + RGB -> YCbCr (jccolor.c rgb_ycc_convert) of the thread's 8x8 position, one row per iteration
 __device__ __forceinline__ void rgb_load_ycc(const RgbParams &P, long long by, int bxi, int tid, bool early, RgbPark &park)
 {
@@ -185,14 +168,6 @@ __device__ __forceinline__ void rgb_store_ycc(const RgbParams &P, long long by, 
 #pragma unroll 1
     for (int r = 0; r < 8; r++) ycc_row_to_rgb(park[0][r][tid], park[1][r][tid], park[2][r][tid], dst + (size_t)r * P.out_pitch);
 }
-// Every machine-filling launch must feed the stream's completion counter (P.chain_feed set by the host): a counter
-// left short would make every later call on the stream believe its predecessor is still running.
-template <class Params>
-__device__ __forceinline__ void rgb_feed_chain(const Params &P, int tid)
-{
-    if (P.chain_feed && tid == 0 && blockIdx.y * gridDim.x + blockIdx.x + (unsigned)P.chain_feed >= gridDim.x * gridDim.y)
-        atomicAdd(P.chain, 1ull); // one of the last CTAs of the grid is (as good as) done
-}
 
 // ZZ: also emit the three zig-zag coefficient streams (its own instantiation: 150 instructions the
 // default kernel does not have to carry through the instruction cache)
@@ -206,7 +181,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb(const __grid_const
     if (bxi >= P.bx || by >= P.by) return;
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     bool early = false;
-    if constexpr (!ZZ) early = rgb_early(P, tid); // the host never offers the early path with streams (written mid-kernel)
+    if constexpr (!ZZ) early = early_check(P.ep, tid == 0); // the host never offers the early path with streams (written mid-kernel)
     if (!early) asm volatile("griddepcontrol.wait;" ::: "memory");
 
     rgb_load_ycc(P, by, bxi, tid, early, park);
@@ -230,7 +205,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb(const __grid_const
 
     if (early) asm volatile("griddepcontrol.wait;" ::: "memory"); // every global write waits for the predecessor
     rgb_store_ycc(P, by, bxi, tid, park);
-    rgb_feed_chain(P, tid);
+    early_feed(P.ep, tid == 0);
 }
 
 // ---- the two halves of k_rgb (b200dct_forward_rgb / b200dct_inverse_rgb): the same arithmetic, so
@@ -246,7 +221,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb_forward(const __gr
     const long long by = (long long)blockIdx.x * 4 + threadIdx.y;
     if (bxi >= P.bx || by >= P.by) return;
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    const bool early = rgb_early(P, tid);
+    const bool early = early_check(P.ep, tid == 0);
     if (!early) asm volatile("griddepcontrol.wait;" ::: "memory");
 
     rgb_load_ycc(P, by, bxi, tid, early, park);
@@ -258,7 +233,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb_forward(const __gr
         if (early && plane == 0) asm volatile("griddepcontrol.wait;" ::: "memory"); // before the first global write
         st_block_zigzag((char *)P.zz + (size_t)plane * P.zz_plane + (size_t)by * P.zz_pitch + (size_t)bxi * 128, p);
     }
-    rgb_feed_chain(P, tid);
+    early_feed(P.ep, tid == 0);
 }
 // Inverse: zig-zag streams -> per plane dequantise + idct + convertToUnsignedChar -> YCbCr -> RGB (reads P.zz,
 // writes P.out).  Both inverse routines read only Q (qp.d), never the mask or 1/Q, so there is no quantiser variant.
@@ -272,7 +247,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb_inverse(const __gr
     const long long by = (long long)blockIdx.x * 4 + threadIdx.y;
     if (bxi >= P.bx || by >= P.by) return;
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    const bool early = rgb_early(P, tid);
+    const bool early = early_check(P.ep, tid == 0);
     if (!early) asm volatile("griddepcontrol.wait;" ::: "memory");
 
 #pragma unroll 1
@@ -293,7 +268,7 @@ __global__ void __launch_bounds__(128, RGB_CTAS_PER_SM) k_rgb_inverse(const __gr
 
     if (early) asm volatile("griddepcontrol.wait;" ::: "memory"); // every global write waits for the predecessor
     rgb_store_ycc(P, by, bxi, tid, park);
-    rgb_feed_chain(P, tid);
+    early_feed(P.ep, tid == 0);
 }
 
 } // namespace b200dct
