@@ -21,7 +21,13 @@ tile).  An f32 plane is placed 32-byte aligned ('a'), at a 16-byte offset ('h') 
 multiple of 16 bytes ('p'); the direct family moves 32-byte aligned f32 planes with 256-bit accesses, one bit
 per plane (DirectParams::v8), and the v8 cells set and clear each bit with the other two fixed.
 
-The last test asserts that passing cells launched every kernel of the inventory.
+Deep twins (DEEP): every cell of the TMA family again at W = 2080 (a partial last tile column) and an H derived from
+the device's SM count and the cell's CTA size, so that every warp of the persistent kernel works through several
+tiles: run tickets, then single tickets, a tail that starts on an odd remainder (tests/tma_depth.py).  A deep cell
+reads its launch's grid and block from the profiler trace and asserts that regime, then checks the whole image.
+
+The last tests assert that passing cells launched every kernel of the inventory, and passing deep cells every
+kernel of the TMA family.
 """
 from __future__ import annotations
 
@@ -35,6 +41,7 @@ import pytest
 import f64ref as R
 import kernel_ledger as KL
 import rgb420_ref
+import tma_depth as D
 
 torch = pytest.importorskip("torch")
 
@@ -56,6 +63,8 @@ ALLOWLIST: dict[str, str] = {}
 
 LAUNCHED: dict[str, str] = {}   # key -> first passing cell that launched it
 CELLS_PASSED: set[str] = set()
+DEEP_LAUNCHED: dict[str, str] = {}   # the same for the deep cells
+DEEP_PASSED: set[str] = set()
 
 
 # ---------------------------------------------------------------- plans
@@ -187,30 +196,41 @@ def inventory():
     return KL.inventory()
 
 
-def launched_by(inventory, fn):
-    """Run fn() under torch.profiler (CUDA activity only); the set of inventory keys it launched."""
+def launched_by(inventory, fn, geometry=False):
+    """Run fn() under torch.profiler (CUDA activity only); the set of inventory keys it launched, and with
+    `geometry` the (name, grid, block) of every kernel from the exported trace (else None)."""
     from torch.profiler import ProfilerActivity, profile
 
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        res = fn()
+    if geometry:
+        res, prof, geo = D.profiled(fn)
+    else:
         torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            D.warm_up()
+            res = fn()
+            torch.cuda.synchronize()
+        geo = None
     keys = {KL.canonical(e.name) for e in prof.events()}
-    return res, keys & set(inventory)
+    return res, keys & set(inventory), geo
 
 
-def expect_launch(inventory, cell_id, want, fn):
+def expect_launch(inventory, cell_id, want, fn, deep_tiles=None):
+    """deep_tiles: the tile count of a deep cell, whose k_tma launch must put every warp past two rounds (R3)."""
     want = {want} if isinstance(want, str) else set(want)
     assert want <= set(inventory), f"{cell_id}: expected kernels {want - set(inventory)} are not in the inventory"
-    res, got = launched_by(inventory, fn)
+    res, got, geo = launched_by(inventory, fn, geometry=deep_tiles is not None)
     assert got == want, f"{cell_id}: launched {sorted(got)}, expected {sorted(want)}"
+    if deep_tiles is not None:
+        key, grid, block = D.tma_launch(geo, KL.canonical)
+        assert deep_tiles > 2 * grid * (block // 32) and D.regime(deep_tiles, grid, block) == "R3", \
+            f"{cell_id}: {deep_tiles} tiles on grid {grid} x {block // 32} warps is not the deep regime"
     return res, want
 
 
-def passed(cell_id, keys):
-    CELLS_PASSED.add(cell_id)
+def passed(cell_id, keys, deep=False):
+    (DEEP_PASSED if deep else CELLS_PASSED).add(cell_id)
     for k in keys:
-        LAUNCHED.setdefault(k, cell_id)
+        (DEEP_LAUNCHED if deep else LAUNCHED).setdefault(k, cell_id)
 
 
 # ---------------------------------------------------------------- the planar cells
@@ -224,11 +244,12 @@ class Cell(NamedTuple):
     layout: str = "aaa"  # alignment of the (input, output, coefficient) f32 planes
     W: int = PART
     H: int = H0
+    deep: bool = False   # H is the deep height of the device and the cell's CTA size (tma_depth.deep_height)
 
     @property
     def id(self):
         return (f"{self.entry}-{self.family}-{self.unit}-{self.pix}-{self.coef or 'none'}-{self.inv}-{self.layout}-"
-                f"{self.H}x{self.W}")
+                f"{'deep' if self.deep else self.H}x{self.W}")
 
 
 MODE = {"fwd": 0, "inv": 1, "rt": 2, "met": 2, "batch": 2}
@@ -318,6 +339,25 @@ def planar_cells():
 PLANAR = planar_cells()
 
 
+def deep_cells():
+    """A twin of every TMA-family cell at the deep width; its height is chosen on the device."""
+    return list({d.id: d for d in (c._replace(W=D.DEEP_W, H=0, deep=True) for c in PLANAR if c.family == "tma")}.values())
+
+
+DEEP = deep_cells()
+
+
+def cta_warps(c: Cell) -> int:
+    """Warps per CTA of the cell's k_tma launch (see tma_depth.cta_warps)."""
+    coef = {"f32": "f32", "i16": "i16", None: None}[c.coef]
+    planes = {"fwd": [c.pix, coef], "inv": [coef, c.pix]}.get(c.entry, [c.pix, c.pix] + ([coef] if coef else []))
+    return D.cta_warps(c.pix, UNITS[c.unit].tk, planes, metrics=c.entry == "met")
+
+
+def sm_count() -> int:
+    return torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+
+
 def _param(c: Cell):
     marks = [pytest.mark.factored] if reassociated(c) else []
     return pytest.param(c, id=c.id, marks=marks)
@@ -355,14 +395,19 @@ def check_pixels(what, got, C, T, Q, exact_want=None):
     if exact_want is not None:
         assert equal(got, exact_want), f"{what}: pixels differ from the oracle"
         return
-    P, Bi = R.inverse64(C, T, Q)
-    ch = R.check_u8(got, P, Bi) if got.dtype == np.uint8 else R.check_close(got, P, Bi)
+    ch = D.check_pixels_banded(got, C, T, Q)
     assert ch.bad == 0, f"{what}: pixels outside the float64 bound: {ch}"
 
 
-@pytest.mark.parametrize("c", [_param(c) for c in PLANAR])
+@pytest.mark.parametrize("c", [_param(c) for c in PLANAR + DEEP])
 def test_cell(dct, oracle, inventory, c: Cell):
     u = UNITS[c.unit]
+    deep_tiles = None
+    if c.deep:
+        c = c._replace(H=D.deep_height(sm_count(), cta_warps(c), c.W))
+        deep_tiles = D.ntiles(c.H, c.W)
+    launch = lambda key, fn: expect_launch(inventory, c.id, key, fn, deep_tiles)  # noqa: E731
+    nthr = oracle.max_threads()
     plan, T, Q, keep = make_plan(dct, oracle, u, c.family, c.inv == "f")
     Tn = None if u.T == "haweel" else T
     key = expected_kernel(c)
@@ -378,45 +423,43 @@ def test_cell(dct, oracle, inventory, c: Cell):
         imgs = [image(oracle, c, seed + k) for k in range(3)]
         ins = [Buf(c.H, c.W, pdt, data=a) for a in imgs]
         outs = [Buf(c.H, c.W, pdt) for _ in imgs]
-        _, keys = expect_launch(inventory, c.id, key, lambda: dct.roundtrip_batch([b.view for b in ins], [o.view for o in outs],
-                                                                                  plan=plan))
+        _, keys = launch(key, lambda: dct.roundtrip_batch([b.view for b in ins], [o.view for o in outs], plan=plan))
         for a, i, o in zip(imgs, ins, outs):
             assert i.unchanged() and o.guards_intact()
             if exact:
                 check_pixels(c.id, o.host(), None, T, Q, oracle.roundtrip(a, T=Tn, Q=Q, keep=keep))
             else:
                 check_pixels(c.id, o.host(), kernel_coefs(dct, c, i, plan), T, Q)
-        passed(c.id, keys)
+        passed(c.id, keys, c.deep)
         return
 
     if c.entry == "fwd":
         src = Buf(c.H, c.W, pdt, lay(0, pdt), data=img)
         dst = Buf(c.H, c.W, cdt, lay(1, cdt), zigzag=zz)
-        _, keys = expect_launch(inventory, c.id, key, lambda: dct.forward(src.view, dst.view, plan=plan, zigzag=zz))
+        _, keys = launch(key, lambda: dct.forward(src.view, dst.view, plan=plan, zigzag=zz))
         assert src.unchanged() and dst.guards_intact(), f"{c.id}: input changed or guard overwritten"
         got = dst.host()
         if exact:
-            assert equal(got, want_coef(oracle, oracle.dct(img.astype(F32), T=Tn, Q=Q, keep=keep), c.coef)), c.id
+            assert equal(got, want_coef(oracle, oracle.dct(img.astype(F32), T=Tn, Q=Q, keep=keep, threads=nthr), c.coef)), c.id
         else:
-            Y, B = R.forward64(img, T)
-            ch = R.check_quant(as_coef_plane(got, c.coef), Y, B, Q, keep)
+            ch = D.check_quant_banded(as_coef_plane(got, c.coef), img, T, Q, keep)
             assert ch.bad == 0, f"{c.id}: {ch}"
-        passed(c.id, keys)
+        passed(c.id, keys, c.deep)
         return
 
     if c.entry == "inv":
-        C = clip16(oracle.dct(img.astype(F32), T=Tn, Q=Q, keep=keep))
+        C = clip16(oracle.dct(img.astype(F32), T=Tn, Q=Q, keep=keep, threads=nthr))
         data = oracle.zigzag_i16(C) if zz else C.astype(np.int16) if c.coef == "i16" else C
         src = Buf(c.H, c.W, cdt, lay(0, cdt), data=data, zigzag=zz)
         dst = Buf(c.H, c.W, pdt, lay(1, pdt))
-        _, keys = expect_launch(inventory, c.id, key, lambda: dct.inverse(src.view, dst.view, plan=plan, zigzag=zz))
+        _, keys = launch(key, lambda: dct.inverse(src.view, dst.view, plan=plan, zigzag=zz))
         assert src.unchanged() and dst.guards_intact(), f"{c.id}: input changed or guard overwritten"
         want = None
         if exact:
-            P = oracle.idct(C, T=Tn, Q=Q)
+            P = oracle.idct(C, T=Tn, Q=Q, threads=nthr)
             want = P if c.pix == "f32" else oracle.to_u8(P)
         check_pixels(c.id, dst.host(), C, T, Q, want)
-        passed(c.id, keys)
+        passed(c.id, keys, c.deep)
         return
 
     # round trips, with or without fused metrics
@@ -428,18 +471,17 @@ def test_cell(dct, oracle, inventory, c: Cell):
         fn = lambda: dct.roundtrip_with_metrics(src.view, out.view, cv, plan=plan, zigzag=zz)  # noqa: E731
     else:
         fn = lambda: dct.roundtrip(src.view, out.view, cv, plan=plan, zigzag=zz)  # noqa: E731
-    res, keys = expect_launch(inventory, c.id, key, fn)
+    res, keys = launch(key, fn)
     assert src.unchanged() and out.guards_intact() and (cb is None or cb.guards_intact()), \
         f"{c.id}: input changed or guard overwritten"
     got = out.host()
     want_out = None
     if u.tk == 2:     # even/odd forward: the kernel's coefficients, within the bound of the exact ones
         C = as_coef_plane(cb.host(), c.coef) if cb is not None else kernel_coefs(dct, c, src, plan)
-        Y, B = R.forward64(img, T)
-        ch = R.check_quant(C, Y, B, Q, keep)
+        ch = D.check_quant_banded(C, img, T, Q, keep)
         assert ch.bad == 0, f"{c.id}: coefficients {ch}"
     else:             # the forward is the chain: the oracle's coefficients
-        want_out, C = oracle.roundtrip(img, T=Tn, Q=Q, keep=keep, want_coef=True, threads=oracle.max_threads())
+        want_out, C = oracle.roundtrip(img, T=Tn, Q=Q, keep=keep, want_coef=True, threads=nthr)
         if cb is not None:
             assert equal(cb.host(), want_coef(oracle, C, c.coef)), f"{c.id}: coefficients differ from the oracle"
     check_pixels(c.id, got, C, T, Q, want_out if exact else None)
@@ -447,7 +489,7 @@ def test_cell(dct, oracle, inventory, c: Cell):
         mse, peen, nnz = res[1]
         check_metrics(oracle, c.id, (mse, peen), img, got)
         assert nnz == int(np.count_nonzero(C)), f"{c.id}: non-zero count {nnz} vs {int(np.count_nonzero(C))}"
-    passed(c.id, keys)
+    passed(c.id, keys, c.deep)
 
 
 # ---------------------------------------------------------------- any size (k_any, k_any_u8)
@@ -720,3 +762,16 @@ def test_zz_every_kernel_launched(request, inventory):
         print(f"  not launched: {k}  ({ALLOWLIST.get(k, 'NOT ALLOWLISTED')})")
     assert set(never) <= set(ALLOWLIST), f"kernels no passing cell launched: {sorted(set(never) - set(ALLOWLIST))}"
     assert not set(ALLOWLIST) & launched, f"allowlisted kernels that were launched: {sorted(set(ALLOWLIST) & launched)}"
+
+
+def test_zz_every_tma_kernel_launched_at_depth(inventory):
+    """Every k_tma kernel of the inventory was launched by a passing deep cell: each one's tile loop ran with
+    several tiles per warp and was checked over the whole image."""
+    if len(DEEP_PASSED) != len(DEEP):
+        pytest.skip(f"{len(DEEP) - len(DEEP_PASSED)} of {len(DEEP)} deep cells did not run or did not pass: the ledger is incomplete")
+    tma = sorted(k for k in inventory if k.startswith("k_tma<"))
+    print(f"{len(tma)} TMA kernels, launched at depth by {len(DEEP_PASSED)} deep cells")
+    for k in tma:
+        print(f"  {k}  {DEEP_LAUNCHED.get(k, 'NOT LAUNCHED AT DEPTH')}")
+    never = sorted(set(tma) - set(DEEP_LAUNCHED))
+    assert not never, f"TMA kernels no passing deep cell launched: {never}"
